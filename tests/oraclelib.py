@@ -201,6 +201,35 @@ class RefScene:
             pass
 
 
+def add_scene(s, kind):
+    """The fixed scenes the pinning tests render, built through the ECS API of `s` (RefScene or hostlib.HostScene)."""
+    if kind == "triangle":
+        s.add_triangle((1, 0, -3), (-1, 0, -3), (0, 1, -3), (1, 0, 0))
+    elif kind == "sphere8":
+        s.add_sphere((0, 0, -3), 1.0, 8, 8, (1, 0, 0))
+    elif kind == "mixed":
+        s.add_sphere((0.6, 0.2, -4), 0.9, 12, 9, (0.2, 0.9, 0.3))
+        s.add_triangle((2, -1, -5), (-2, -1, -5), (0, 2, -6), (0.1, 0.2, 1.0))
+        s.add_sphere((-0.8, -0.3, -2.5), 0.5, 5, 4, (1, 1, 0))
+
+
+def add_random_scene(s, seed):
+    """Triangles and tessellated spheres at random places (in front of, around and behind the camera, overlapping, some
+    degenerate) added to `s`; returns the random frame size (W, H) drawn after them."""
+    rng = np.random.default_rng(1000 + seed)
+    for _ in range(int(rng.integers(1, 7))):
+        if rng.random() < 0.5:
+            c = rng.uniform(-3, 3, 3) + np.array([0, 0, -4.0])
+            pts = c + rng.uniform(-2, 2, (3, 3))
+            if rng.random() < 0.15:
+                pts[2] = pts[1]                                  # degenerate: NaN normal in the reference (Triangle.cpp:48)
+            s.add_triangle(tuple(pts[0]), tuple(pts[1]), tuple(pts[2]), tuple(rng.uniform(0, 1, 3)))
+        else:
+            c = rng.uniform(-2.5, 2.5, 3) + np.array([0, 0, -3.0 if rng.random() < 0.8 else 3.0])
+            s.add_sphere(tuple(c), float(rng.uniform(0.2, 1.5)), int(rng.integers(3, 14)), int(rng.integers(3, 12)), tuple(rng.uniform(0, 1, 3)))
+    return int(rng.integers(2, 140)), int(rng.integers(2, 90))
+
+
 def fnv64(words):
     """64-bit FNV-1a variant over uint32 words (xor the whole word, then multiply)."""
     h = 0xcbf29ce484222325

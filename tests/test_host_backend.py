@@ -13,7 +13,6 @@ from conftest import ROOT, load_golden
 from rt3_b200 import abi, scenes
 
 META = json.load(open(os.path.join(ROOT, "tests", "golden", "goldens.json")))
-needs_ref = pytest.mark.skipif(not ol.have_ref(), reason="oracle/_ref not built (needs /root/reference)")
 
 
 def same_scene(a: abi.SceneArrays, b: abi.SceneArrays):
@@ -48,8 +47,41 @@ def test_large_tessellated_sphere_counts(built):
     assert f"{ol.fnv64(frame[:35]):016x}" == m["frame_fnv64_rows_0_to_Hm2"]
 
 
-@needs_ref
-def test_flatten_matches_compiled_reference(built):
+def teddy_obj_from_golden(path, golden):
+    """Writes an OBJ of the teddy (entity 0 of the reference's default scene) whose vertices the reference's transform maps exactly
+    onto the reference's own export of them in tests/golden/default_400x225.npz: v = (p - centre) / scale, moved by whole ulps until
+    fp32 centre + scale * v gives p back. The original teddy.obj is not in the repository; its faces are written as exported."""
+    f = np.float32
+    scale, centre = f(1.0) / f(17.0), np.array([0, 0, -3], f)
+    faces = golden.faces["v"][golden.face_entity == 0]
+    want = golden.vertices.view(f).reshape(-1, 4)[:int(faces.max()) + 1, :3]
+    guess = ((want.astype(np.float64) - centre) / np.float64(scale)).astype(f)
+    v = np.full(want.shape, np.nan, f)
+    for k in range(-8, 9):
+        cand = guess
+        for _ in range(abs(k)):
+            cand = np.nextafter(cand, f(np.inf) if k > 0 else f(-np.inf))
+        found = np.isnan(v) & (centre + scale * cand == want)
+        v[found] = cand[found]
+    assert not np.isnan(v).any()
+    with open(path, "w") as fh:
+        fh.writelines(f"v {float(x)!r} {float(y)!r} {float(z)!r}\n" for x, y, z in v)   # repr: strtof reads each value back exactly
+        fh.writelines(f"f {a + 1} {b + 1} {c + 1}\n" for a, b, c in faces)
+
+
+def test_flatten_matches_compiled_reference(built, tmp_path):
+    """The reference's default scene (src/Main.cpp:278-283: teddy at (0, 0, -3) scaled 1/17, an 8x8 sphere) through the host's OBJ
+    loader and flatten equals the reference's own export of it, bit for bit: faces, normals, colours, vertices, entity map. With
+    the compiled reference built, a five-entity scene with the original teddy.obj is also compared with it directly."""
+    _, golden = load_golden("default_400x225")
+    teddy = str(tmp_path / "teddy.obj")
+    teddy_obj_from_golden(teddy, golden)
+    hs = hostlib.HostScene()
+    hs.add_object(teddy, (0, 0, -3), 1.0 / 17.0, (1, 0, 0))
+    hs.add_sphere((-2, 0, -5), 1.0, 8, 8, (0, 0, 1))
+    same_scene(hs.flatten(), golden)
+    if not ol.have_ref():
+        return
     ref, hs = ol.RefScene(), hostlib.HostScene()
     for s in (ref, hs):
         s.add_object(ol.REF_TEDDY, (0, 0, -3), 1.0 / 17.0, (1, 0, 0))
