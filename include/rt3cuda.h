@@ -244,6 +244,31 @@ int rt3_render(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params,
 int rt3_render_aov(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, uint32_t* host_frame,
                    uint32_t* host_hit_prim, uint32_t* host_hit_entity, float* host_hit_t);
 
+/* AOVs of a path-traced render: the buffers an image denoiser takes next to the noisy colour (albedo, normal) and the
+ * primary hit per pixel (primitive, entity, depth). Host pointers, width*height pixels in frame order; any may be NULL. */
+typedef struct rt3_path_aovs {
+    uint32_t* hit_prim;   /* primitive id of the closest hit of sample first_sample (0xFFFFFFFF on a miss) */
+    uint32_t* hit_entity; /* its entity id (0xFFFFFFFF on a miss) */
+    float* hit_t;         /* its distance along the UNIT primary direction (+inf on a miss); rt3_render_aov's hit_t is measured
+                           * along the un-normalised reference-mode direction instead */
+    float* albedo;        /* 3 per pixel, mean over the samples: the albedo the path tracer multiplies by at the first hit (the
+                           * material's, or the primitive's colour without a material; 1 for a dielectric); a miss: the sky of
+                           * that direction (1 under RT3_FLAG_UNIFORM_SKY) */
+    float* normal;        /* 3 per pixel, mean over the samples (not renormalised) of the front-facing normal at the first hit
+                           * (faces: the stored face normal; spheres: (hit point - centre) / radius); a miss: 0 */
+} rt3_path_aovs;
+
+/* Renders the AOVs of the path tracer's primary rays for RT3_MODE_PATHTRACE parameters: exactly the primary rays a render
+ * with the same parameters traces for its samples [first_sample, first_sample + spp) of every owned pixel (seed, jitter,
+ * thin lens, partition), with the path tracer's closest-hit tests. Reads spp (the number of AOV samples: the parameters
+ * of a 500-spp render with spp = 16 give the AOVs of that render's first 16 samples), seed, first_sample, the partition
+ * and the flags RT3_FLAG_NO_JITTER, RT3_FLAG_UNIFORM_SKY and RT3_FLAG_BVH; max_depth and the other flags are ignored.
+ * Writes only the owned rows. Sums are kept in fixed point (2^24), so the result does not depend on scheduling,
+ * partition or GPU count. Blocking. The path tracer's accumulators and RT3_FLAG_ACCUMULATE state are not touched:
+ * rt3_read_radiance and a following accumulating render behave as if this call had not happened. rt3_get_stats then
+ * describes this call (device_ms, trace_kernel_ms, rays = primary rays traced, the test or hierarchy counters). */
+int rt3_render_path_aovs(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, const rt3_path_aovs* out);
+
 /* Device-resident variant for multi-GPU plumbing: renders this partition's
  * rows into `device_frame` (a device pointer to width*height uint32, full-frame
  * indexing) asynchronously on `cuda_stream` (a cudaStream_t; NULL = the

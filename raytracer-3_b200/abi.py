@@ -88,6 +88,11 @@ class Stats(C.Structure):
     ]
 
 
+class PathAovs(C.Structure):
+    """rt3_path_aovs: host output pointers of rt3_render_path_aovs (any may be NULL)."""
+    _fields_ = [("hit_prim", C.c_void_p), ("hit_entity", C.c_void_p), ("hit_t", C.c_void_p), ("albedo", C.c_void_p), ("normal", C.c_void_p)]
+
+
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
@@ -198,6 +203,7 @@ def load_core():
     lib.rt3_tessellate_spheres_device.argtypes = [vp, C.POINTER(UvSphere), u32, u32, u32, vp, vp, vp]
     lib.rt3_render.argtypes = [vp, C.POINTER(Camera), C.POINTER(Params), u32p]
     lib.rt3_render_aov.argtypes = [vp, C.POINTER(Camera), C.POINTER(Params), u32p, u32p, u32p, vp]
+    lib.rt3_render_path_aovs.argtypes = [vp, C.POINTER(Camera), C.POINTER(Params), C.POINTER(PathAovs)]
     lib.rt3_render_device.argtypes = [vp, C.POINTER(Camera), C.POINTER(Params), vp, vp]
     lib.rt3_partition_rows.argtypes = [u32, u32, u32, u32]
     lib.rt3_partition_rows.restype = u32
@@ -226,7 +232,7 @@ def load_core():
 EXPORTED_SYMBOLS = [
     "rt3_last_error", "rt3_create", "rt3_destroy", "rt3_scene_upload", "rt3_scene_upload_device", "rt3_buffer_alloc", "rt3_buffer_free",
     "rt3_buffer_write", "rt3_buffer_read", "rt3_tessellate_spheres_device", "rt3_render", "rt3_render_aov",
-    "rt3_render_device", "rt3_partition_rows", "rt3_pack_partition", "rt3_unpack_partition", "rt3_frame_bytes",
+    "rt3_render_path_aovs", "rt3_render_device", "rt3_partition_rows", "rt3_pack_partition", "rt3_unpack_partition", "rt3_frame_bytes",
     "rt3_frame_alloc", "rt3_frame_free", "rt3_frame_export", "rt3_frame_import", "rt3_frame_release",
     "rt3_frame_attach", "rt3_frame_read",
     "rt3_uv_sphere_faces", "rt3_uv_sphere_vertices", "rt3_tessellate_spheres",
@@ -320,6 +326,18 @@ class Context:
         self._check(self.lib.rt3_render_aov(self.handle, C.byref(camera), C.byref(params),
                                             _ptr(frame), _ptr(prim), _ptr(ent), _ptr(t)))
         return frame, prim, ent, t
+
+    def render_path_aovs(self, camera, params):
+        """rt3_render_path_aovs: AOVs of the path tracer's primary rays for pathtrace ``params`` (its spp = the AOV samples).
+
+        Returns {"hit_prim", "hit_entity": uint32 [H, W], "hit_t": float32 [H, W], "albedo", "normal": float32 [H, W, 3]};
+        rows of other partitions are 0."""
+        h, w = params.height, params.width
+        out = {"hit_prim": np.zeros((h, w), np.uint32), "hit_entity": np.zeros((h, w), np.uint32), "hit_t": np.zeros((h, w), np.float32),
+               "albedo": np.zeros((h, w, 3), np.float32), "normal": np.zeros((h, w, 3), np.float32)}
+        aovs = PathAovs(*(_ptr(out[k]) for k in ("hit_prim", "hit_entity", "hit_t", "albedo", "normal")))
+        self._check(self.lib.rt3_render_path_aovs(self.handle, C.byref(camera), C.byref(params), C.byref(aovs)))
+        return out
 
     def render_device(self, camera, params, device_ptr, stream_ptr=None):
         self._check(self.lib.rt3_render_device(self.handle, C.byref(camera), C.byref(params),

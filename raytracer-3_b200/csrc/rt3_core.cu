@@ -114,6 +114,8 @@ struct rt3_ctx {
 
     DeviceBuffer<uint32_t> frame, aov_prim, aov_entity;
     DeviceBuffer<float> aov_t;
+    DeviceBuffer<unsigned long long> aov_sums; /* rt3_render_path_aovs: RT3_AOV_SUMS per pixel, apart from the path tracer's accumulators */
+    DeviceBuffer<float> aov_albedo, aov_normal;
     DeviceBuffer<unsigned long long> accum, counters;
     uint32_t accum_width = 0, accum_height = 0; /* frame the accumulators were last cleared for */
     rt3_kparams accum_kp{};                      /* the path-traced render the accumulators currently hold */
@@ -219,6 +221,20 @@ int launch_pathtrace(rt3_ctx* ctx, const rt3_camera& cam, const rt3_kparams& kp,
     unsigned grid = (unsigned) ctx->sm_count * (unsigned) per_sm;
     if (want < grid) { grid = want ? (unsigned) want : 1u; }
     pathtrace_kernel<RESIDENT, SPHERES_ONLY, ACCEL, BIN, BEAM><<<grid, RT3_CTA_THREADS, smem, stream>>>(ctx->view, ctx->bvh, cam, kp, ctx->accum.ptr, ctx->counters.ptr);
+    RT3_CUDA(cudaGetLastError());
+    return RT3_OK;
+}
+
+template <bool RESIDENT, bool SPHERES_ONLY, bool ACCEL>
+int launch_path_aovs(rt3_ctx* ctx, const rt3_camera& cam, const rt3_kparams& kp, size_t smem, uint32_t* prim, uint32_t* ent, float* t,
+                     cudaStream_t stream) {
+    int rc = configure(path_aov_kernel<RESIDENT, SPHERES_ONLY, ACCEL>, smem, nullptr);
+    if (rc != RT3_OK) { return rc; }
+    const unsigned long long per_cta = (unsigned long long) RT3_CTA_THREADS * RT3_REF_RAYS;
+    const unsigned long long grid = (kp.n_items + per_cta - 1) / per_cta;
+    if (grid > 0x7FFFFFFFull) { return fail(RT3_ERR_INVALID, "too many AOV samples in one call (%llu)", kp.n_items); }
+    path_aov_kernel<RESIDENT, SPHERES_ONLY, ACCEL><<<(unsigned) grid, RT3_CTA_THREADS, smem, stream>>>(ctx->view, ctx->bvh, cam, kp, ctx->aov_sums.ptr, prim, ent, t,
+                                                                                                     ctx->counters.ptr);
     RT3_CUDA(cudaGetLastError());
     return RT3_OK;
 }
@@ -494,6 +510,81 @@ int render_to_host(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params
     return RT3_OK;
 }
 
+/* rt3_render_path_aovs: the AOV pass of the path tracer's primary rays on the context's stream, blocking. The sums live in
+ * buffers of their own; the accumulators, accum_kp / accum_valid and the stream rt3_read_radiance orders itself behind are
+ * left as they were. */
+int render_path_aovs(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params, const rt3_path_aovs* out) {
+    if (!params || !out) { return fail(RT3_ERR_INVALID, "params or out is NULL"); }
+    if (params->mode != RT3_MODE_PATHTRACE) { return fail(RT3_ERR_INVALID, "rt3_render_path_aovs takes RT3_MODE_PATHTRACE parameters only"); }
+    rt3_params p = *params;
+    p.max_depth = 1; /* ignored: primary rays only */
+    p.flags &= RT3_FLAG_NO_JITTER | RT3_FLAG_UNIFORM_SKY | RT3_FLAG_BVH;
+    rt3_kparams kp;
+    int rc = check_render_args(ctx, cam, &p, &kp);
+    if (rc != RT3_OK) { return rc; }
+    const size_t n = (size_t) kp.width * kp.height;
+    uint32_t *d_prim = nullptr, *d_ent = nullptr;
+    float* d_t = nullptr;
+    if ((rc = ctx->aov_sums.reserve(RT3_AOV_SUMS * n)) != RT3_OK || (rc = ctx->aov_albedo.reserve(3 * n)) != RT3_OK || (rc = ctx->aov_normal.reserve(3 * n)) != RT3_OK) { return rc; }
+    if (out->hit_prim) { if ((rc = ctx->aov_prim.reserve(n)) != RT3_OK) { return rc; } d_prim = ctx->aov_prim.ptr; }
+    if (out->hit_entity) { if ((rc = ctx->aov_entity.reserve(n)) != RT3_OK) { return rc; } d_ent = ctx->aov_entity.ptr; }
+    if (out->hit_t) { if ((rc = ctx->aov_t.reserve(n)) != RT3_OK) { return rc; } d_t = ctx->aov_t.ptr; }
+    cudaStream_t stream = ctx->stream;
+    bool resident = false;
+    size_t smem = render_smem_bytes(ctx->view, false, &resident);
+    const bool accel = (p.flags & RT3_FLAG_BVH) != 0;
+    if (accel) {
+        if ((rc = build_bvh(ctx, stream)) != RT3_OK) { return rc; }
+        resident = false; /* no constant-bank records needed */
+        smem = rt3_accel_smem_bytes(false);
+    }
+    kp.resident = resident ? 1u : 0u;
+    cudaStream_t radiance_stream = ctx->last_stream;
+    ctx->stats.accel = accel ? 1u : 0u;
+    ctx->stats_beam = false; ctx->stats_beam_accel = false;
+    ctx->stats.kernel_launches = 0;
+    ctx->stats.rows_rendered = kp.owned_rows;
+    ctx->last_stream = stream;
+    ctx->stats_pending = true;
+    ctx->copy_timed = false;
+    {
+        std::unique_lock<std::mutex> bank_lock; /* held until the kernel that reads the bank is enqueued */
+        if (resident && kp.n_pixels != 0 && (rc = claim_constant_bank(ctx, stream, bank_lock)) != RT3_OK) { return rc; }
+        RT3_CUDA(cudaEventRecord(ctx->ev_begin, stream));
+        RT3_CUDA(cudaMemsetAsync(ctx->counters.ptr, 0, 8 * sizeof(unsigned long long), stream));
+        RT3_CUDA(cudaMemsetAsync(ctx->aov_sums.ptr, 0, RT3_AOV_SUMS * n * sizeof(unsigned long long), stream));
+        RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
+        if (kp.n_pixels != 0) {
+            const bool so = ctx->view.n_faces == 0;
+            rc = accel ? launch_path_aovs<true, false, true>(ctx, *cam, kp, smem, d_prim, d_ent, d_t, stream)
+               : resident ? (so ? launch_path_aovs<true, true, false>(ctx, *cam, kp, smem, d_prim, d_ent, d_t, stream)
+                                : launch_path_aovs<true, false, false>(ctx, *cam, kp, smem, d_prim, d_ent, d_t, stream))
+                          : (so ? launch_path_aovs<false, true, false>(ctx, *cam, kp, smem, d_prim, d_ent, d_t, stream)
+                                : launch_path_aovs<false, false, false>(ctx, *cam, kp, smem, d_prim, d_ent, d_t, stream));
+            if (rc != RT3_OK) { return rc; }
+        }
+    }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k1, stream));
+    if (kp.n_pixels != 0) {
+        path_aov_resolve_kernel<<<(unsigned) ((kp.n_pixels + 255ull) / 256ull), 256, 0, stream>>>(kp, ctx->aov_sums.ptr, ctx->aov_albedo.ptr, ctx->aov_normal.ptr);
+        RT3_CUDA(cudaGetLastError());
+        ctx->stats.kernel_launches = 2;
+    }
+    RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
+    if (d_prim && (rc = copy_owned_rows(kp, d_prim, out->hit_prim, stream)) != RT3_OK) { return rc; }
+    if (d_ent && (rc = copy_owned_rows(kp, d_ent, out->hit_entity, stream)) != RT3_OK) { return rc; }
+    if (d_t && (rc = copy_owned_rows(kp, d_t, out->hit_t, stream)) != RT3_OK) { return rc; }
+    /* three floats per pixel: rows of float3 */
+    if (out->albedo && (rc = copy_owned_rows(kp, reinterpret_cast<const float3*>(ctx->aov_albedo.ptr), reinterpret_cast<float3*>(out->albedo), stream)) != RT3_OK) { return rc; }
+    if (out->normal && (rc = copy_owned_rows(kp, reinterpret_cast<const float3*>(ctx->aov_normal.ptr), reinterpret_cast<float3*>(out->normal), stream)) != RT3_OK) { return rc; }
+    RT3_CUDA(cudaEventRecord(ctx->ev_copy, stream));
+    ctx->copy_timed = true;
+    RT3_CUDA(cudaStreamSynchronize(stream));
+    rc = collect_stats(ctx);
+    if (radiance_stream) { ctx->last_stream = radiance_stream; } /* rt3_read_radiance stays behind the render that filled the accumulators */
+    return rc;
+}
+
 /* Reads back the timings and counters of the most recent render (synchronises its stream). */
 int collect_stats(rt3_ctx* ctx) {
     if (!ctx->stats_pending) { return RT3_OK; }
@@ -707,6 +798,7 @@ int rt3_destroy(rt3_ctx* ctx) {
     ctx->pair_xy.release(); ctx->pair_w.release(); ctx->filt3.release(); ctx->face_rec.release();
     ctx->spheres.release(); ctx->prim_color.release(); ctx->materials.release(); ctx->prim_material.release(); ctx->prim_entity.release();
     ctx->frame.release(); ctx->aov_prim.release(); ctx->aov_entity.release(); ctx->aov_t.release(); ctx->accum.release(); ctx->counters.release();
+    ctx->aov_sums.release(); ctx->aov_albedo.release(); ctx->aov_normal.release();
     if (ctx->ev_begin) { cudaEventDestroy(ctx->ev_begin); }
     if (ctx->ev_end) { cudaEventDestroy(ctx->ev_end); }
     if (ctx->ev_copy) { cudaEventDestroy(ctx->ev_copy); }
@@ -807,6 +899,10 @@ int rt3_render(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params,
 int rt3_render_aov(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, uint32_t* host_frame, uint32_t* host_hit_prim,
                    uint32_t* host_hit_entity, float* host_hit_t) {
     return render_to_host(ctx, camera, params, host_frame, host_hit_prim, host_hit_entity, host_hit_t, true);
+}
+
+int rt3_render_path_aovs(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, const rt3_path_aovs* out) {
+    return render_path_aovs(ctx, camera, params, out);
 }
 
 int rt3_render_device(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, uint32_t* device_frame, void* cuda_stream) {

@@ -1395,6 +1395,154 @@ pathtrace_kernel(rt3_scene_view S, rt3_bvh_view B, rt3_camera cam, rt3_kparams P
     }
 }
 
+/* ------------------------------------------------------------------------ *
+ * AOVs of the path tracer's primary rays (rt3_render_path_aovs, DESIGN.md 3.7)
+ * ------------------------------------------------------------------------ */
+
+/* Signed 2^24 fixed point for the normal sums: round to nearest even, clamped to +-2^20 (as to_fixed clamps), NaN -> 0. */
+__device__ __forceinline__ long long to_fixed_signed(float c) {
+    float s = c * RT3_ACC_SCALE;
+    if (!(s == s)) { return 0ll; }
+    s = fminf(fmaxf(s, -17592186044416.0f), 17592186044416.0f); /* 2^20 * 2^24 */
+    return __float2ll_rn(s);
+}
+
+/* Per-pixel sums of the AOV pass: albedo r, g, b (to_fixed), normal x, y, z (to_fixed_signed, two's complement). */
+#define RT3_AOV_SUMS 6
+
+/* One thread-ray per (pixel, sample) item, pixel-major: the primary ray start_path makes for that item, its closest hit
+ * through the path tracer's tests (the path-mode sweep of the constant bank or of streamed tiles, or the hierarchy), and the
+ * values shade_path sees at bounce 0 -- the albedo it multiplies by (dielectric: 1; miss: the sky of shade_miss with
+ * throughput 1) and the front-facing normal (miss: 0). Item `first_sample` of a pixel also stores the pixel's primitive,
+ * entity and distance along the unit direction. A warp's 32 consecutive items fall into one or two pixels once spp >= 32:
+ * they are summed in the warp (a segmented scan over equal pixels) and the first lane of each pixel adds the sums with
+ * six 64-bit atomics; integer sums do not depend on the order. */
+template <bool RESIDENT, bool SPHERES_ONLY, bool ACCEL>
+__global__ void __launch_bounds__(RT3_CTA_THREADS, RT3_REF_CTAS_PER_SM)
+path_aov_kernel(rt3_scene_view S, rt3_bvh_view B, rt3_camera cam, rt3_kparams P, unsigned long long* __restrict__ sums,
+                uint32_t* __restrict__ hit_prim, uint32_t* __restrict__ hit_entity, float* __restrict__ hit_t,
+                unsigned long long* __restrict__ counters) {
+    constexpr int R = RT3_REF_RAYS;
+    extern __shared__ __align__(128) unsigned char smem_raw[];
+    const rt3_smem_view sm = smem_view<RESIDENT, ACCEL, RT3_MASK_BYTES_FOR(RT3_REF_RAYS)>(smem_raw);
+    scene_prologue<RESIDENT>(sm);
+    uint32_t phase = 0u;
+
+    rt3_cam_view C;
+    C.origin = v3(cam.origin[0], cam.origin[1], cam.origin[2]);
+    C.hor = v3(cam.horizontal[0], cam.horizontal[1], cam.horizontal[2]);
+    C.ver = v3(cam.vertical[0], cam.vertical[1], cam.vertical[2]);
+    C.llc = v3(cam.lower_left_corner[0], cam.lower_left_corner[1], cam.lower_left_corner[2]);
+    C.lens_u = v3(cam.lens_u[0], cam.lens_u[1], cam.lens_u[2]);
+    C.lens_v = v3(cam.lens_v[0], cam.lens_v[1], cam.lens_v[2]);
+    C.lens_radius = cam.lens_radius;
+    C.wm1 = (float) P.width - 1.0f; C.hm1 = (float) P.height - 1.0f;
+
+    rt3_vec3 o[R], d[R];
+    bool live[R];
+    uint32_t pixel[R], sample[R], pix[R];
+    rt3_hit best[R];
+    const unsigned long long cta_first = (unsigned long long) blockIdx.x * (RT3_CTA_THREADS * R);
+#pragma unroll
+    for (int r = 0; r < R; r++) {
+        unsigned long long item = cta_first + (unsigned long long) r * RT3_CTA_THREADS + threadIdx.x;
+        live[r] = item < P.n_items;
+        if (!live[r]) { item = 0; }
+        const unsigned long long p = item / P.spp;
+        pixel[r] = (uint32_t) p; sample[r] = (uint32_t) (item - p * P.spp);
+        rt3_path s;
+        start_path(s, C, P, pixel[r], sample[r]);
+        o[r] = s.o; d[r] = s.d; pix[r] = s.pix;
+    }
+    uint32_t visits = 0, tests = 0;
+    if (ACCEL) {
+#pragma unroll
+        for (int r = 0; r < R; r++) {
+            best[r].t = __int_as_float(0x7f800000); best[r].prim = RT3_NO_HIT;
+            if (live[r]) { bvh_closest_hit<true>(S, B, o[r], d[r], best[r], visits, tests); }
+        }
+    } else {
+        sweep_scene<true, RESIDENT, SPHERES_ONLY, R>(S, sm, phase, o, d, d, live, best);
+    }
+    const uint32_t lane = threadIdx.x & 31u;
+    unsigned long long rays = 0;
+#pragma unroll
+    for (int r = 0; r < R; r++) {
+        rt3_vec3 albedo = v3(0.0f, 0.0f, 0.0f), n = v3(0.0f, 0.0f, 0.0f);
+        const uint32_t prim = best[r].prim;
+        if (live[r]) {
+            rays++;
+            if (prim == RT3_NO_HIT) {
+                albedo = shade_miss(v3(1.0f, 1.0f, 1.0f), d[r], P);
+            } else {
+                /* shade_path's bounce-0 values, in its arithmetic */
+                RT3_ASSERT(prim < S.n_prims);
+                const rt3_vec3 hp = o[r] + best[r].t * d[r];
+                rt3_vec3 outward;
+                if (prim < S.n_faces) {
+                    const float4 fn = __ldg(&S.face_rec[4 * (size_t) prim]);
+                    outward = v3(fn.x, fn.y, fn.z);
+                } else {
+                    const float4 sp = __ldg(&S.spheres[prim - S.n_faces]);
+                    const rt3_vec3 pc = hp - v3(sp.x, sp.y, sp.z);
+                    outward = v3(pc.x / sp.w, pc.y / sp.w, pc.z / sp.w);
+                }
+                n = dot3(d[r], outward) < 0.0f ? outward : -outward;
+                const uint32_t mi = __ldg(&S.prim_material[prim]);
+                if (mi == RT3_NO_HIT) {
+                    const float4 c = __ldg(&S.prim_color[prim]);
+                    albedo = v3(c.x, c.y, c.z);
+                } else {
+                    const float4 m0 = __ldg(&S.materials[2 * mi]);
+                    albedo = __float_as_uint(m0.x) == RT3_MAT_DIELECTRIC ? v3(1.0f, 1.0f, 1.0f) : v3(m0.y, m0.z, m0.w);
+                }
+            }
+            if (sample[r] == 0u) {
+                if (hit_prim) { hit_prim[pix[r]] = prim; }
+                if (hit_entity) { hit_entity[pix[r]] = prim == RT3_NO_HIT ? RT3_NO_HIT : __ldg(&S.prim_entity[prim]); }
+                if (hit_t) { hit_t[pix[r]] = best[r].t; }
+            }
+        }
+        unsigned long long v[RT3_AOV_SUMS] = { to_fixed(albedo.x), to_fixed(albedo.y), to_fixed(albedo.z), (unsigned long long) to_fixed_signed(n.x),
+                                               (unsigned long long) to_fixed_signed(n.y), (unsigned long long) to_fixed_signed(n.z) };
+        /* segmented suffix scan: after it the first lane of each run of equal pixels holds the run's sums */
+        const uint32_t key = live[r] ? pixel[r] : RT3_NO_HIT;
+#pragma unroll
+        for (uint32_t off = 1; off < 32u; off <<= 1) {
+            const uint32_t other = __shfl_down_sync(0xffffffffu, key, off);
+            const bool same = lane + off < 32u && other == key;
+#pragma unroll
+            for (int k = 0; k < RT3_AOV_SUMS; k++) {
+                const unsigned long long ov = __shfl_down_sync(0xffffffffu, v[k], off);
+                if (same) { v[k] += ov; }
+            }
+        }
+        const uint32_t prev = __shfl_up_sync(0xffffffffu, key, 1);
+        if (live[r] && (lane == 0u || prev != key)) {
+            unsigned long long* acc = sums + RT3_AOV_SUMS * (size_t) pix[r];
+#pragma unroll
+            for (int k = 0; k < RT3_AOV_SUMS; k++) { if (v[k]) { atomicAdd(acc + k, v[k]); } }
+        }
+    }
+    for (int off = 16; off > 0; off >>= 1) { rays += __shfl_down_sync(0xffffffffu, rays, off); }
+    if (lane == 0 && rays) { atomicAdd(&counters[1], rays); }
+    if (ACCEL) { count_accel(visits, tests, counters); }
+}
+
+/* The AOV sums as float means over the AOV samples (as radiance_kernel does for the radiance). */
+__global__ void path_aov_resolve_kernel(rt3_kparams P, const unsigned long long* __restrict__ sums, float* __restrict__ albedo, float* __restrict__ normal) {
+    unsigned long long p = (unsigned long long) blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= P.n_pixels) { return; }
+    uint32_t local_row = (uint32_t) (p / P.width), x = (uint32_t) (p - (unsigned long long) local_row * P.width);
+    size_t idx = (size_t) owned_row_to_global(P, local_row) * P.width + x;
+    const double scale = (double) P.spp * (double) RT3_ACC_SCALE;
+#pragma unroll
+    for (int c = 0; c < 3; c++) {
+        albedo[3 * idx + c] = (float) ((double) sums[RT3_AOV_SUMS * idx + c] / scale);
+        normal[3 * idx + c] = (float) ((double) (long long) sums[RT3_AOV_SUMS * idx + 3 + c] / scale);
+    }
+}
+
 /* Mean over samples, gamma 2, reference packing (SequentialRenderer.cpp:297). */
 __global__ void resolve_kernel(rt3_kparams P, const unsigned long long* __restrict__ accum, uint32_t* __restrict__ frame) {
     unsigned long long p = (unsigned long long) blockIdx.x * blockDim.x + threadIdx.x;

@@ -193,6 +193,29 @@ int rt3host_radiance(void* s, uint32_t width, uint32_t height, float* rgb_out, c
         if (path) { hs->renderer->write_radiance_pfm(width, height, path); }
     });
 }
+/* CudaRenderer::render_path_aovs with the reference camera and settings.aov_spp = aov_spp (out: host arrays of width * height
+ * pixels, any may be NULL) and, if dir != NULL, write_path_aovs_pfm into dir. */
+int rt3host_path_aovs(void* s, uint32_t width, uint32_t height, float focal, float vw, float vh, uint32_t aov_spp, const rt3_path_aovs* out, const char* dir) {
+    HostScene* hs = (HostScene*) s;
+    if (!hs->renderer) { g_error = "create the renderer first"; return -1; }
+    return guarded([&] {
+        hs->camera.update(width, height, focal, vw, vh);
+        CudaRenderSettings st = hs->renderer->get_settings();
+        st.aov_spp = aov_spp;
+        hs->renderer->set_settings(st);
+        CudaPathAovs aovs;
+        hs->renderer->render_path_aovs(hs->camera, aovs);
+        if (out) {
+            const size_t n = (size_t) width * height;
+            if (out->hit_prim) { std::memcpy(out->hit_prim, aovs.hit_prim.data(), n * sizeof(uint32_t)); }
+            if (out->hit_entity) { std::memcpy(out->hit_entity, aovs.hit_entity.data(), n * sizeof(uint32_t)); }
+            if (out->hit_t) { std::memcpy(out->hit_t, aovs.hit_t.data(), n * sizeof(float)); }
+            if (out->albedo) { std::memcpy(out->albedo, aovs.albedo.data(), 3 * n * sizeof(float)); }
+            if (out->normal) { std::memcpy(out->normal, aovs.normal.data(), 3 * n * sizeof(float)); }
+        }
+        if (dir) { hs->renderer->write_path_aovs_pfm(aovs, dir); }
+    });
+}
 int rt3host_camera_vectors(uint32_t width, uint32_t height, const float* look, float* out19) {
     return guarded([&] {
         Camera cam;

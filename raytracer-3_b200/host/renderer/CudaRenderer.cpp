@@ -288,18 +288,35 @@ void CudaRenderer::render_progressive(Camera& camera, uint32_t passes, FrameCall
     }
 }
 
-void CudaRenderer::render_samples(Camera& camera, uint32_t first_sample, bool accumulate) const {
-    rt3_camera cam;
-    std::memset(&cam, 0, sizeof cam);
-    const glm::vec3* src[4] = { &camera.origin, &camera.horizontal, &camera.vertical, &camera.lower_left_corner };
-    float* dst[4] = { cam.origin, cam.horizontal, cam.vertical, cam.lower_left_corner };
-    for (int i = 0; i < 4; i++) { dst[i][0] = src[i]->x; dst[i][1] = src[i]->y; dst[i][2] = src[i]->z; }
+namespace {
+    rt3_camera camera_of(const Camera& camera) {
+        rt3_camera cam;
+        std::memset(&cam, 0, sizeof cam);
+        const glm::vec3* src[4] = { &camera.origin, &camera.horizontal, &camera.vertical, &camera.lower_left_corner };
+        float* dst[4] = { cam.origin, cam.horizontal, cam.vertical, cam.lower_left_corner };
+        for (int i = 0; i < 4; i++) { dst[i][0] = src[i]->x; dst[i][1] = src[i]->y; dst[i][2] = src[i]->z; }
 #ifdef RT3_HOST_CAMERA_CAMERA_HPP /* the thin lens exists only in this repo's Camera, not in the reference's */
-    cam.lens_radius = camera.lens_radius;
-    cam.lens_u[0] = camera.lens_u.x; cam.lens_u[1] = camera.lens_u.y; cam.lens_u[2] = camera.lens_u.z;
-    cam.lens_v[0] = camera.lens_v.x; cam.lens_v[1] = camera.lens_v.y; cam.lens_v[2] = camera.lens_v.z;
+        cam.lens_radius = camera.lens_radius;
+        cam.lens_u[0] = camera.lens_u.x; cam.lens_u[1] = camera.lens_u.y; cam.lens_u[2] = camera.lens_u.z;
+        cam.lens_v[0] = camera.lens_v.x; cam.lens_v[1] = camera.lens_v.y; cam.lens_v[2] = camera.lens_v.z;
 #endif
+        return cam;
+    }
 
+    /* A Portable Float Map of `channels` (3: "PF", 1: "Pf") floats per pixel, little-endian, rows bottom to top. */
+    void write_pfm(const std::string& path, uint32_t width, uint32_t height, uint32_t channels, const float* data) {
+        FILE* f = std::fopen(path.c_str(), "wb");
+        if (!f) { DLOG(fatal, "Could not open '" + path + "' for writing."); }
+        std::fprintf(f, "%s\n%u %u\n-1.0\n", channels == 3 ? "PF" : "Pf", width, height); /* negative scale: little-endian */
+        const size_t row = (size_t) width * channels;
+        bool ok = true;
+        for (uint32_t y = height; y-- > 0 && ok;) { ok = std::fwrite(data + (size_t) y * row, sizeof(float), row, f) == row; }
+        ok = (std::fclose(f) == 0) && ok;
+        if (!ok) { DLOG(fatal, "Could not write '" + path + "'."); }
+    }
+}
+
+rt3_params CudaRenderer::make_params(const Camera& camera, uint32_t first_sample, bool accumulate) const {
     rt3_params params;
     std::memset(&params, 0, sizeof params);
     params.width = camera.w();
@@ -314,6 +331,12 @@ void CudaRenderer::render_samples(Camera& camera, uint32_t first_sample, bool ac
     params.tile_rows = this->settings.tile_rows;
     params.part_index = this->settings.part_index;
     params.part_count = this->settings.part_count;
+    return params;
+}
+
+void CudaRenderer::render_samples(Camera& camera, uint32_t first_sample, bool accumulate) const {
+    const rt3_camera cam = camera_of(camera);
+    const rt3_params params = this->make_params(camera, first_sample, accumulate);
     if (this->helpers.empty()) {
         check(rt3_render(this->ctx, &cam, &params, camera.get_frame().d()), "Render failed");
         check(rt3_get_stats(this->ctx, &this->last_stats), "Could not read render statistics");
@@ -369,13 +392,45 @@ void CudaRenderer::read_radiance(uint32_t width, uint32_t height, std::vector<fl
 void CudaRenderer::write_radiance_pfm(uint32_t width, uint32_t height, const std::string& path) const {
     std::vector<float> rgb;
     this->read_radiance(width, height, rgb);
-    FILE* f = std::fopen(path.c_str(), "wb");
-    if (!f) { DLOG(fatal, "Could not open '" + path + "' for writing."); }
-    std::fprintf(f, "PF\n%u %u\n-1.0\n", width, height); /* negative scale: little-endian */
-    bool ok = true;
-    for (uint32_t y = height; y-- > 0 && ok;) { ok = std::fwrite(rgb.data() + (size_t) y * width * 3, sizeof(float), (size_t) width * 3, f) == (size_t) width * 3; }
-    ok = (std::fclose(f) == 0) && ok;
-    if (!ok) { DLOG(fatal, "Could not write '" + path + "'."); }
+    write_pfm(path, width, height, 3, rgb.data());
+}
+
+void CudaRenderer::render_path_aovs(const Camera& camera, CudaPathAovs& out) const {
+    if (this->settings.mode != RT3_MODE_PATHTRACE) { DLOG(fatal, "Path-traced AOVs need the path-tracing mode."); }
+    const rt3_camera cam = camera_of(camera);
+    rt3_params params = this->make_params(camera, 0, false);
+    if (this->settings.aov_spp) { params.spp = this->settings.aov_spp; }
+    const size_t n = (size_t) params.width * params.height;
+    out.width = params.width; out.height = params.height;
+    out.hit_prim.assign(n, 0u); out.hit_entity.assign(n, 0u); out.hit_t.assign(n, 0.0f); out.albedo.assign(3 * n, 0.0f); out.normal.assign(3 * n, 0.0f);
+    const rt3_path_aovs dst = { out.hit_prim.data(), out.hit_entity.data(), out.hit_t.data(), out.albedo.data(), out.normal.data() };
+    /* one context after the other, each writing its row tiles (the call is blocking) */
+    const uint32_t n_ctx = (uint32_t) this->n_devices();
+    const uint32_t outer = params.part_count ? params.part_count : 1;
+    rt3_stats total;
+    std::memset(&total, 0, sizeof total);
+    for (uint32_t i = 0; i < n_ctx; i++) {
+        rt3_ctx* c = i == 0 ? this->ctx : this->helpers[i - 1];
+        rt3_params mine = params;
+        mine.part_count = outer * n_ctx;
+        mine.part_index = i * outer + params.part_index;
+        check(rt3_render_path_aovs(c, &cam, &mine, &dst), "Path-traced AOVs failed");
+        rt3_stats st;
+        check(rt3_get_stats(c, &st), "Could not read render statistics");
+        if (i == 0) { total = st; continue; }
+        total.rays += st.rays; total.sphere_tests += st.sphere_tests; total.face_tests += st.face_tests;
+        total.accel_node_visits += st.accel_node_visits; total.accel_prim_tests += st.accel_prim_tests;
+        total.rows_rendered += st.rows_rendered; total.kernel_launches += st.kernel_launches;
+        total.device_ms += st.device_ms; total.trace_kernel_ms += st.trace_kernel_ms; /* the contexts ran one after the other */
+    }
+    this->last_stats = total;
+}
+
+void CudaRenderer::write_path_aovs_pfm(const CudaPathAovs& aovs, const std::string& dir) const {
+    const std::string base = dir.empty() ? std::string(".") : dir;
+    write_pfm(base + "/albedo.pfm", aovs.width, aovs.height, 3, aovs.albedo.data());
+    write_pfm(base + "/normal.pfm", aovs.width, aovs.height, 3, aovs.normal.data());
+    write_pfm(base + "/depth.pfm", aovs.width, aovs.height, 1, aovs.hit_t.data());
 }
 
 /* Factory of this backend (reference Renderer.hpp:63; counterpart of SequentialRenderer.cpp:315-323). */

@@ -49,10 +49,18 @@ namespace RayTracer {
         bool device_tessellation = false;   /* build the flattened scene in device memory: ECS spheres are tessellated there (rt3_tessellate_spheres_device),
                                              * the host's triangles / object files are copied next to them, and nothing is derived on the host (rt3_scene_upload_device) */
         uint32_t tile_rows = 8, part_index = 0, part_count = 1;
+        uint32_t aov_spp = 0; /* samples per pixel of render_path_aovs; 0: spp */
         /* Reads RT3_MODE (reference|pathtrace), RT3_SPP, RT3_DEPTH, RT3_SEED, RT3_ANALYTIC_SPHERES, RT3_DEVICE_TESSELLATION, RT3_BVH, RT3_BVH_ABOVE, RT3_DEVICE. */
         static CudaRenderSettings from_environment(int* device);
         /* RT3_DEVICES = comma-separated device ids ("0,1,2,3") or "all"; falls back to the single RT3_DEVICE. */
         static std::vector<int> devices_from_environment();
+    };
+
+    /* AOVs of a path-traced frame (rt3_render_path_aovs): width * height pixels in frame order, albedo and normal 3 floats each. */
+    struct CudaPathAovs {
+        uint32_t width = 0, height = 0;
+        std::vector<uint32_t> hit_prim, hit_entity;
+        std::vector<float> hit_t, albedo, normal;
     };
 
     class CudaRenderer : public Renderer {
@@ -64,6 +72,7 @@ namespace RayTracer {
         std::map<size_t, Material> materials;
         mutable rt3_stats last_stats;
         void render_samples(Camera& camera, uint32_t first_sample, bool accumulate) const;
+        rt3_params make_params(const Camera& camera, uint32_t first_sample, bool accumulate) const;
         void release() noexcept;
 
     public:
@@ -97,6 +106,14 @@ namespace RayTracer {
         void read_radiance(uint32_t width, uint32_t height, std::vector<float>& rgb) const;
         /* The same as a Portable Float Map ("PF", little-endian, rows bottom to top), the float counterpart of Frame::to_ppm. */
         void write_radiance_pfm(uint32_t width, uint32_t height, const std::string& path) const;
+
+        /* AOVs of the path tracer's primary rays for the frame render() would path-trace with these settings (its first
+         * settings.aov_spp samples, or spp): the albedo and normal buffers an image denoiser takes next to the noisy colour,
+         * and per pixel the primitive, entity and distance of the first sample's hit. With several devices every context
+         * renders its row tiles into the same arrays. Leaves the accumulators of render() / render_progressive() alone. */
+        void render_path_aovs(const Camera& camera, CudaPathAovs& out) const;
+        /* albedo.pfm and normal.pfm ("PF", 3 channels) and depth.pfm ("Pf", hit_t; +inf where the primary ray missed) in `dir`. */
+        void write_path_aovs_pfm(const CudaPathAovs& aovs, const std::string& dir) const;
 
         /* Device timings / ray counters of the last render(). */
         const rt3_stats& stats() const { return this->last_stats; }

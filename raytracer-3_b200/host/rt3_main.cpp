@@ -3,9 +3,12 @@
  *
  *   rt3_render [-W width] [-H height] [-s scene] [-o out.ppm|out.png] [--teddy path/to/teddy.obj]
  *              [--pathtrace] [--spp n] [--depth n] [--seed n] [--analytic] [--passes k] [--pfm out.pfm]
+ *              [--aov DIR] [--aov-spp n]
  *   --pathtrace / --spp / --depth / --seed: CudaRenderSettings (default: the reference's ray caster); --analytic keeps
  *   ECS spheres analytic; --passes k renders k progressive passes of spp samples each (render_progressive) and writes
- *   the frame after every pass to <out>.<pass>.<ext>; --pfm also writes the linear float radiance (path tracing only).
+ *   the frame after every pass to <out>.<pass>.<ext>; --pfm also writes the linear float radiance (path tracing only); --aov writes the AOVs of the path tracer's primary
+ *   rays (albedo.pfm, normal.pfm, depth.pfm: what a denoiser takes next to the colour) into DIR, from the first --aov-spp
+ *   samples of every pixel (default: --spp).
  *   scenes: default (reference Main.cpp:280-283, needs --teddy), triangle, sphere, rtiow (path traced, C1),
  *           or the path of a SceneLang file (*.scene)
  */
@@ -26,9 +29,9 @@ using namespace RayTracer;
 
 int main(int argc, const char** argv) {
     uint32_t width = 800, height = 600; /* reference defaults, Main.cpp:78-79 */
-    std::string scene = "triangle", out = "result.ppm", teddy = "bin/objects/teddy.obj", pfm;
+    std::string scene = "triangle", out = "result.ppm", teddy = "bin/objects/teddy.obj", pfm, aov_dir;
     bool pathtrace = false, analytic = false;
-    uint32_t spp = 0, depth = 0, seed = 0, passes = 1;
+    uint32_t spp = 0, depth = 0, seed = 0, passes = 1, aov_spp = 0;
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
         auto next = [&]() -> const char* { if (i + 1 >= argc) { std::fprintf(stderr, "missing value for %s\n", a.c_str()); std::exit(1); } return argv[++i]; };
@@ -43,9 +46,11 @@ int main(int argc, const char** argv) {
         else if (a == "--depth") { depth = (uint32_t) std::strtoul(next(), nullptr, 0); }
         else if (a == "--seed") { seed = (uint32_t) std::strtoul(next(), nullptr, 0); }
         else if (a == "--pfm") { pfm = next(); pathtrace = true; }
+        else if (a == "--aov") { aov_dir = next(); pathtrace = true; }
+        else if (a == "--aov-spp") { aov_spp = (uint32_t) std::strtoul(next(), nullptr, 0); }
         else if (a == "--passes") { passes = (uint32_t) std::strtoul(next(), nullptr, 0); pathtrace = true; }
         else { std::fprintf(stderr, "usage: %s [-W w] [-H h] [-s default|triangle|sphere|rtiow|file.scene] [-o out.ppm|out.png] [--teddy file] "
-                               "[--pathtrace] [--spp n] [--depth n] [--seed n] [--analytic] [--passes k] [--pfm out.pfm]\n", argv[0]); return a == "-h" ? 0 : 1; }
+                               "[--pathtrace] [--spp n] [--depth n] [--seed n] [--analytic] [--passes k] [--pfm out.pfm] [--aov DIR] [--aov-spp n]\n", argv[0]); return a == "-h" ? 0 : 1; }
     }
     try {
         Renderer* renderer = initialize_renderer();
@@ -84,6 +89,7 @@ int main(int argc, const char** argv) {
             if (spp) { st.spp = spp; }
             if (depth) { st.max_depth = depth; }
             if (seed) { st.seed = seed; }
+            st.aov_spp = aov_spp;
             cuda->set_settings(st);
         }
         if (scene == "rtiow") { cam.update(width, height, 1.0f, ((float) width / (float) height) * 2.0f, 2.0f); }
@@ -112,6 +118,13 @@ int main(int argc, const char** argv) {
         if (!pfm.empty()) { cuda->write_radiance_pfm(width, height, pfm); }
         std::printf("%s: %ux%u, %.3f ms on the device, %llu rays -> %s\n", scene.c_str(), width, height, cuda->stats().device_ms,
                     (unsigned long long) cuda->stats().rays, out.c_str());
+        if (!aov_dir.empty()) {
+            CudaPathAovs aovs;
+            cuda->render_path_aovs(cam, aovs);
+            cuda->write_path_aovs_pfm(aovs, aov_dir);
+            std::printf("AOVs: %u samples per pixel, %.3f ms on the device -> %s/{albedo,normal,depth}.pfm\n", cuda->get_settings().aov_spp ? cuda->get_settings().aov_spp : cuda->get_settings().spp,
+                        cuda->stats().device_ms, aov_dir.c_str());
+        }
         delete renderer;
     } catch (CppDebugger::Fatal& e) {
         std::fprintf(stderr, "fatal: %s\n", e.what());
