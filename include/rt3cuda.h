@@ -269,6 +269,26 @@ typedef struct rt3_path_aovs {
  * describes this call (device_ms, trace_kernel_ms, rays = primary rays traced, the test or hierarchy counters). */
 int rt3_render_path_aovs(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, const rt3_path_aovs* out);
 
+/* Parameters of rt3_denoise (defaults: SVGF's, Schied et al. 2017). */
+typedef struct rt3_denoise_params {
+    uint32_t width, height; /* the frame host_frame and host_rgb hold: must be the render's */
+    uint32_t iterations;   /* à-trous passes, 1..8 (default 5: steps 1, 2, 4, 8, 16, a reach of 64 pixels) */
+    float sigma_luminance; /* luminance edge-stopping, finite and > 0 (default 4) */
+    float sigma_normal;    /* exponent of the normal term, a whole number in 1..1024 (default 128) */
+    float sigma_depth;     /* relative depth edge-stopping, finite and > 0 (default 1) */
+} rt3_denoise_params;
+
+/* Denoises the last path-traced render on this context: an edge-avoiding à-trous wavelet filter (the spatial filter of
+ * SVGF) on its radiance (bit-equal to rt3_read_radiance), divided by the albedo and guided by the normal and depth of the
+ * last rt3_render_path_aovs on this context; the result is multiplied by the albedo again and resolved like the render's
+ * frame (gamma 2 unless the render had RT3_FLAG_NO_GAMMA, 8-bit pack). The formulas are in include/rt3_denoise.h and
+ * DESIGN.md 3.8. Needs both calls to cover the whole frame (part_count <= 1) with the same width, height, camera and
+ * scene upload; otherwise RT3_ERR_INVALID, with a message that names the condition, and nothing changes. Writes
+ * width*height packed pixels to host_frame and 3 linear floats per pixel to host_rgb; either may be NULL. Blocking. The
+ * accumulators, the AOV buffers and the RT3_FLAG_ACCUMULATE state are not touched. rt3_get_stats then describes this
+ * call (device_ms, kernel_launches, rays = 0). */
+int rt3_denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb);
+
 /* Device-resident variant for multi-GPU plumbing: renders this partition's
  * rows into `device_frame` (a device pointer to width*height uint32, full-frame
  * indexing) asynchronously on `cuda_stream` (a cudaStream_t; NULL = the

@@ -93,6 +93,16 @@ class PathAovs(C.Structure):
     _fields_ = [("hit_prim", C.c_void_p), ("hit_entity", C.c_void_p), ("hit_t", C.c_void_p), ("albedo", C.c_void_p), ("normal", C.c_void_p)]
 
 
+class DenoiseParams(C.Structure):
+    """rt3_denoise_params."""
+    _fields_ = [("width", C.c_uint32), ("height", C.c_uint32), ("iterations", C.c_uint32), ("sigma_luminance", C.c_float), ("sigma_normal", C.c_float), ("sigma_depth", C.c_float)]
+
+
+def denoise_params(width=0, height=0, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
+    """rt3_denoise_params with SVGF's defaults."""
+    return DenoiseParams(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
+
+
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
@@ -223,6 +233,7 @@ def load_core():
     lib.rt3_uv_sphere_vertices.restype = u32
     lib.rt3_tessellate_spheres.argtypes = [vp, C.POINTER(UvSphere), u32, u32, vp, vp, vp]
     lib.rt3_read_radiance.argtypes = [vp, vp, u32, u32]
+    lib.rt3_denoise.argtypes = [vp, C.POINTER(DenoiseParams), vp, vp]
     lib.rt3_get_stats.argtypes = [vp, C.POINTER(Stats)]
     lib.rt3_measure_fma_peak.argtypes = [vp, C.POINTER(C.c_double)]
     _core = lib
@@ -236,7 +247,7 @@ EXPORTED_SYMBOLS = [
     "rt3_frame_alloc", "rt3_frame_free", "rt3_frame_export", "rt3_frame_import", "rt3_frame_release",
     "rt3_frame_attach", "rt3_frame_read",
     "rt3_uv_sphere_faces", "rt3_uv_sphere_vertices", "rt3_tessellate_spheres",
-    "rt3_read_radiance", "rt3_get_stats", "rt3_measure_fma_peak",
+    "rt3_read_radiance", "rt3_denoise", "rt3_get_stats", "rt3_measure_fma_peak",
 ]
 
 
@@ -409,6 +420,15 @@ class Context:
         out = np.zeros((height, width, 3), np.float32)
         self._check(self.lib.rt3_read_radiance(self.handle, _ptr(out), width, height))
         return out
+
+    def denoise(self, width, height, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
+        """rt3_denoise: the last path-traced render of this (width x height) frame, filtered under the guidance of the last
+        render_path_aovs. Returns (frame [H, W] uint32 packed like render's, rgb [H, W, 3] float32 linear)."""
+        frame = np.zeros((height, width), np.uint32)
+        rgb = np.zeros((height, width, 3), np.float32)
+        p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
+        self._check(self.lib.rt3_denoise(self.handle, C.byref(p), _ptr(frame), _ptr(rgb)))
+        return frame, rgb
 
     def stats(self):
         st = Stats()

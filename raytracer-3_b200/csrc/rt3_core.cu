@@ -26,6 +26,7 @@
 #include <cub/device/device_radix_sort.cuh>
 
 #include "rt3_kernels.cuh"
+#include "rt3_denoise.cuh"
 #include "rt3_scene.cuh"
 #include "rt3_upload.cuh"
 
@@ -120,6 +121,20 @@ struct rt3_ctx {
     uint32_t accum_width = 0, accum_height = 0; /* frame the accumulators were last cleared for */
     rt3_kparams accum_kp{};                      /* the path-traced render the accumulators currently hold */
     bool accum_valid = false;
+    rt3_camera accum_cam{};                      /* its camera (rt3_denoise) ... */
+    bool accum_cam_mixed = false;                /* ... unless an accumulating pass used another one */
+
+    /* the last rt3_render_path_aovs, whose albedo, normal and depth (aov_t) guide rt3_denoise */
+    bool path_aovs_valid = false;
+    rt3_kparams path_aovs_kp{};
+    rt3_camera path_aovs_cam{};
+    uint64_t path_aovs_scene_id = 0;
+
+    /* rt3_denoise: ping-pong filter state, guides and outputs, sized on first use */
+    DeviceBuffer<rt3_dn_px> dn_col[2];
+    DeviceBuffer<rt3_dn_guide> dn_guide;
+    DeviceBuffer<float> dn_rgb;
+    DeviceBuffer<uint32_t> dn_frame;
 
     rt3_stats stats{};
     double upload_ms = 0.0, upload_h2d_ms = 0.0, upload_device_ms = 0.0; /* most recent scene upload */
@@ -449,6 +464,8 @@ int enqueue_render(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params
     ctx->stats.kernel_launches = accumulate ? 2 : 3;
     ctx->accum_kp = kp;
     ctx->accum_valid = true;
+    if (!accumulate) { ctx->accum_cam = *cam; ctx->accum_cam_mixed = false; }
+    else if (memcmp(&ctx->accum_cam, cam, sizeof *cam) != 0) { ctx->accum_cam_mixed = true; }
     return RT3_OK;
 }
 
@@ -495,7 +512,11 @@ int render_to_host(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params
     if (want_aov) {
         if (host_prim) { if ((rc = ctx->aov_prim.reserve(n)) != RT3_OK) { return rc; } d_prim = ctx->aov_prim.ptr; }
         if (host_ent) { if ((rc = ctx->aov_entity.reserve(n)) != RT3_OK) { return rc; } d_ent = ctx->aov_entity.ptr; }
-        if (host_t) { if ((rc = ctx->aov_t.reserve(n)) != RT3_OK) { return rc; } d_t = ctx->aov_t.ptr; }
+        if (host_t) {
+            ctx->path_aovs_valid = false; /* the depth buffer is the path-traced AOVs' too */
+            if ((rc = ctx->aov_t.reserve(n)) != RT3_OK) { return rc; }
+            d_t = ctx->aov_t.ptr;
+        }
     }
     rc = enqueue_render(ctx, cam, params, kp, ctx->frame.ptr, d_prim, d_ent, d_t, ctx->stream);
     if (rc != RT3_OK) { return rc; }
@@ -524,11 +545,15 @@ int render_path_aovs(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* para
     if (rc != RT3_OK) { return rc; }
     const size_t n = (size_t) kp.width * kp.height;
     uint32_t *d_prim = nullptr, *d_ent = nullptr;
-    float* d_t = nullptr;
-    if ((rc = ctx->aov_sums.reserve(RT3_AOV_SUMS * n)) != RT3_OK || (rc = ctx->aov_albedo.reserve(3 * n)) != RT3_OK || (rc = ctx->aov_normal.reserve(3 * n)) != RT3_OK) { return rc; }
+    ctx->path_aovs_valid = false;
+    /* depth is kept on the device even when the caller does not want it: it guides rt3_denoise */
+    if ((rc = ctx->aov_sums.reserve(RT3_AOV_SUMS * n)) != RT3_OK || (rc = ctx->aov_albedo.reserve(3 * n)) != RT3_OK ||
+        (rc = ctx->aov_normal.reserve(3 * n)) != RT3_OK || (rc = ctx->aov_t.reserve(n)) != RT3_OK) {
+        return rc;
+    }
+    float* d_t = ctx->aov_t.ptr;
     if (out->hit_prim) { if ((rc = ctx->aov_prim.reserve(n)) != RT3_OK) { return rc; } d_prim = ctx->aov_prim.ptr; }
     if (out->hit_entity) { if ((rc = ctx->aov_entity.reserve(n)) != RT3_OK) { return rc; } d_ent = ctx->aov_entity.ptr; }
-    if (out->hit_t) { if ((rc = ctx->aov_t.reserve(n)) != RT3_OK) { return rc; } d_t = ctx->aov_t.ptr; }
     cudaStream_t stream = ctx->stream;
     bool resident = false;
     size_t smem = render_smem_bytes(ctx->view, false, &resident);
@@ -573,7 +598,7 @@ int render_path_aovs(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* para
     RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
     if (d_prim && (rc = copy_owned_rows(kp, d_prim, out->hit_prim, stream)) != RT3_OK) { return rc; }
     if (d_ent && (rc = copy_owned_rows(kp, d_ent, out->hit_entity, stream)) != RT3_OK) { return rc; }
-    if (d_t && (rc = copy_owned_rows(kp, d_t, out->hit_t, stream)) != RT3_OK) { return rc; }
+    if (out->hit_t && (rc = copy_owned_rows(kp, d_t, out->hit_t, stream)) != RT3_OK) { return rc; }
     /* three floats per pixel: rows of float3 */
     if (out->albedo && (rc = copy_owned_rows(kp, reinterpret_cast<const float3*>(ctx->aov_albedo.ptr), reinterpret_cast<float3*>(out->albedo), stream)) != RT3_OK) { return rc; }
     if (out->normal && (rc = copy_owned_rows(kp, reinterpret_cast<const float3*>(ctx->aov_normal.ptr), reinterpret_cast<float3*>(out->normal), stream)) != RT3_OK) { return rc; }
@@ -582,7 +607,81 @@ int render_path_aovs(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* para
     RT3_CUDA(cudaStreamSynchronize(stream));
     rc = collect_stats(ctx);
     if (radiance_stream) { ctx->last_stream = radiance_stream; } /* rt3_read_radiance stays behind the render that filled the accumulators */
+    if (rc == RT3_OK) {
+        ctx->path_aovs_valid = true;
+        ctx->path_aovs_kp = kp;
+        ctx->path_aovs_cam = *cam;
+        ctx->path_aovs_scene_id = ctx->scene_id;
+    }
     return rc;
+}
+
+/* rt3_denoise: prepare, variance and `iterations` à-trous passes over the accumulators and the path-traced AOVs, on the
+ * stream rt3_read_radiance orders itself behind (the one of the render that filled the accumulators), blocking. Reads the
+ * accumulators and the AOV buffers and writes only the dn_* buffers; every condition is checked before anything changes. */
+int denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb) {
+    if (!ctx) { return fail(RT3_ERR_INVALID, "ctx is NULL"); }
+    if (const char* why = rt3_dn_check_params(params)) { return fail(RT3_ERR_INVALID, "rt3_denoise: %s", why); }
+    if (!ctx->accum_valid) { return fail(RT3_ERR_INVALID, "rt3_denoise needs a path-traced render on this context"); }
+    const rt3_kparams& kp = ctx->accum_kp;
+    if (params->width != kp.width || params->height != kp.height) {
+        return fail(RT3_ERR_INVALID, "rt3_denoise: the last path-traced frame was %ux%u, not %ux%u", kp.width, kp.height, params->width, params->height);
+    }
+    if (kp.part_count > 1) { return fail(RT3_ERR_INVALID, "rt3_denoise: the path-traced render covers part %u of %u of the frame, not all of it", kp.part_index, kp.part_count); }
+    if (ctx->accum_cam_mixed) { return fail(RT3_ERR_INVALID, "rt3_denoise: the accumulated render's passes used different cameras"); }
+    if (!ctx->path_aovs_valid) { return fail(RT3_ERR_INVALID, "rt3_denoise needs an rt3_render_path_aovs on this context (after any rt3_render_aov with hit_t)"); }
+    const rt3_kparams& ak = ctx->path_aovs_kp;
+    if (ak.part_count > 1) { return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs cover part %u of %u of the frame, not all of it", ak.part_index, ak.part_count); }
+    if (ak.width != kp.width || ak.height != kp.height) {
+        return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs are %ux%u, the render %ux%u", ak.width, ak.height, kp.width, kp.height);
+    }
+    if (memcmp(&ctx->path_aovs_cam, &ctx->accum_cam, sizeof(rt3_camera)) != 0) { return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs and the render used different cameras"); }
+    if (!ctx->has_scene || ctx->path_aovs_scene_id != ctx->scene_id) { return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs were rendered from another scene upload than the render"); }
+    RT3_CUDA(cudaSetDevice(ctx->device));
+    const size_t n = (size_t) kp.width * kp.height;
+    int rc;
+    if ((rc = ctx->dn_col[0].reserve(n)) != RT3_OK || (rc = ctx->dn_col[1].reserve(n)) != RT3_OK || (rc = ctx->dn_guide.reserve(n)) != RT3_OK ||
+        (rc = ctx->dn_frame.reserve(n)) != RT3_OK || (host_rgb && (rc = ctx->dn_rgb.reserve(3 * n)) != RT3_OK)) {
+        return rc;
+    }
+    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
+    const uint32_t w = kp.width, h = kp.height, n_pow = (uint32_t) params->sigma_normal;
+    const float sigma_l = params->sigma_luminance, sigma_z = params->sigma_depth;
+    const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid((w + RT3_DN_BLOCK_X - 1) / RT3_DN_BLOCK_X, (h + RT3_DN_BLOCK_Y - 1) / RT3_DN_BLOCK_Y);
+    ctx->stats.accel = 0;
+    ctx->stats_beam = false; ctx->stats_beam_accel = false;
+    ctx->stats.rows_rendered = h;
+    ctx->stats_pending = true;
+    ctx->copy_timed = false;
+    RT3_CUDA(cudaEventRecord(ctx->ev_begin, stream));
+    RT3_CUDA(cudaMemsetAsync(ctx->counters.ptr, 0, 8 * sizeof(unsigned long long), stream));
+    RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
+    denoise_prepare_kernel<<<(unsigned) ((n + 255) / 256), 256, 0, stream>>>(kp, ctx->accum.ptr, ctx->aov_albedo.ptr, ctx->aov_normal.ptr, ctx->aov_t.ptr,
+                                                                           ctx->dn_col[1].ptr, ctx->dn_guide.ptr);
+    RT3_CUDA(cudaGetLastError());
+    denoise_variance_kernel<<<grid, block, 0, stream>>>(w, h, sigma_z, n_pow, ctx->dn_col[1].ptr, ctx->dn_guide.ptr, ctx->dn_col[0].ptr);
+    RT3_CUDA(cudaGetLastError());
+    const bool gamma = !(kp.flags & RT3_FLAG_NO_GAMMA);
+    for (uint32_t i = 0; i < params->iterations; i++) {
+        const rt3_dn_px* in = ctx->dn_col[i & 1u].ptr;
+        rt3_dn_px* out = ctx->dn_col[(i + 1u) & 1u].ptr;
+        if (i + 1u < params->iterations) {
+            denoise_atrous_kernel<false><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, ctx->dn_guide.ptr, out, nullptr, gamma, nullptr, nullptr);
+        } else {
+            denoise_atrous_kernel<true><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, ctx->dn_guide.ptr, nullptr, ctx->aov_albedo.ptr, gamma,
+                                                                    ctx->dn_frame.ptr, host_rgb ? ctx->dn_rgb.ptr : nullptr);
+        }
+        RT3_CUDA(cudaGetLastError());
+    }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k1, stream));
+    RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
+    ctx->stats.kernel_launches = 2 + params->iterations;
+    if (host_frame) { RT3_CUDA(cudaMemcpyAsync(host_frame, ctx->dn_frame.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream)); }
+    if (host_rgb) { RT3_CUDA(cudaMemcpyAsync(host_rgb, ctx->dn_rgb.ptr, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, stream)); }
+    RT3_CUDA(cudaEventRecord(ctx->ev_copy, stream));
+    ctx->copy_timed = true;
+    RT3_CUDA(cudaStreamSynchronize(stream));
+    return collect_stats(ctx);
 }
 
 /* Reads back the timings and counters of the most recent render (synchronises its stream). */
@@ -799,6 +898,7 @@ int rt3_destroy(rt3_ctx* ctx) {
     ctx->spheres.release(); ctx->prim_color.release(); ctx->materials.release(); ctx->prim_material.release(); ctx->prim_entity.release();
     ctx->frame.release(); ctx->aov_prim.release(); ctx->aov_entity.release(); ctx->aov_t.release(); ctx->accum.release(); ctx->counters.release();
     ctx->aov_sums.release(); ctx->aov_albedo.release(); ctx->aov_normal.release();
+    ctx->dn_col[0].release(); ctx->dn_col[1].release(); ctx->dn_guide.release(); ctx->dn_rgb.release(); ctx->dn_frame.release();
     if (ctx->ev_begin) { cudaEventDestroy(ctx->ev_begin); }
     if (ctx->ev_end) { cudaEventDestroy(ctx->ev_end); }
     if (ctx->ev_copy) { cudaEventDestroy(ctx->ev_copy); }
@@ -903,6 +1003,10 @@ int rt3_render_aov(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* par
 
 int rt3_render_path_aovs(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, const rt3_path_aovs* out) {
     return render_path_aovs(ctx, camera, params, out);
+}
+
+int rt3_denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb) {
+    return denoise(ctx, params, host_frame, host_rgb);
 }
 
 int rt3_render_device(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, uint32_t* device_frame, void* cuda_stream) {

@@ -1,0 +1,67 @@
+/* rt3_denoise.cuh — kernels of rt3_denoise (DESIGN.md 3.8): the edge-avoiding à-trous filter on the radiance of the last
+ * path-traced render, guided by the last path-traced AOVs. The arithmetic is include/rt3_denoise.h's; these kernels only
+ * load, call it and store. Every kernel covers the whole frame (rt3_denoise needs part_count <= 1), one thread per pixel.
+ *
+ *   denoise_prepare_kernel   : radiance (radiance_kernel's expression) / albedo -> colour + luminance, normal + depth -> guide.
+ *   denoise_variance_kernel  : 7x7 luminance variance.
+ *   denoise_atrous_kernel<F> : one 5x5 pass at step 2^i; F = the last pass, which remodulates and resolves like resolve_kernel.
+ *
+ * Taps are read straight from global memory through L1 (float4 loads): a 2^i-strided 5x5 footprint is 25 float4 of colour
+ * and 25 of guide, all but the far ones shared with the neighbouring threads of the CTA. */
+#pragma once
+
+#include "rt3_denoise.h"
+#include "rt3_device.cuh"
+
+#define RT3_DN_BLOCK_X 32
+#define RT3_DN_BLOCK_Y 8
+
+__global__ void __launch_bounds__(256) denoise_prepare_kernel(rt3_kparams P, const unsigned long long* __restrict__ accum, const float* __restrict__ albedo,
+                                                             const float* __restrict__ normal, const float* __restrict__ depth, rt3_dn_px* __restrict__ col,
+                                                             rt3_dn_guide* __restrict__ guide) {
+    const unsigned long long idx = (unsigned long long) blockIdx.x * blockDim.x + threadIdx.x;
+    if (idx >= P.n_pixels) { return; }
+    float c[3], a[3], n[3];
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        c[k] = (float) ((double) accum[3 * idx + k] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE));
+        a[k] = albedo[3 * idx + k];
+        n[k] = normal[3 * idx + k];
+    }
+    rt3_dn_px px;
+    rt3_dn_guide g;
+    rt3_dn_prepare_px(c, a, n, depth[idx], &px, &g);
+    col[idx] = px;
+    guide[idx] = g;
+}
+
+__global__ void __launch_bounds__(RT3_DN_BLOCK_X * RT3_DN_BLOCK_Y) denoise_variance_kernel(uint32_t w, uint32_t h, float sigma_z, uint32_t n_pow,
+                                                                                         const rt3_dn_px* __restrict__ col, const rt3_dn_guide* __restrict__ guide,
+                                                                                         rt3_dn_px* __restrict__ out) {
+    const uint32_t x = blockIdx.x * RT3_DN_BLOCK_X + threadIdx.x, y = blockIdx.y * RT3_DN_BLOCK_Y + threadIdx.y;
+    if (x >= w || y >= h) { return; }
+    const size_t p = (size_t) y * w + x;
+    rt3_dn_px px = col[p];
+    px.v = rt3_dn_variance_px(col, guide, w, h, x, y, sigma_z, n_pow);
+    out[p] = px;
+}
+
+template <bool FINAL>
+__global__ void __launch_bounds__(RT3_DN_BLOCK_X * RT3_DN_BLOCK_Y) denoise_atrous_kernel(uint32_t w, uint32_t h, uint32_t step, float sigma_l, float sigma_z,
+                                                                                       uint32_t n_pow, const rt3_dn_px* __restrict__ col,
+                                                                                       const rt3_dn_guide* __restrict__ guide, rt3_dn_px* __restrict__ out,
+                                                                                       const float* __restrict__ albedo, bool gamma, uint32_t* __restrict__ frame,
+                                                                                       float* __restrict__ rgb) {
+    const uint32_t x = blockIdx.x * RT3_DN_BLOCK_X + threadIdx.x, y = blockIdx.y * RT3_DN_BLOCK_Y + threadIdx.y;
+    if (x >= w || y >= h) { return; }
+    const size_t p = (size_t) y * w + x;
+    const rt3_dn_px f = rt3_dn_atrous_px(col, guide, w, h, x, y, step, sigma_l, sigma_z, n_pow);
+    if (!FINAL) {
+        out[p] = f;
+        return;
+    }
+    const float r = rt3_dn_remodulate(f.r, albedo[3 * p]), g = rt3_dn_remodulate(f.g, albedo[3 * p + 1]), b = rt3_dn_remodulate(f.b, albedo[3 * p + 2]);
+    if (rgb) { rgb[3 * p] = r; rgb[3 * p + 1] = g; rgb[3 * p + 2] = b; }
+    frame[p] = gamma ? (unorm8(sqrtf(r)) << 24) | (unorm8(sqrtf(g)) << 16) | (unorm8(sqrtf(b)) << 8) | 0xFFu
+                     : (unorm8(r) << 24) | (unorm8(g) << 16) | (unorm8(b) << 8) | 0xFFu;
+}

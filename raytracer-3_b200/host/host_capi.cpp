@@ -216,6 +216,20 @@ int rt3host_path_aovs(void* s, uint32_t width, uint32_t height, float focal, flo
         if (dir) { hs->renderer->write_path_aovs_pfm(aovs, dir); }
     });
 }
+/* CudaRenderer::denoise with the reference camera (frame_out: width * height words, rgb_out: width * height * 3 floats; either may be NULL). */
+int rt3host_denoise(void* s, uint32_t width, uint32_t height, float focal, float vw, float vh, const rt3_denoise_params* p, uint32_t* frame_out, float* rgb_out) {
+    HostScene* hs = (HostScene*) s;
+    if (!hs->renderer) { g_error = "create the renderer first"; return -1; }
+    return guarded([&] {
+        hs->camera.update(width, height, focal, vw, vh);
+        CudaDenoiseSettings st;
+        st.iterations = p->iterations; st.sigma_luminance = p->sigma_luminance; st.sigma_normal = p->sigma_normal; st.sigma_depth = p->sigma_depth;
+        std::vector<float> rgb;
+        hs->renderer->denoise(hs->camera, st, rgb_out ? &rgb : nullptr);
+        if (frame_out) { std::memcpy(frame_out, hs->camera.get_frame().d(), (size_t) width * height * sizeof(uint32_t)); }
+        if (rgb_out) { std::memcpy(rgb_out, rgb.data(), rgb.size() * sizeof(float)); }
+    });
+}
 int rt3host_camera_vectors(uint32_t width, uint32_t height, const float* look, float* out19) {
     return guarded([&] {
         Camera cam;

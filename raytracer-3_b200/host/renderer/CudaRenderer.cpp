@@ -426,6 +426,21 @@ void CudaRenderer::render_path_aovs(const Camera& camera, CudaPathAovs& out) con
     this->last_stats = total;
 }
 
+void CudaRenderer::denoise(Camera& camera, const CudaDenoiseSettings& settings, std::vector<float>* rgb) const {
+    if (!this->helpers.empty()) {
+        DLOG(fatal, "Denoising needs a renderer on one device: with " + std::to_string(this->n_devices()) +
+                    " each context holds only its own rows of the frame, and the filter reaches across them.");
+    }
+    rt3_denoise_params params;
+    std::memset(&params, 0, sizeof params);
+    params.width = camera.w(); params.height = camera.h();
+    params.iterations = settings.iterations;
+    params.sigma_luminance = settings.sigma_luminance; params.sigma_normal = settings.sigma_normal; params.sigma_depth = settings.sigma_depth;
+    if (rgb) { rgb->assign((size_t) params.width * params.height * 3, 0.0f); }
+    check(rt3_denoise(this->ctx, &params, camera.get_frame().d(), rgb ? rgb->data() : nullptr), "Denoising failed");
+    check(rt3_get_stats(this->ctx, &this->last_stats), "Could not read the statistics");
+}
+
 void CudaRenderer::write_path_aovs_pfm(const CudaPathAovs& aovs, const std::string& dir) const {
     const std::string base = dir.empty() ? std::string(".") : dir;
     write_pfm(base + "/albedo.pfm", aovs.width, aovs.height, 3, aovs.albedo.data());

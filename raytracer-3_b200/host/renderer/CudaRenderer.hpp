@@ -63,6 +63,12 @@ namespace RayTracer {
         std::vector<float> hit_t, albedo, normal;
     };
 
+    /* Parameters of CudaRenderer::denoise (rt3_denoise_params; SVGF's defaults). */
+    struct CudaDenoiseSettings {
+        uint32_t iterations = 5;
+        float sigma_luminance = 4.0f, sigma_normal = 128.0f, sigma_depth = 1.0f;
+    };
+
     class CudaRenderer : public Renderer {
         rt3_ctx* ctx;                 /* first device: owns the frame when there are several */
         std::vector<rt3_ctx*> helpers; /* further devices (SURVEY 8e): each renders its row tiles straight into ctx's frame */
@@ -112,6 +118,11 @@ namespace RayTracer {
          * and per pixel the primitive, entity and distance of the first sample's hit. With several devices every context
          * renders its row tiles into the same arrays. Leaves the accumulators of render() / render_progressive() alone. */
         void render_path_aovs(const Camera& camera, CudaPathAovs& out) const;
+        /* Denoises the last render() / render_progressive() of this camera's frame (rt3_denoise), guided by the last
+         * render_path_aovs() with the same camera, and writes the result into the camera's frame; `rgb`, when given, receives
+         * the linear float image (3 per pixel). One device only: each context of a renderer with several holds only its own
+         * rows, and the filter reaches across them. */
+        void denoise(Camera& camera, const CudaDenoiseSettings& settings = {}, std::vector<float>* rgb = nullptr) const;
         /* albedo.pfm and normal.pfm ("PF", 3 channels) and depth.pfm ("Pf", hit_t; +inf where the primary ray missed) in `dir`. */
         void write_path_aovs_pfm(const CudaPathAovs& aovs, const std::string& dir) const;
 

@@ -3,12 +3,13 @@
  *
  *   rt3_render [-W width] [-H height] [-s scene] [-o out.ppm|out.png] [--teddy path/to/teddy.obj]
  *              [--pathtrace] [--spp n] [--depth n] [--seed n] [--analytic] [--passes k] [--pfm out.pfm]
- *              [--aov DIR] [--aov-spp n]
+ *              [--aov DIR] [--aov-spp n] [--denoise]
  *   --pathtrace / --spp / --depth / --seed: CudaRenderSettings (default: the reference's ray caster); --analytic keeps
  *   ECS spheres analytic; --passes k renders k progressive passes of spp samples each (render_progressive) and writes
  *   the frame after every pass to <out>.<pass>.<ext>; --pfm also writes the linear float radiance (path tracing only); --aov writes the AOVs of the path tracer's primary
  *   rays (albedo.pfm, normal.pfm, depth.pfm: what a denoiser takes next to the colour) into DIR, from the first --aov-spp
- *   samples of every pixel (default: --spp).
+ *   samples of every pixel (default: --spp); --denoise runs that AOV pass too and writes the frame denoised by it
+ *   (CudaRenderer::denoise: edge-avoiding à-trous filter, SVGF's defaults) to <out> instead of the noisy one.
  *   scenes: default (reference Main.cpp:280-283, needs --teddy), triangle, sphere, rtiow (path traced, C1),
  *           or the path of a SceneLang file (*.scene)
  */
@@ -30,7 +31,7 @@ using namespace RayTracer;
 int main(int argc, const char** argv) {
     uint32_t width = 800, height = 600; /* reference defaults, Main.cpp:78-79 */
     std::string scene = "triangle", out = "result.ppm", teddy = "bin/objects/teddy.obj", pfm, aov_dir;
-    bool pathtrace = false, analytic = false;
+    bool pathtrace = false, analytic = false, denoise = false;
     uint32_t spp = 0, depth = 0, seed = 0, passes = 1, aov_spp = 0;
     for (int i = 1; i < argc; i++) {
         std::string a = argv[i];
@@ -48,9 +49,10 @@ int main(int argc, const char** argv) {
         else if (a == "--pfm") { pfm = next(); pathtrace = true; }
         else if (a == "--aov") { aov_dir = next(); pathtrace = true; }
         else if (a == "--aov-spp") { aov_spp = (uint32_t) std::strtoul(next(), nullptr, 0); }
+        else if (a == "--denoise") { denoise = true; pathtrace = true; }
         else if (a == "--passes") { passes = (uint32_t) std::strtoul(next(), nullptr, 0); pathtrace = true; }
         else { std::fprintf(stderr, "usage: %s [-W w] [-H h] [-s default|triangle|sphere|rtiow|file.scene] [-o out.ppm|out.png] [--teddy file] "
-                               "[--pathtrace] [--spp n] [--depth n] [--seed n] [--analytic] [--passes k] [--pfm out.pfm] [--aov DIR] [--aov-spp n]\n", argv[0]); return a == "-h" ? 0 : 1; }
+                               "[--pathtrace] [--spp n] [--depth n] [--seed n] [--analytic] [--passes k] [--pfm out.pfm] [--aov DIR] [--aov-spp n] [--denoise]\n", argv[0]); return a == "-h" ? 0 : 1; }
     }
     try {
         Renderer* renderer = initialize_renderer();
@@ -114,16 +116,21 @@ int main(int argc, const char** argv) {
             else if (entities[i]->type == ECS::et_sphere) { delete (ECS::Sphere*) entities[i]; }
             else { delete (ECS::Triangle*) entities[i]; }
         }
-        save(cam.get_frame(), out);
+        if (!denoise) { save(cam.get_frame(), out); }
         if (!pfm.empty()) { cuda->write_radiance_pfm(width, height, pfm); }
         std::printf("%s: %ux%u, %.3f ms on the device, %llu rays -> %s\n", scene.c_str(), width, height, cuda->stats().device_ms,
-                    (unsigned long long) cuda->stats().rays, out.c_str());
-        if (!aov_dir.empty()) {
+                    (unsigned long long) cuda->stats().rays, denoise ? "denoiser" : out.c_str());
+        if (!aov_dir.empty() || denoise) {
             CudaPathAovs aovs;
             cuda->render_path_aovs(cam, aovs);
-            cuda->write_path_aovs_pfm(aovs, aov_dir);
-            std::printf("AOVs: %u samples per pixel, %.3f ms on the device -> %s/{albedo,normal,depth}.pfm\n", cuda->get_settings().aov_spp ? cuda->get_settings().aov_spp : cuda->get_settings().spp,
-                        cuda->stats().device_ms, aov_dir.c_str());
+            if (!aov_dir.empty()) { cuda->write_path_aovs_pfm(aovs, aov_dir); }
+            std::printf("AOVs: %u samples per pixel, %.3f ms on the device -> %s\n", cuda->get_settings().aov_spp ? cuda->get_settings().aov_spp : cuda->get_settings().spp,
+                        cuda->stats().device_ms, aov_dir.empty() ? "denoiser" : (aov_dir + "/{albedo,normal,depth}.pfm").c_str());
+        }
+        if (denoise) {
+            cuda->denoise(cam);
+            save(cam.get_frame(), out);
+            std::printf("denoised: %u kernels, %.3f ms on the device -> %s\n", cuda->stats().kernel_launches, cuda->stats().device_ms, out.c_str());
         }
         delete renderer;
     } catch (CppDebugger::Fatal& e) {
