@@ -314,6 +314,31 @@ namespace {
         ok = (std::fclose(f) == 0) && ok;
         if (!ok) { DLOG(fatal, "Could not write '" + path + "'."); }
     }
+
+    /* `params` for context i of n: the frame's row tiles are dealt round-robin over the contexts, within this process's own part
+     * of a larger split (tile % (outer n) == i outer + p  implies  tile % outer == p). */
+    rt3_params context_part(const rt3_params& params, uint32_t i, uint32_t n) {
+        const uint32_t outer = params.part_count ? params.part_count : 1;
+        rt3_params mine = params;
+        mine.part_count = outer * n;
+        mine.part_index = i * outer + params.part_index;
+        return mine;
+    }
+
+    /* Adds one context's statistics to a total: counts add up; times are the longest one when the contexts ran concurrently,
+     * their sum when they ran one after the other. */
+    void add_stats(rt3_stats& total, const rt3_stats& st, bool concurrent) {
+        total.rays += st.rays; total.sphere_tests += st.sphere_tests; total.face_tests += st.face_tests;
+        total.accel_node_visits += st.accel_node_visits; total.accel_prim_tests += st.accel_prim_tests;
+        total.beam_rays += st.beam_rays; total.beam_tests += st.beam_tests;
+        total.rows_rendered += st.rows_rendered; total.kernel_launches += st.kernel_launches;
+        if (concurrent) {
+            if (st.device_ms > total.device_ms) { total.device_ms = st.device_ms; }
+            if (st.trace_kernel_ms > total.trace_kernel_ms) { total.trace_kernel_ms = st.trace_kernel_ms; }
+        } else {
+            total.device_ms += st.device_ms; total.trace_kernel_ms += st.trace_kernel_ms;
+        }
+    }
 }
 
 rt3_params CudaRenderer::make_params(const Camera& camera, uint32_t first_sample, bool accumulate) const {
@@ -352,11 +377,8 @@ void CudaRenderer::render_samples(Camera& camera, uint32_t first_sample, bool ac
         this->shared_pixels = n_pixels;
     }
     const uint32_t n = (uint32_t) this->n_devices();
-    const uint32_t outer = params.part_count ? params.part_count : 1; /* this process may itself be one part of a larger split */
     for (uint32_t i = 0; i < n; i++) {
-        rt3_params mine = params;
-        mine.part_count = outer * n;
-        mine.part_index = i * outer + params.part_index; /* tile % (outer n) == i outer + p  implies  tile % outer == p */
+        const rt3_params mine = context_part(params, i, n);
         check(rt3_render_device(i == 0 ? this->ctx : this->helpers[i - 1], &cam, &mine, this->shared_frame, nullptr), "Render failed");
     }
     rt3_stats total;
@@ -364,13 +386,7 @@ void CudaRenderer::render_samples(Camera& camera, uint32_t first_sample, bool ac
     for (uint32_t i = 0; i < n; i++) {
         rt3_stats st;
         check(rt3_get_stats(i == 0 ? this->ctx : this->helpers[i - 1], &st), "Could not read render statistics");
-        if (i == 0) { total = st; continue; }
-        total.rays += st.rays; total.sphere_tests += st.sphere_tests; total.face_tests += st.face_tests;
-        total.accel_node_visits += st.accel_node_visits; total.accel_prim_tests += st.accel_prim_tests;
-        total.beam_rays += st.beam_rays; total.beam_tests += st.beam_tests;
-        total.rows_rendered += st.rows_rendered; total.kernel_launches += st.kernel_launches;
-        if (st.device_ms > total.device_ms) { total.device_ms = st.device_ms; }
-        if (st.trace_kernel_ms > total.trace_kernel_ms) { total.trace_kernel_ms = st.trace_kernel_ms; }
+        if (i == 0) { total = st; } else { add_stats(total, st, true); }
     }
     check(rt3_frame_read(this->ctx, this->shared_frame, camera.get_frame().d(), n_pixels), "Could not read the frame");
     this->last_stats = total;
@@ -406,22 +422,15 @@ void CudaRenderer::render_path_aovs(const Camera& camera, CudaPathAovs& out) con
     const rt3_path_aovs dst = { out.hit_prim.data(), out.hit_entity.data(), out.hit_t.data(), out.albedo.data(), out.normal.data() };
     /* one context after the other, each writing its row tiles (the call is blocking) */
     const uint32_t n_ctx = (uint32_t) this->n_devices();
-    const uint32_t outer = params.part_count ? params.part_count : 1;
     rt3_stats total;
     std::memset(&total, 0, sizeof total);
     for (uint32_t i = 0; i < n_ctx; i++) {
         rt3_ctx* c = i == 0 ? this->ctx : this->helpers[i - 1];
-        rt3_params mine = params;
-        mine.part_count = outer * n_ctx;
-        mine.part_index = i * outer + params.part_index;
+        const rt3_params mine = context_part(params, i, n_ctx);
         check(rt3_render_path_aovs(c, &cam, &mine, &dst), "Path-traced AOVs failed");
         rt3_stats st;
         check(rt3_get_stats(c, &st), "Could not read render statistics");
-        if (i == 0) { total = st; continue; }
-        total.rays += st.rays; total.sphere_tests += st.sphere_tests; total.face_tests += st.face_tests;
-        total.accel_node_visits += st.accel_node_visits; total.accel_prim_tests += st.accel_prim_tests;
-        total.rows_rendered += st.rows_rendered; total.kernel_launches += st.kernel_launches;
-        total.device_ms += st.device_ms; total.trace_kernel_ms += st.trace_kernel_ms; /* the contexts ran one after the other */
+        if (i == 0) { total = st; } else { add_stats(total, st, false); }
     }
     this->last_stats = total;
 }
