@@ -98,9 +98,16 @@ RT3_HD float rt3_dn_luminance(float r, float g, float b) { return (0.2126f * r +
 /* max(a, 1e-3): the albedo the radiance is divided by (demodulation) and multiplied by again after the last pass. */
 RT3_HD float rt3_dn_albedo(float a) { return a > RT3_DN_MIN_ALBEDO ? a : RT3_DN_MIN_ALBEDO; }
 
+/* n / |n|, 0 where |n| = 0. Where |n|^2 would leave the normal range (|n| below about 2^-50 or above 2^50), n is first scaled
+ * by 2^100 or 2^-100: exact, so the direction is kept, and no other normal takes this branch or changes a bit. */
 RT3_HD rt3_dn_guide rt3_dn_make_guide(float nx, float ny, float nz, float hit_t) {
     rt3_dn_guide g;
-    const float len2 = (nx * nx + ny * ny) + nz * nz;
+    float len2 = (nx * nx + ny * ny) + nz * nz;
+    if (len2 < 0x1p-100f || len2 > 0x1p100f) {
+        const float s = len2 < 0x1p-100f ? 0x1p100f : 0x1p-100f;
+        nx = nx * s; ny = ny * s; nz = nz * s;
+        len2 = (nx * nx + ny * ny) + nz * nz;
+    }
     if (len2 > 0.0f) {
         const float inv = 1.0f / sqrtf(len2);
         g.nx = nx * inv; g.ny = ny * inv; g.nz = nz * inv;

@@ -12,6 +12,9 @@
 int orc_denoise(uint32_t w, uint32_t h, const float* rgb, const float* albedo, const float* normal, const float* depth, const rt3_denoise_params* p,
                 uint32_t flags, uint32_t* frame, float* rgb_out, int n_threads);
 const char* orc_denoise_check(const rt3_denoise_params* p);
+void orc_dn_exp_neg(const float* x, float* y, size_t count);
+void orc_dn_pow(const float* b, const uint32_t* n_pow, float* y, size_t count);
+void orc_dn_make_guide(const float* normal, const float* depth, float* guide, size_t count);
 
 typedef struct {
     uint32_t w, h, step, n_pow, final_pass, gamma;
@@ -58,6 +61,23 @@ static void atrous_row(void* ctx, uint32_t y) {
 }
 
 const char* orc_denoise_check(const rt3_denoise_params* p) { return rt3_dn_check_params(p); }
+
+/* The header's primitives over whole arrays, for their float64 checks (tests/test_denoise_reference.py): y = exp(-x),
+ * y = b^n, and guide = (n^x, n^y, n^z, z) per pixel of normal [count][3] and depth [count]. */
+void orc_dn_exp_neg(const float* x, float* y, size_t count) {
+    for (size_t i = 0; i < count; i++) { y[i] = rt3_dn_exp_neg(x[i]); }
+}
+
+void orc_dn_pow(const float* b, const uint32_t* n_pow, float* y, size_t count) {
+    for (size_t i = 0; i < count; i++) { y[i] = rt3_dn_pow(b[i], n_pow[i]); }
+}
+
+void orc_dn_make_guide(const float* normal, const float* depth, float* guide, size_t count) {
+    for (size_t i = 0; i < count; i++) {
+        const rt3_dn_guide g = rt3_dn_make_guide(normal[3 * i], normal[3 * i + 1], normal[3 * i + 2], depth[i]);
+        guide[4 * i] = g.nx; guide[4 * i + 1] = g.ny; guide[4 * i + 2] = g.nz; guide[4 * i + 3] = g.z;
+    }
+}
 
 int orc_denoise(uint32_t w, uint32_t h, const float* rgb, const float* albedo, const float* normal, const float* depth, const rt3_denoise_params* p,
                 uint32_t flags, uint32_t* frame, float* rgb_out, int n_threads) {
