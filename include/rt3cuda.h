@@ -289,6 +289,48 @@ typedef struct rt3_denoise_params {
  * call (device_ms, kernel_launches, rays = 0). */
 int rt3_denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb);
 
+/* Denoising a frame rendered in parts (several contexts, GPUs or processes, each with its own row tiles): every part
+ * prepares its own rows into one shared stage buffer (rt3_denoise_stage), and the stage's owner filters the whole frame
+ * from it (rt3_denoise_staged). The result is bit-equal to rt3_denoise of a one-context render of the same frame: every
+ * input of the filter's prepare step is per pixel and does not depend on the partition.
+ *
+ * The stage is plain device memory of rt3_denoise_stage_words(width, height) 32-bit words from rt3_frame_alloc(owner, ...),
+ * shared like a frame (rt3_frame_export / rt3_frame_import / rt3_frame_attach / rt3_frame_release). Layout, n = width *
+ * height pixels in frame order (index y * width + x), offsets in words:
+ *   [0, 4n)           colour plane: rt3_dn_px per pixel (16 B: radiance / max(albedo, 1e-3) per channel, its luminance);
+ *   [4n, 8n)          guide plane:  rt3_dn_guide per pixel (16 B: unit normal, depth);
+ *   [8n, 11n)         albedo plane: 3 floats per pixel, the AOV albedo as it is;
+ *   [F, F + 2 height) one 64-bit fingerprint per row (little-endian), F = 11n rounded up to an even word.
+ * A row's fingerprint is a nonzero hash of the caller's frame_tag and of everything that changes the filter's input
+ * pixels: width, height, the camera, seed, max_depth, the accumulated sample range and resolve count, RT3_FLAG_NO_JITTER,
+ * RT3_FLAG_UNIFORM_SKY, RT3_FLAG_NO_GAMMA, tile_rows, part_count, and the AOV call's seed, spp, first_sample and sampling
+ * flags (not RT3_FLAG_BVH or part_index: they change no pixel). rt3_frame_alloc zeroes the stage, so a row no part
+ * staged has fingerprint 0. */
+
+/* Words (uint32) of the stage for a width x height frame; 0 for an empty frame or when it would exceed what
+ * rt3_frame_alloc takes (2^32 - 1 words). */
+uint64_t rt3_denoise_stage_words(uint32_t width, uint32_t height);
+
+/* This context's part of a frame rendered in parts: prepares the rows its last path-traced render owns (the radiance
+ * divided by the albedo, the luminance, the guide and the raw albedo) and stores them and one fingerprint per owned row
+ * into device_stage, which uses full-frame indexing and may be a peer or IPC mapping. Checks what rt3_denoise checks,
+ * except that a partition is allowed: the render and the AOVs must have the same one (tile_rows, part_index,
+ * part_count). device_stage must not be NULL. A refusal is RT3_ERR_INVALID with a message that names the condition,
+ * and nothing changes. Asynchronous on cuda_stream (a cudaStream_t); NULL means the stream of the render that filled the
+ * accumulators. rt3_get_stats then waits for it and describes it (device_ms, kernel_launches = 1, rows_rendered). The
+ * accumulators, the AOV buffers and the RT3_FLAG_ACCUMULATE state are not touched. */
+int rt3_denoise_stage(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, uint32_t* device_stage, void* cuda_stream);
+
+/* On the stage's owner, which must be one of the parts, after every part's rt3_denoise_stage has completed: computes the
+ * fingerprint from its own render and AOV state (checked as by rt3_denoise_stage), compares it with every row's, and
+ * refuses (RT3_ERR_INVALID, naming the first row that differs and how many do; nothing written) when a row was not
+ * staged for this frame: a part that did not run, a stale row of an earlier frame_tag, or a part with other parameters.
+ * Then filters the whole frame from the stage with rt3_denoise's kernels and writes host_frame and host_rgb as
+ * rt3_denoise does (the gamma follows this context's render). Blocking. The accumulators, the AOV buffers and the
+ * RT3_FLAG_ACCUMULATE state are not touched; rt3_get_stats then describes this call (device_ms of the filter). */
+int rt3_denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, const uint32_t* device_stage,
+                       uint32_t* host_frame, float* host_rgb);
+
 /* Device-resident variant for multi-GPU plumbing: renders this partition's
  * rows into `device_frame` (a device pointer to width*height uint32, full-frame
  * indexing) asynchronously on `cuda_stream` (a cudaStream_t; NULL = the

@@ -234,6 +234,10 @@ def load_core():
     lib.rt3_tessellate_spheres.argtypes = [vp, C.POINTER(UvSphere), u32, u32, vp, vp, vp]
     lib.rt3_read_radiance.argtypes = [vp, vp, u32, u32]
     lib.rt3_denoise.argtypes = [vp, C.POINTER(DenoiseParams), vp, vp]
+    lib.rt3_denoise_stage_words.argtypes = [u32, u32]
+    lib.rt3_denoise_stage_words.restype = C.c_uint64
+    lib.rt3_denoise_stage.argtypes = [vp, C.POINTER(DenoiseParams), C.c_uint64, vp, vp]
+    lib.rt3_denoise_staged.argtypes = [vp, C.POINTER(DenoiseParams), C.c_uint64, vp, vp, vp]
     lib.rt3_get_stats.argtypes = [vp, C.POINTER(Stats)]
     lib.rt3_measure_fma_peak.argtypes = [vp, C.POINTER(C.c_double)]
     _core = lib
@@ -247,8 +251,13 @@ EXPORTED_SYMBOLS = [
     "rt3_frame_alloc", "rt3_frame_free", "rt3_frame_export", "rt3_frame_import", "rt3_frame_release",
     "rt3_frame_attach", "rt3_frame_read",
     "rt3_uv_sphere_faces", "rt3_uv_sphere_vertices", "rt3_tessellate_spheres",
-    "rt3_read_radiance", "rt3_denoise", "rt3_get_stats", "rt3_measure_fma_peak",
+    "rt3_read_radiance", "rt3_denoise", "rt3_denoise_stage_words", "rt3_denoise_stage", "rt3_denoise_staged", "rt3_get_stats", "rt3_measure_fma_peak",
 ]
+
+
+def denoise_stage_words(width, height):
+    """rt3_denoise_stage_words: 32-bit words of the stage of a (width x height) frame rendered in parts (0: too large)."""
+    return int(load_core().rt3_denoise_stage_words(width, height))
 
 
 class Context:
@@ -428,6 +437,22 @@ class Context:
         rgb = np.zeros((height, width, 3), np.float32)
         p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
         self._check(self.lib.rt3_denoise(self.handle, C.byref(p), _ptr(frame), _ptr(rgb)))
+        return frame, rgb
+
+    def denoise_stage(self, width, height, stage_ptr, tag, stream_ptr=None, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
+        """rt3_denoise_stage: this context's rows of a frame rendered in parts, prepared into the stage at ``stage_ptr`` (a device
+        pointer of denoise_stage_words(width, height) words, possibly mapped from another process) for frame ``tag``.
+        Asynchronous: ``stats()`` waits for it."""
+        p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
+        self._check(self.lib.rt3_denoise_stage(self.handle, C.byref(p), int(tag), C.c_void_p(stage_ptr), C.c_void_p(stream_ptr or 0)))
+
+    def denoise_staged(self, width, height, stage_ptr, tag, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
+        """rt3_denoise_staged: on the stage's owner, after every part staged frame ``tag``: the whole frame filtered from the stage.
+        Returns (frame [H, W] uint32, rgb [H, W, 3] float32) like ``denoise``."""
+        frame = np.zeros((height, width), np.uint32)
+        rgb = np.zeros((height, width, 3), np.float32)
+        p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
+        self._check(self.lib.rt3_denoise_staged(self.handle, C.byref(p), int(tag), C.c_void_p(stage_ptr), _ptr(frame), _ptr(rgb)))
         return frame, rgb
 
     def stats(self):

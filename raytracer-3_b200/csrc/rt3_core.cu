@@ -121,6 +121,7 @@ struct rt3_ctx {
     DeviceBuffer<unsigned long long> accum, counters;
     rt3_kparams accum_kp{};                      /* the path-traced render the accumulators currently hold */
     bool accum_valid = false;
+    uint32_t accum_first = 0;                    /* the first sample it holds (rt3_denoise_stage's fingerprint) */
     rt3_camera accum_cam{};                      /* its camera (rt3_denoise) ... */
     bool accum_cam_mixed = false;                /* ... unless an accumulating pass used another one */
 
@@ -494,7 +495,7 @@ int enqueue_render(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params
     ctx->stats.kernel_launches = accumulate ? 2 : 3;
     ctx->accum_kp = kp;
     ctx->accum_valid = true;
-    if (!accumulate) { ctx->accum_cam = *cam; ctx->accum_cam_mixed = false; }
+    if (!accumulate) { ctx->accum_cam = *cam; ctx->accum_cam_mixed = false; ctx->accum_first = kp.first_sample; }
     else if (memcmp(&ctx->accum_cam, cam, sizeof *cam) != 0) { ctx->accum_cam_mixed = true; }
     return RT3_OK;
 }
@@ -624,64 +625,183 @@ int render_path_aovs(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* para
     return rc;
 }
 
-/* rt3_denoise: prepare, variance and `iterations` à-trous passes over the accumulators and the path-traced AOVs, on the
- * stream rt3_read_radiance orders itself behind (the one of the render that filled the accumulators), blocking. Reads the
- * accumulators and the AOV buffers and writes only the dn_* buffers; every condition is checked before anything changes. */
-int denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb) {
+/* The conditions rt3_denoise and the calls for frames rendered in parts share: valid parameters, a path-traced render of
+ * the frame's size whose passes used one camera, and path AOVs of the same size, camera and scene upload. `parts`: a
+ * partition is allowed, and then the AOVs must have the render's. `fn` names the call in the messages. */
+int check_denoise_inputs(rt3_ctx* ctx, const rt3_denoise_params* params, const char* fn, bool parts) {
     if (!ctx) { return fail(RT3_ERR_INVALID, "ctx is NULL"); }
-    if (const char* why = rt3_dn_check_params(params)) { return fail(RT3_ERR_INVALID, "rt3_denoise: %s", why); }
-    if (!ctx->accum_valid) { return fail(RT3_ERR_INVALID, "rt3_denoise needs a path-traced render on this context"); }
+    if (const char* why = rt3_dn_check_params(params)) { return fail(RT3_ERR_INVALID, "%s: %s", fn, why); }
+    if (!ctx->accum_valid) { return fail(RT3_ERR_INVALID, "%s needs a path-traced render on this context", fn); }
     const rt3_kparams& kp = ctx->accum_kp;
     if (params->width != kp.width || params->height != kp.height) {
-        return fail(RT3_ERR_INVALID, "rt3_denoise: the last path-traced frame was %ux%u, not %ux%u", kp.width, kp.height, params->width, params->height);
+        return fail(RT3_ERR_INVALID, "%s: the last path-traced frame was %ux%u, not %ux%u", fn, kp.width, kp.height, params->width, params->height);
     }
-    if (kp.part_count > 1) { return fail(RT3_ERR_INVALID, "rt3_denoise: the path-traced render covers part %u of %u of the frame, not all of it", kp.part_index, kp.part_count); }
-    if (ctx->accum_cam_mixed) { return fail(RT3_ERR_INVALID, "rt3_denoise: the accumulated render's passes used different cameras"); }
-    if (!ctx->path_aovs_valid) { return fail(RT3_ERR_INVALID, "rt3_denoise needs an rt3_render_path_aovs on this context (after any rt3_render_aov with hit_t)"); }
+    if (!parts && kp.part_count > 1) { return fail(RT3_ERR_INVALID, "%s: the path-traced render covers part %u of %u of the frame, not all of it", fn, kp.part_index, kp.part_count); }
+    if (ctx->accum_cam_mixed) { return fail(RT3_ERR_INVALID, "%s: the accumulated render's passes used different cameras", fn); }
+    if (!ctx->path_aovs_valid) { return fail(RT3_ERR_INVALID, "%s needs an rt3_render_path_aovs on this context (after any rt3_render_aov with hit_t)", fn); }
     const rt3_kparams& ak = ctx->path_aovs_kp;
-    if (ak.part_count > 1) { return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs cover part %u of %u of the frame, not all of it", ak.part_index, ak.part_count); }
+    if (!parts && ak.part_count > 1) { return fail(RT3_ERR_INVALID, "%s: the AOVs cover part %u of %u of the frame, not all of it", fn, ak.part_index, ak.part_count); }
     if (ak.width != kp.width || ak.height != kp.height) {
-        return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs are %ux%u, the render %ux%u", ak.width, ak.height, kp.width, kp.height);
+        return fail(RT3_ERR_INVALID, "%s: the AOVs are %ux%u, the render %ux%u", fn, ak.width, ak.height, kp.width, kp.height);
     }
-    if (memcmp(&ctx->path_aovs_cam, &ctx->accum_cam, sizeof(rt3_camera)) != 0) { return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs and the render used different cameras"); }
-    if (!ctx->has_scene || ctx->path_aovs_scene_id != ctx->scene_id) { return fail(RT3_ERR_INVALID, "rt3_denoise: the AOVs were rendered from another scene upload than the render"); }
-    RT3_CUDA(cudaSetDevice(ctx->device));
-    const size_t n = (size_t) kp.width * kp.height;
-    int rc;
-    if ((rc = ctx->dn_col[0].reserve(n)) != RT3_OK || (rc = ctx->dn_col[1].reserve(n)) != RT3_OK || (rc = ctx->dn_guide.reserve(n)) != RT3_OK ||
-        (rc = ctx->dn_frame.reserve(n)) != RT3_OK || (host_rgb && (rc = ctx->dn_rgb.reserve(3 * n)) != RT3_OK)) {
-        return rc;
+    if (parts && (ak.tile_rows != kp.tile_rows || ak.part_index != kp.part_index || ak.part_count != kp.part_count)) {
+        return fail(RT3_ERR_INVALID, "%s: the AOVs' partition (tile_rows %u, part %u of %u) differs from the render's (%u, %u of %u)", fn, ak.tile_rows,
+                    ak.part_index, ak.part_count, kp.tile_rows, kp.part_index, kp.part_count);
     }
-    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
-    const uint32_t w = kp.width, h = kp.height, n_pow = (uint32_t) params->sigma_normal;
+    if (memcmp(&ctx->path_aovs_cam, &ctx->accum_cam, sizeof(rt3_camera)) != 0) { return fail(RT3_ERR_INVALID, "%s: the AOVs and the render used different cameras", fn); }
+    if (!ctx->has_scene || ctx->path_aovs_scene_id != ctx->scene_id) { return fail(RT3_ERR_INVALID, "%s: the AOVs were rendered from another scene upload than the render", fn); }
+    return RT3_OK;
+}
+
+/* The variance and `iterations` à-trous passes over prepared colour `col` and guides `guide`, ping-ponging through dn_col
+ * (col itself is only read), the last pass remodulating by `albedo`; then the copies to the host. Ends the pass begun by
+ * the caller, blocking; `launches` is the number of kernels the caller enqueued before. */
+int filter_to_host(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_px* col, const rt3_dn_guide* guide, const float* albedo, uint32_t launches,
+                   uint32_t* host_frame, float* host_rgb, cudaStream_t stream) {
+    const uint32_t w = params->width, h = params->height, n_pow = (uint32_t) params->sigma_normal;
+    const size_t n = (size_t) w * h;
     const float sigma_l = params->sigma_luminance, sigma_z = params->sigma_depth;
     const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid((w + RT3_DN_BLOCK_X - 1) / RT3_DN_BLOCK_X, (h + RT3_DN_BLOCK_Y - 1) / RT3_DN_BLOCK_Y);
-    if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
-    RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
-    denoise_prepare_kernel<<<(unsigned) ((n + 255) / 256), 256, 0, stream>>>(kp, ctx->accum.ptr, ctx->aov_albedo.ptr, ctx->aov_normal.ptr, ctx->aov_t.ptr,
-                                                                           ctx->dn_col[1].ptr, ctx->dn_guide.ptr);
+    denoise_variance_kernel<<<grid, block, 0, stream>>>(w, h, sigma_z, n_pow, col, guide, ctx->dn_col[0].ptr);
     RT3_CUDA(cudaGetLastError());
-    denoise_variance_kernel<<<grid, block, 0, stream>>>(w, h, sigma_z, n_pow, ctx->dn_col[1].ptr, ctx->dn_guide.ptr, ctx->dn_col[0].ptr);
-    RT3_CUDA(cudaGetLastError());
-    const bool gamma = !(kp.flags & RT3_FLAG_NO_GAMMA);
+    const bool gamma = !(ctx->accum_kp.flags & RT3_FLAG_NO_GAMMA);
     for (uint32_t i = 0; i < params->iterations; i++) {
         const rt3_dn_px* in = ctx->dn_col[i & 1u].ptr;
         rt3_dn_px* out = ctx->dn_col[(i + 1u) & 1u].ptr;
         if (i + 1u < params->iterations) {
-            denoise_atrous_kernel<false><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, ctx->dn_guide.ptr, out, nullptr, gamma, nullptr, nullptr);
+            denoise_atrous_kernel<false><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, guide, out, nullptr, gamma, nullptr, nullptr);
         } else {
-            denoise_atrous_kernel<true><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, ctx->dn_guide.ptr, nullptr, ctx->aov_albedo.ptr, gamma,
+            denoise_atrous_kernel<true><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, guide, nullptr, albedo, gamma,
                                                                     ctx->dn_frame.ptr, host_rgb ? ctx->dn_rgb.ptr : nullptr);
         }
         RT3_CUDA(cudaGetLastError());
     }
     RT3_CUDA(cudaEventRecord(ctx->ev_k1, stream));
     RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
-    ctx->stats.kernel_launches = 2 + params->iterations;
+    ctx->stats.kernel_launches = launches + 1 + params->iterations;
     if (host_frame) { RT3_CUDA(cudaMemcpyAsync(host_frame, ctx->dn_frame.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream)); }
     if (host_rgb) { RT3_CUDA(cudaMemcpyAsync(host_rgb, ctx->dn_rgb.ptr, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, stream)); }
-    if ((rc = end_pass(ctx, stream)) != RT3_OK) { return rc; }
+    int rc = end_pass(ctx, stream);
+    if (rc != RT3_OK) { return rc; }
     return collect_stats(ctx);
+}
+
+/* The filter's ping-pong buffers and outputs (plus the guides when `guide`), sized on first use. */
+int reserve_denoise(rt3_ctx* ctx, size_t n, bool guide, bool rgb) {
+    int rc;
+    if ((rc = ctx->dn_col[0].reserve(n)) != RT3_OK || (rc = ctx->dn_col[1].reserve(n)) != RT3_OK || (guide && (rc = ctx->dn_guide.reserve(n)) != RT3_OK) ||
+        (rc = ctx->dn_frame.reserve(n)) != RT3_OK || (rgb && (rc = ctx->dn_rgb.reserve(3 * n)) != RT3_OK)) {
+        return rc;
+    }
+    return RT3_OK;
+}
+
+/* rt3_denoise: prepare, variance and `iterations` à-trous passes over the accumulators and the path-traced AOVs, on the
+ * stream rt3_read_radiance orders itself behind (the one of the render that filled the accumulators), blocking. Reads the
+ * accumulators and the AOV buffers and writes only the dn_* buffers; every condition is checked before anything changes. */
+int denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb) {
+    int rc = check_denoise_inputs(ctx, params, "rt3_denoise", false);
+    if (rc != RT3_OK) { return rc; }
+    RT3_CUDA(cudaSetDevice(ctx->device));
+    const rt3_kparams& kp = ctx->accum_kp;
+    const size_t n = (size_t) kp.width * kp.height;
+    if ((rc = reserve_denoise(ctx, n, true, host_rgb != nullptr)) != RT3_OK) { return rc; }
+    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
+    if ((rc = begin_pass(ctx, false, kp.height, stream, nullptr)) != RT3_OK) { return rc; }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
+    denoise_prepare_kernel<<<(unsigned) ((n + 255) / 256), 256, 0, stream>>>(kp, ctx->accum.ptr, ctx->aov_albedo.ptr, ctx->aov_normal.ptr, ctx->aov_t.ptr,
+                                                                           ctx->dn_col[1].ptr, ctx->dn_guide.ptr);
+    RT3_CUDA(cudaGetLastError());
+    return filter_to_host(ctx, params, ctx->dn_col[1].ptr, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, 1u, host_frame, host_rgb, stream);
+}
+
+/* Where the planes of a stage of rt3_denoise_stage_words(w, h) words start (include/rt3cuda.h). */
+struct stage_view {
+    rt3_dn_px* col;
+    rt3_dn_guide* guide;
+    float* albedo;
+    unsigned long long* fingerprint;
+};
+
+uint64_t stage_fingerprint_offset(uint64_t n) { return (11ull * n + 1ull) & ~1ull; }
+
+stage_view stage_planes(uint32_t* stage, uint32_t w, uint32_t h) {
+    const uint64_t n = (uint64_t) w * h;
+    return { reinterpret_cast<rt3_dn_px*>(stage), reinterpret_cast<rt3_dn_guide*>(stage + 4 * n), reinterpret_cast<float*>(stage + 8 * n),
+             reinterpret_cast<unsigned long long*>(stage + stage_fingerprint_offset(n)) };
+}
+
+uint64_t fnv1a(uint64_t hash, const void* data, size_t bytes) {
+    const unsigned char* b = static_cast<const unsigned char*>(data);
+    for (size_t i = 0; i < bytes; i++) { hash = (hash ^ b[i]) * 0x100000001b3ull; }
+    return hash;
+}
+
+/* The rows' fingerprint for this context's render and AOVs (include/rt3cuda.h): nonzero, and equal on two parts exactly
+ * when their filter inputs are pixels of the same frame. */
+uint64_t stage_fingerprint(const rt3_ctx* ctx, uint64_t frame_tag) {
+    const rt3_kparams& kp = ctx->accum_kp;
+    const rt3_kparams& ak = ctx->path_aovs_kp;
+    const uint32_t sampling = RT3_FLAG_NO_JITTER | RT3_FLAG_UNIFORM_SKY;
+    const uint32_t fields[] = { kp.width, kp.height, kp.seed, kp.max_depth, ctx->accum_first, kp.first_sample + kp.spp, kp.resolve_spp,
+                                kp.flags & (sampling | RT3_FLAG_NO_GAMMA), kp.tile_rows, kp.part_count, ak.seed, ak.spp, ak.first_sample, ak.flags & sampling };
+    uint64_t hash = fnv1a(0xcbf29ce484222325ull, &frame_tag, sizeof frame_tag);
+    hash = fnv1a(hash, fields, sizeof fields);
+    hash = fnv1a(hash, &ctx->accum_cam, sizeof(rt3_camera));
+    return hash ? hash : 1ull;
+}
+
+/* rt3_denoise_stage: denoise_stage_kernel over the owned rows, asynchronous on `stream`; rt3_get_stats waits for it. */
+int denoise_stage(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, uint32_t* device_stage, cudaStream_t user_stream) {
+    int rc = check_denoise_inputs(ctx, params, "rt3_denoise_stage", true);
+    if (rc != RT3_OK) { return rc; }
+    if (!device_stage) { return fail(RT3_ERR_INVALID, "rt3_denoise_stage: device_stage is NULL"); }
+    const rt3_kparams& kp = ctx->accum_kp;
+    if (rt3_denoise_stage_words(kp.width, kp.height) == 0) { return fail(RT3_ERR_INVALID, "rt3_denoise_stage: a %ux%u frame does not fit in a stage", kp.width, kp.height); }
+    RT3_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t stream = user_stream ? user_stream : ctx->last_stream ? ctx->last_stream : ctx->stream;
+    const stage_view s = stage_planes(device_stage, kp.width, kp.height);
+    if ((rc = begin_pass(ctx, false, kp.owned_rows, stream, nullptr)) != RT3_OK) { return rc; }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
+    if (kp.n_pixels != 0) {
+        denoise_stage_kernel<<<(unsigned) ((kp.n_pixels + 255ull) / 256ull), 256, 0, stream>>>(kp, ctx->accum.ptr, ctx->aov_albedo.ptr, ctx->aov_normal.ptr,
+                                                                                              ctx->aov_t.ptr, s.col, s.guide, s.albedo, s.fingerprint,
+                                                                                              stage_fingerprint(ctx, frame_tag));
+        RT3_CUDA(cudaGetLastError());
+        ctx->stats.kernel_launches = 1;
+    }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k1, stream));
+    RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
+    return RT3_OK;
+}
+
+/* rt3_denoise_staged: checks every row's fingerprint on the host, then the filter over the stage's planes, blocking. */
+int denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, const uint32_t* device_stage, uint32_t* host_frame, float* host_rgb) {
+    int rc = check_denoise_inputs(ctx, params, "rt3_denoise_staged", true);
+    if (rc != RT3_OK) { return rc; }
+    if (!device_stage) { return fail(RT3_ERR_INVALID, "rt3_denoise_staged: device_stage is NULL"); }
+    const rt3_kparams& kp = ctx->accum_kp;
+    const uint32_t w = kp.width, h = kp.height;
+    if (rt3_denoise_stage_words(w, h) == 0) { return fail(RT3_ERR_INVALID, "rt3_denoise_staged: a %ux%u frame does not fit in a stage", w, h); }
+    RT3_CUDA(cudaSetDevice(ctx->device));
+    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
+    const stage_view s = stage_planes(const_cast<uint32_t*>(device_stage), w, h);
+    std::vector<unsigned long long> rows(h);
+    RT3_CUDA(cudaMemcpyAsync(rows.data(), s.fingerprint, h * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
+    RT3_CUDA(cudaStreamSynchronize(stream));
+    const unsigned long long expect = stage_fingerprint(ctx, frame_tag);
+    uint32_t bad = 0, first_bad = 0;
+    for (uint32_t y = 0; y < h; y++) {
+        if (rows[y] != expect && bad++ == 0) { first_bad = y; }
+    }
+    if (bad) {
+        return fail(RT3_ERR_INVALID, "rt3_denoise_staged: row %u (and %u rows in all, of %u) was not staged for this frame: a part that did not run, a stale row of "
+                    "another frame_tag, or a part rendered with other parameters", first_bad, bad, h);
+    }
+    if ((rc = reserve_denoise(ctx, (size_t) w * h, false, host_rgb != nullptr)) != RT3_OK) { return rc; }
+    if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
+    return filter_to_host(ctx, params, s.col, s.guide, s.albedo, 0u, host_frame, host_rgb, stream);
 }
 
 /* Reads back the timings and counters of the most recent render (synchronises its stream). */
@@ -1000,6 +1120,22 @@ int rt3_render_path_aovs(rt3_ctx* ctx, const rt3_camera* camera, const rt3_param
 
 int rt3_denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb) {
     return denoise(ctx, params, host_frame, host_rgb);
+}
+
+uint64_t rt3_denoise_stage_words(uint32_t width, uint32_t height) {
+    const uint64_t n = (uint64_t) width * height;
+    if (n == 0) { return 0; }
+    const uint64_t words = stage_fingerprint_offset(n) + 2ull * height;
+    return words > 0xFFFFFFFFull ? 0 : words;
+}
+
+int rt3_denoise_stage(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, uint32_t* device_stage, void* cuda_stream) {
+    return denoise_stage(ctx, params, frame_tag, device_stage, (cudaStream_t) cuda_stream);
+}
+
+int rt3_denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, const uint32_t* device_stage, uint32_t* host_frame,
+                       float* host_rgb) {
+    return denoise_staged(ctx, params, frame_tag, device_stage, host_frame, host_rgb);
 }
 
 int rt3_render_device(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, uint32_t* device_frame, void* cuda_stream) {

@@ -1,8 +1,10 @@
 /* rt3_denoise.cuh — kernels of rt3_denoise (DESIGN.md 3.8): the edge-avoiding à-trous filter on the radiance of the last
  * path-traced render, guided by the last path-traced AOVs. The arithmetic is include/rt3_denoise.h's; these kernels only
- * load, call it and store. Every kernel covers the whole frame (rt3_denoise needs part_count <= 1), one thread per pixel.
+ * load, call it and store. Every kernel but the stage covers the whole frame (rt3_denoise needs part_count <= 1), one
+ * thread per pixel.
  *
  *   denoise_prepare_kernel   : radiance (radiance_kernel's expression) / albedo -> colour + luminance, normal + depth -> guide.
+ *   denoise_stage_kernel     : the same for a partition's owned rows, into a stage buffer (rt3_denoise_stage), + row fingerprints.
  *   denoise_variance_kernel  : 7x7 luminance variance.
  *   denoise_atrous_kernel<F> : one 5x5 pass at step 2^i; F = the last pass, which remodulates and resolves like resolve_kernel.
  *
@@ -12,6 +14,7 @@
 
 #include "rt3_denoise.h"
 #include "rt3_device.cuh"
+#include "rt3_kernels.cuh" /* owned_row_to_global */
 
 #define RT3_DN_BLOCK_X 32
 #define RT3_DN_BLOCK_Y 8
@@ -33,6 +36,35 @@ __global__ void __launch_bounds__(256) denoise_prepare_kernel(rt3_kparams P, con
     rt3_dn_prepare_px(c, a, n, depth[idx], &px, &g);
     col[idx] = px;
     guide[idx] = g;
+}
+
+/* rt3_denoise_stage: denoise_prepare_kernel's step for the rows a partitioned render owns (one thread per owned pixel, the
+ * row mapping of resolve_kernel), stored at full-frame indices into the stage's colour, guide and albedo planes, which may
+ * live on another GPU; the first thread of each row also stores the row's fingerprint. */
+__global__ void __launch_bounds__(256) denoise_stage_kernel(rt3_kparams P, const unsigned long long* __restrict__ accum, const float* __restrict__ albedo,
+                                                           const float* __restrict__ normal, const float* __restrict__ depth, rt3_dn_px* __restrict__ col,
+                                                           rt3_dn_guide* __restrict__ guide, float* __restrict__ stage_albedo,
+                                                           unsigned long long* __restrict__ row_fingerprint, unsigned long long fingerprint) {
+    const unsigned long long p = (unsigned long long) blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= P.n_pixels) { return; }
+    const uint32_t local_row = (uint32_t) (p / P.width), x = (uint32_t) (p - (unsigned long long) local_row * P.width);
+    const uint32_t y = owned_row_to_global(P, local_row);
+    const size_t idx = (size_t) y * P.width + x;
+    float c[3], a[3], n[3];
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        c[k] = (float) ((double) accum[3 * idx + k] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE));
+        a[k] = albedo[3 * idx + k];
+        n[k] = normal[3 * idx + k];
+    }
+    rt3_dn_px px;
+    rt3_dn_guide g;
+    rt3_dn_prepare_px(c, a, n, depth[idx], &px, &g);
+    col[idx] = px;
+    guide[idx] = g;
+#pragma unroll
+    for (int k = 0; k < 3; k++) { stage_albedo[3 * idx + k] = a[k]; }
+    if (x == 0) { row_fingerprint[y] = fingerprint; }
 }
 
 __global__ void __launch_bounds__(RT3_DN_BLOCK_X * RT3_DN_BLOCK_Y) denoise_variance_kernel(uint32_t w, uint32_t h, float sigma_z, uint32_t n_pow,

@@ -68,6 +68,12 @@ class SharedFrame:
     Construction and ``close()`` are collective. If any rank cannot map the frame (no peer access
     between two GPUs, IPC unavailable), ``ok`` is False on every rank and ``error`` says why: the
     caller then closes it and gathers with NCCL instead.
+
+    ``n_pixels`` counts 32-bit words, so the same class shares the stage of a frame denoised in parts:
+    ``SharedFrame(ctx, dist, abi.denoise_stage_words(w, h), rank, world, device)``. Each rank then calls
+    ``ctx.denoise_stage(w, h, shared.ptr, tag)`` and ``ctx.stats()`` (which waits for its stores), all ranks meet in a
+    barrier that holds the host (``dist.barrier()``; ``finish()`` only orders torch's stream, not the library's), and the
+    owner calls ``ctx.denoise_staged(w, h, shared.ptr, tag)``.
     """
 
     def __init__(self, ctx, dist, n_pixels, rank, world, device, owner=0):
