@@ -2,8 +2,8 @@
  *
  * One definition for both sides: the kernels (csrc/rt3_denoise.cuh, nvcc -fmad=false) and the CPU restatement
  * (tests/denoise_oracle.c, gcc -ffp-contract=off) call these functions, so they agree bit for bit. As in rt3_rng.h,
- * every floating-point operation is one IEEE-754 binary32 operation in the order written; the only library call is
- * sqrtf (correctly rounded on both sides). exp(-x) is a fixed polynomial with range reduction, and the normal term's
+ * every floating-point operation is one IEEE-754 binary32 operation in the order written; the only library calls are
+ * sqrtf (correctly rounded on both sides) and floorf (exact). exp(-x) is a fixed polynomial with range reduction, and the normal term's
  * power is taken by repeated squaring.
  *
  * Filter (Dammertz et al. 2010; the spatial filter of SVGF, Schied et al. 2017, without its temporal part):
@@ -23,6 +23,7 @@
 #ifndef RT3_DENOISE_H
 #define RT3_DENOISE_H
 
+#include <math.h>
 #include <stdint.h>
 #include <string.h>
 
@@ -38,10 +39,12 @@
 
 #if defined(__CUDACC__)
 #define RT3_DN_ALIGN16 __align__(16)
+#define RT3_DN_ALIGN8 __align__(8)
 #define RT3_DN_RESTRICT __restrict__
 #define RT3_DN_UNROLL _Pragma("unroll")
 #else
 #define RT3_DN_ALIGN16 __attribute__((aligned(16)))
+#define RT3_DN_ALIGN8 __attribute__((aligned(8)))
 #define RT3_DN_RESTRICT restrict
 #define RT3_DN_UNROLL
 #endif
@@ -253,6 +256,147 @@ static inline const char* rt3_dn_check_params(const rt3_denoise_params* p) {
     if (!(p->sigma_normal >= 1.0f && p->sigma_normal <= RT3_DN_MAX_NORMAL_POWER) || (float) (uint32_t) p->sigma_normal != p->sigma_normal) {
         return "sigma_normal must be a whole number in 1..1024 (the exponent of the normal term)";
     }
+    return NULL;
+}
+
+/* ---- temporal accumulation (rt3_denoise_temporal, DESIGN.md 3.9) -------------------------------------------------------
+ * For pixel p = (x, y): e, L and the guide from rt3_dn_prepare_px; the surface point X = o + z d^ of the primary ray (o, d^)
+ * of the AOV call's sample first_sample (a miss: the direction d^, a point at infinity); its continuous position in the
+ * previous frame pos = (x, y) + (proj(prev, X) - proj(cur, X)); the 2x2 bilinear taps of the history around pos that
+ * agree in geometry, weight-normalised, give c_h, m1_h, m2_h, n_h (none when their weights sum to <= 0.01); then
+ * n = n_h + 1, c = c_h + max(alpha_color, 1/n) (e - c_h), m1, m2 likewise towards L and L L with alpha_moments; without
+ * history c = e, m1 = L, m2 = L L, n = 1. The variance is max(0, m2 - m1 m1) from n >= 4, else the 7x7 estimate over the
+ * accumulated colour. */
+
+#define RT3_DN_MIN_HISTORY_WEIGHT 0.01f
+#define RT3_DN_MOMENT_FRAMES 4.0f
+
+/* Per-pixel history: accumulated demodulated colour and the history length n; the luminance moments E[L], E[L^2]. */
+typedef struct RT3_DN_ALIGN16 rt3_dn_hist {
+    float r, g, b, n;
+} rt3_dn_hist;
+
+typedef struct RT3_DN_ALIGN8 rt3_dn_moments {
+    float m1, m2;
+} rt3_dn_moments;
+
+/* det[u v w] = u . (v x w) */
+RT3_HD float rt3_dn_det3(float ux, float uy, float uz, float vx, float vy, float vz, float wx, float wy, float wz) {
+    return (ux * (vy * wz - vz * wy) + uy * (vz * wx - vx * wz)) + uz * (vx * wy - vy * wx);
+}
+
+/* proj(cam, X): solves X - O = s (llc - O) + a hor + b ver by Cramer's rule (O the camera origin, the lens centre; for a
+ * miss, X is the direction and takes the place of X - O) and writes the continuous pixel position
+ * (a/s (W-1), (H-1) - b/s (H-1)): the inverse of start_path's mapping of an unjittered pinhole ray. Returns 0 (no
+ * position) unless s > 0. */
+RT3_HD int rt3_dn_project(rt3_camera cam, float x, float y, float z, int miss, uint32_t w, uint32_t h, float* px, float* py) {
+    const float rx = miss ? x : x - cam.origin[0], ry = miss ? y : y - cam.origin[1], rz = miss ? z : z - cam.origin[2];
+    const float ax = cam.lower_left_corner[0] - cam.origin[0], ay = cam.lower_left_corner[1] - cam.origin[1], az = cam.lower_left_corner[2] - cam.origin[2];
+    const float bx = cam.horizontal[0], by = cam.horizontal[1], bz = cam.horizontal[2];
+    const float cx = cam.vertical[0], cy = cam.vertical[1], cz = cam.vertical[2];
+    const float det = rt3_dn_det3(ax, ay, az, bx, by, bz, cx, cy, cz);
+    const float s = rt3_dn_det3(rx, ry, rz, bx, by, bz, cx, cy, cz) / det;
+    const float a = rt3_dn_det3(ax, ay, az, rx, ry, rz, cx, cy, cz) / det;
+    const float b = rt3_dn_det3(ax, ay, az, bx, by, bz, rx, ry, rz) / det;
+    if (!(s > 0.0f)) { return 0; }
+    const float wm1 = (float) w - 1.0f, hm1 = (float) h - 1.0f;
+    *px = (a / s) * wm1;
+    *py = hm1 - (b / s) * hm1;
+    return 1;
+}
+
+/* Steps 2-4: the surface point X = o + z d^ (a miss, z = +inf: d^), its position (*px, *py) in the previous frame and, for a
+ * hit, its distance |X - O_prev| from the previous camera's origin (*dist). Returns 0 when either projection has s <= 0. */
+RT3_HD int rt3_dn_reproject(rt3_camera cur, rt3_camera prev, uint32_t w, uint32_t h, uint32_t x, uint32_t y, float ox, float oy, float oz, float dx,
+                            float dy, float dz, float z, float* px, float* py, float* dist) {
+    const int miss = z > RT3_DN_FLT_MAX;
+    const float X = miss ? dx : ox + z * dx, Y = miss ? dy : oy + z * dy, Z = miss ? dz : oz + z * dz;
+    float cpx, cpy, ppx, ppy;
+    if (!rt3_dn_project(cur, X, Y, Z, miss, w, h, &cpx, &cpy) || !rt3_dn_project(prev, X, Y, Z, miss, w, h, &ppx, &ppy)) { return 0; }
+    *px = (float) x + (ppx - cpx);
+    *py = (float) y + (ppy - cpy);
+    const float ex = X - prev.origin[0], ey = Y - prev.origin[1], ez = Z - prev.origin[2];
+    *dist = miss ? 0.0f : sqrtf((ex * ex + ey * ey) + ez * ez);
+    return 1;
+}
+
+/* Whether history tap q is used for pixel p: both misses, or both hits with |z_q - dist| <= depth_tolerance dist and
+ * n^_p . n^_q >= normal_cos (dist = |X - O_prev|). */
+RT3_HD int rt3_dn_history_tap_ok(rt3_dn_guide p, rt3_dn_guide q, float dist, float depth_tolerance, float normal_cos) {
+    const int miss_p = p.z > RT3_DN_FLT_MAX, miss_q = q.z > RT3_DN_FLT_MAX;
+    if (miss_p != miss_q) { return 0; }
+    if (miss_p) { return 1; }
+    const float dz = q.z - dist;
+    if (!((dz < 0.0f ? -dz : dz) <= depth_tolerance * dist)) { return 0; }
+    return (p.nx * q.nx + p.ny * q.ny) + p.nz * q.nz >= normal_cos;
+}
+
+/* Steps 5-6 at pixel p with prepared colour e (v = L) and guide gp: reads the previous history (w x h, frame order) at the
+ * bilinear taps around (px, py) when `have` (a position exists), writes the new history's colour and length to *col and
+ * its moments to *mom. */
+RT3_HD void rt3_dn_accumulate_px(const rt3_dn_hist* RT3_DN_RESTRICT prev_col, const rt3_dn_moments* RT3_DN_RESTRICT prev_mom,
+                                 const rt3_dn_guide* RT3_DN_RESTRICT prev_guide, uint32_t w, uint32_t h, int have, float px, float py, float dist,
+                                 rt3_dn_px e, rt3_dn_guide gp, const rt3_denoise_temporal_params* tp, rt3_dn_hist* col, rt3_dn_moments* mom) {
+    float sw = 0.0f, sr = 0.0f, sg = 0.0f, sb = 0.0f, sn = 0.0f, s1 = 0.0f, s2 = 0.0f;
+    if (have && px > -1.0f && px < (float) w && py > -1.0f && py < (float) h) {
+        const float fx0 = floorf(px), fy0 = floorf(py);
+        const float fx = px - fx0, fy = py - fy0;
+        const int x0 = (int) fx0, y0 = (int) fy0;
+        RT3_DN_UNROLL
+        for (int ty = 0; ty < 2; ty++) {
+            const int qy = y0 + ty;
+            const float wy = ty ? fy : 1.0f - fy;
+            RT3_DN_UNROLL
+            for (int tx = 0; tx < 2; tx++) {
+                const int qx = x0 + tx;
+                const float wt = wy * (tx ? fx : 1.0f - fx);
+                if (!(wt > 0.0f) || qx < 0 || qx >= (int) w || qy < 0 || qy >= (int) h) { continue; }
+                const size_t q = (size_t) qy * w + (size_t) qx;
+                if (!rt3_dn_history_tap_ok(gp, prev_guide[q], dist, tp->depth_tolerance, tp->normal_cos)) { continue; }
+                const rt3_dn_hist hq = prev_col[q];
+                const rt3_dn_moments mq = prev_mom[q];
+                sw = sw + wt;
+                sr = sr + wt * hq.r; sg = sg + wt * hq.g; sb = sb + wt * hq.b;
+                sn = sn + wt * hq.n;
+                s1 = s1 + wt * mq.m1; s2 = s2 + wt * mq.m2;
+            }
+        }
+    }
+    const float l = e.v;
+    if (!(sw > RT3_DN_MIN_HISTORY_WEIGHT)) {
+        col->r = e.r; col->g = e.g; col->b = e.b; col->n = 1.0f;
+        mom->m1 = l; mom->m2 = l * l;
+        return;
+    }
+    const float hr = sr / sw, hg = sg / sw, hb = sb / sw, h1 = s1 / sw, h2 = s2 / sw;
+    const float n = sn / sw + 1.0f;
+    const float inv = 1.0f / n;
+    const float ac = tp->alpha_color > inv ? tp->alpha_color : inv, am = tp->alpha_moments > inv ? tp->alpha_moments : inv;
+    col->r = hr + ac * (e.r - hr); col->g = hg + ac * (e.g - hg); col->b = hb + ac * (e.b - hb); col->n = n;
+    mom->m1 = h1 + am * (l - h1);
+    mom->m2 = h2 + am * (l * l - h2);
+}
+
+/* Step 7: the luminance variance of the accumulated state at (x, y): from the moments once n >= 4, else
+ * rt3_dn_variance_px over `acc` (colour, v = L(colour)). */
+RT3_HD float rt3_dn_temporal_variance_px(const rt3_dn_px* RT3_DN_RESTRICT acc, const rt3_dn_guide* RT3_DN_RESTRICT guide, float n, rt3_dn_moments m,
+                                         uint32_t w, uint32_t h, uint32_t x, uint32_t y, float sigma_z, uint32_t n_pow) {
+    if (n >= RT3_DN_MOMENT_FRAMES) {
+        const float var = m.m2 - m.m1 * m.m1;
+        return var > 0.0f ? var : 0.0f;
+    }
+    return rt3_dn_variance_px(acc, guide, w, h, x, y, sigma_z, n_pow);
+}
+
+/* NULL when the parameters of rt3_denoise_temporal are valid, else what is wrong with them. */
+static inline const char* rt3_dn_check_temporal_params(const rt3_denoise_temporal_params* p) {
+    if (!p) { return "params is NULL"; }
+    const char* why = rt3_dn_check_params(&p->filter);
+    if (why) { return why; }
+    if (!(p->alpha_color > 0.0f && p->alpha_color <= 1.0f)) { return "alpha_color must be in (0, 1]"; }
+    if (!(p->alpha_moments > 0.0f && p->alpha_moments <= 1.0f)) { return "alpha_moments must be in (0, 1]"; }
+    if (!(p->depth_tolerance > 0.0f && p->depth_tolerance <= RT3_DN_FLT_MAX)) { return "depth_tolerance must be finite and > 0"; }
+    if (!(p->normal_cos >= -1.0f && p->normal_cos <= 1.0f)) { return "normal_cos must be in [-1, 1]"; }
     return NULL;
 }
 

@@ -289,6 +289,35 @@ typedef struct rt3_denoise_params {
  * call (device_ms, kernel_launches, rays = 0). */
 int rt3_denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb);
 
+/* Parameters of rt3_denoise_temporal (defaults: SVGF's). */
+typedef struct rt3_denoise_temporal_params {
+    rt3_denoise_params filter; /* the spatial passes, checked exactly as rt3_denoise checks them */
+    float alpha_color;         /* (0, 1], default 0.2: smallest weight of the new frame in the colour history */
+    float alpha_moments;       /* (0, 1], default 0.2: the same for the luminance moments */
+    float depth_tolerance;     /* finite, > 0, default 0.05: relative depth test of a history tap */
+    float normal_cos;          /* [-1, 1], default 0.9: smallest n^_p . n^_q of a history tap */
+    uint32_t reset;            /* nonzero: ignore and replace the context's history */
+} rt3_denoise_temporal_params;
+
+/* rt3_denoise with temporal accumulation (the temporal half of SVGF): for a sequence of frames of one scene upload and
+ * size whose camera moves, each pixel's surface point (the primary ray of sample first_sample of the last
+ * rt3_render_path_aovs, at its depth; a miss: its direction) is reprojected into the previous call's camera, the 2x2
+ * bilinear taps of the history there that agree in geometry (both misses, or both hits within depth_tolerance of the
+ * distance and normal_cos of the normal) are blended into an exponential moving average of the demodulated colour and
+ * of the luminance moments, and the luminance variance comes from those moments once 4 frames are behind a pixel. The
+ * unchanged à-trous passes of rt3_denoise then filter the accumulated colour. Formulas: include/rt3_denoise.h, DESIGN.md
+ * 3.9. Takes and checks what rt3_denoise takes and checks (messages name rt3_denoise_temporal), plus the parameters
+ * above. The history (unfiltered colour, moments and length per pixel, the guide, and the camera, size and scene upload
+ * that produced it) lives on the context; it is dropped, and every pixel starts at length 1, when reset is set, when
+ * there is none yet, or when the width, height or scene upload differ from the history's. Render every frame with its
+ * own seed: repeated noise is not averaged away. A call with no usable history anywhere is bit-equal to rt3_denoise.
+ * Writes host_frame and host_rgb as rt3_denoise does, and each pixel's new history length to host_history_length; any
+ * may be NULL. Blocking. A refused call (RT3_ERR_INVALID) changes nothing; a call that fails with a CUDA error drops the
+ * history. The accumulators, the AOV buffers and the RT3_FLAG_ACCUMULATE state are not touched, and rt3_denoise is not
+ * affected by it. rt3_get_stats then describes this call (device_ms, kernel_launches, rays = 0). */
+int rt3_denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* params, uint32_t* host_frame, float* host_rgb,
+                         float* host_history_length);
+
 /* Denoising a frame rendered in parts (several contexts, GPUs or processes, each with its own row tiles): every part
  * prepares its own rows into one shared stage buffer (rt3_denoise_stage), and the stage's owner filters the whole frame
  * from it (rt3_denoise_staged). The result is bit-equal to rt3_denoise of a one-context render of the same frame: every

@@ -103,6 +103,17 @@ def denoise_params(width=0, height=0, iterations=5, sigma_luminance=4.0, sigma_n
     return DenoiseParams(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
 
 
+class DenoiseTemporalParams(C.Structure):
+    """rt3_denoise_temporal_params."""
+    _fields_ = [("filter", DenoiseParams), ("alpha_color", C.c_float), ("alpha_moments", C.c_float), ("depth_tolerance", C.c_float),
+                ("normal_cos", C.c_float), ("reset", C.c_uint32)]
+
+
+def denoise_temporal_params(width=0, height=0, reset=False, alpha_color=0.2, alpha_moments=0.2, depth_tolerance=0.05, normal_cos=0.9, **filter):
+    """rt3_denoise_temporal_params with SVGF's defaults; ``filter`` takes denoise_params' keywords."""
+    return DenoiseTemporalParams(denoise_params(width, height, **filter), alpha_color, alpha_moments, depth_tolerance, normal_cos, 1 if reset else 0)
+
+
 def _ptr(a):
     return None if a is None else a.ctypes.data_as(C.c_void_p)
 
@@ -234,6 +245,7 @@ def load_core():
     lib.rt3_tessellate_spheres.argtypes = [vp, C.POINTER(UvSphere), u32, u32, vp, vp, vp]
     lib.rt3_read_radiance.argtypes = [vp, vp, u32, u32]
     lib.rt3_denoise.argtypes = [vp, C.POINTER(DenoiseParams), vp, vp]
+    lib.rt3_denoise_temporal.argtypes = [vp, C.POINTER(DenoiseTemporalParams), vp, vp, vp]
     lib.rt3_denoise_stage_words.argtypes = [u32, u32]
     lib.rt3_denoise_stage_words.restype = C.c_uint64
     lib.rt3_denoise_stage.argtypes = [vp, C.POINTER(DenoiseParams), C.c_uint64, vp, vp]
@@ -251,7 +263,7 @@ EXPORTED_SYMBOLS = [
     "rt3_frame_alloc", "rt3_frame_free", "rt3_frame_export", "rt3_frame_import", "rt3_frame_release",
     "rt3_frame_attach", "rt3_frame_read",
     "rt3_uv_sphere_faces", "rt3_uv_sphere_vertices", "rt3_tessellate_spheres",
-    "rt3_read_radiance", "rt3_denoise", "rt3_denoise_stage_words", "rt3_denoise_stage", "rt3_denoise_staged", "rt3_get_stats", "rt3_measure_fma_peak",
+    "rt3_read_radiance", "rt3_denoise", "rt3_denoise_temporal", "rt3_denoise_stage_words", "rt3_denoise_stage", "rt3_denoise_staged", "rt3_get_stats", "rt3_measure_fma_peak",
 ]
 
 
@@ -438,6 +450,17 @@ class Context:
         p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
         self._check(self.lib.rt3_denoise(self.handle, C.byref(p), _ptr(frame), _ptr(rgb)))
         return frame, rgb
+
+    def denoise_temporal(self, width, height, reset=False, alpha_color=0.2, alpha_moments=0.2, depth_tolerance=0.05, normal_cos=0.9, **filter):
+        """rt3_denoise_temporal: ``denoise`` with the context's history of earlier frames reprojected through the camera's motion
+        and accumulated (``reset`` drops it first); ``filter`` takes ``denoise``'s keywords. Render each frame with its own seed.
+        Returns (frame [H, W] uint32, rgb [H, W, 3] float32, history_length [H, W] float32)."""
+        frame = np.zeros((height, width), np.uint32)
+        rgb = np.zeros((height, width, 3), np.float32)
+        length = np.zeros((height, width), np.float32)
+        p = denoise_temporal_params(width, height, reset, alpha_color, alpha_moments, depth_tolerance, normal_cos, **filter)
+        self._check(self.lib.rt3_denoise_temporal(self.handle, C.byref(p), _ptr(frame), _ptr(rgb), _ptr(length)))
+        return frame, rgb, length
 
     def denoise_stage(self, width, height, stage_ptr, tag, stream_ptr=None, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
         """rt3_denoise_stage: this context's rows of a frame rendered in parts, prepared into the stage at ``stage_ptr`` (a device

@@ -137,6 +137,18 @@ struct rt3_ctx {
     DeviceBuffer<float> dn_rgb;
     DeviceBuffer<uint32_t> dn_frame;
 
+    /* rt3_denoise_temporal: two histories, the valid one read and the other written; they swap when a call succeeds. The
+     * camera, size and scene upload are those of the frame that produced the valid one. */
+    DeviceBuffer<rt3_dn_hist> dn_hist_col[2];
+    DeviceBuffer<rt3_dn_moments> dn_hist_mom[2];
+    DeviceBuffer<rt3_dn_guide> dn_hist_guide[2];
+    DeviceBuffer<float> dn_hist_length;
+    uint32_t dn_hist_cur = 0;
+    bool dn_hist_valid = false;
+    rt3_camera dn_hist_cam{};
+    uint32_t dn_hist_width = 0, dn_hist_height = 0;
+    uint64_t dn_hist_scene_id = 0;
+
     rt3_stats stats{};
     double upload_ms = 0.0, upload_h2d_ms = 0.0, upload_device_ms = 0.0; /* most recent scene upload */
 };
@@ -653,17 +665,16 @@ int check_denoise_inputs(rt3_ctx* ctx, const rt3_denoise_params* params, const c
     return RT3_OK;
 }
 
-/* The variance and `iterations` à-trous passes over prepared colour `col` and guides `guide`, ping-ponging through dn_col
- * (col itself is only read), the last pass remodulating by `albedo`; then the copies to the host. Ends the pass begun by
- * the caller, blocking; `launches` is the number of kernels the caller enqueued before. */
-int filter_to_host(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_px* col, const rt3_dn_guide* guide, const float* albedo, uint32_t launches,
-                   uint32_t* host_frame, float* host_rgb, cudaStream_t stream) {
+dim3 denoise_grid(uint32_t w, uint32_t h) { return dim3((w + RT3_DN_BLOCK_X - 1) / RT3_DN_BLOCK_X, (h + RT3_DN_BLOCK_Y - 1) / RT3_DN_BLOCK_Y); }
+
+/* The `iterations` à-trous passes over dn_col[0] (colour and variance) and guides `guide`, ping-ponging through dn_col, the
+ * last pass remodulating by `albedo` into dn_frame and dn_rgb; ends the timed kernels. `launches` is the number of
+ * kernels the caller enqueued before. */
+int enqueue_atrous(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_guide* guide, const float* albedo, uint32_t launches, bool want_rgb,
+                   cudaStream_t stream) {
     const uint32_t w = params->width, h = params->height, n_pow = (uint32_t) params->sigma_normal;
-    const size_t n = (size_t) w * h;
     const float sigma_l = params->sigma_luminance, sigma_z = params->sigma_depth;
-    const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid((w + RT3_DN_BLOCK_X - 1) / RT3_DN_BLOCK_X, (h + RT3_DN_BLOCK_Y - 1) / RT3_DN_BLOCK_Y);
-    denoise_variance_kernel<<<grid, block, 0, stream>>>(w, h, sigma_z, n_pow, col, guide, ctx->dn_col[0].ptr);
-    RT3_CUDA(cudaGetLastError());
+    const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid = denoise_grid(w, h);
     const bool gamma = !(ctx->accum_kp.flags & RT3_FLAG_NO_GAMMA);
     for (uint32_t i = 0; i < params->iterations; i++) {
         const rt3_dn_px* in = ctx->dn_col[i & 1u].ptr;
@@ -672,18 +683,38 @@ int filter_to_host(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_
             denoise_atrous_kernel<false><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, guide, out, nullptr, gamma, nullptr, nullptr);
         } else {
             denoise_atrous_kernel<true><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, guide, nullptr, albedo, gamma,
-                                                                    ctx->dn_frame.ptr, host_rgb ? ctx->dn_rgb.ptr : nullptr);
+                                                                    ctx->dn_frame.ptr, want_rgb ? ctx->dn_rgb.ptr : nullptr);
         }
         RT3_CUDA(cudaGetLastError());
     }
     RT3_CUDA(cudaEventRecord(ctx->ev_k1, stream));
     RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
-    ctx->stats.kernel_launches = launches + 1 + params->iterations;
+    ctx->stats.kernel_launches = launches + params->iterations;
+    return RT3_OK;
+}
+
+/* Copies the filtered frame and rgb to the host (after any copies the caller enqueued), ends the pass, blocking, and
+ * reads its statistics. */
+int read_back_denoised(rt3_ctx* ctx, size_t n, uint32_t* host_frame, float* host_rgb, cudaStream_t stream) {
     if (host_frame) { RT3_CUDA(cudaMemcpyAsync(host_frame, ctx->dn_frame.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream)); }
     if (host_rgb) { RT3_CUDA(cudaMemcpyAsync(host_rgb, ctx->dn_rgb.ptr, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, stream)); }
     int rc = end_pass(ctx, stream);
     if (rc != RT3_OK) { return rc; }
     return collect_stats(ctx);
+}
+
+/* The variance and `iterations` à-trous passes over prepared colour `col` and guides `guide`, ping-ponging through dn_col
+ * (col itself is only read), the last pass remodulating by `albedo`; then the copies to the host. Ends the pass begun by
+ * the caller, blocking; `launches` is the number of kernels the caller enqueued before. */
+int filter_to_host(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_px* col, const rt3_dn_guide* guide, const float* albedo, uint32_t launches,
+                   uint32_t* host_frame, float* host_rgb, cudaStream_t stream) {
+    const uint32_t w = params->width, h = params->height;
+    denoise_variance_kernel<<<denoise_grid(w, h), dim3(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), 0, stream>>>(w, h, params->sigma_depth, (uint32_t) params->sigma_normal,
+                                                                                                   col, guide, ctx->dn_col[0].ptr);
+    RT3_CUDA(cudaGetLastError());
+    int rc = enqueue_atrous(ctx, params, guide, albedo, launches + 1, host_rgb != nullptr, stream);
+    if (rc != RT3_OK) { return rc; }
+    return read_back_denoised(ctx, (size_t) w * h, host_frame, host_rgb, stream);
 }
 
 /* The filter's ping-pong buffers and outputs (plus the guides when `guide`), sized on first use. */
@@ -713,6 +744,54 @@ int denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame
                                                                            ctx->dn_col[1].ptr, ctx->dn_guide.ptr);
     RT3_CUDA(cudaGetLastError());
     return filter_to_host(ctx, params, ctx->dn_col[1].ptr, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, 1u, host_frame, host_rgb, stream);
+}
+
+/* rt3_denoise_temporal: rt3_denoise's checks and the temporal parameters', then the accumulation into the history not in
+ * use, its variance, the à-trous passes and the read-back, blocking. The history is dropped when the call proceeds and
+ * kept (swapped in) only when everything succeeded; a refusal changes nothing. */
+int denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* tp, uint32_t* host_frame, float* host_rgb, float* host_length) {
+    if (!ctx) { return fail(RT3_ERR_INVALID, "ctx is NULL"); }
+    if (!tp) { return fail(RT3_ERR_INVALID, "rt3_denoise_temporal: params is NULL"); }
+    int rc = check_denoise_inputs(ctx, &tp->filter, "rt3_denoise_temporal", false);
+    if (rc != RT3_OK) { return rc; }
+    if (const char* why = rt3_dn_check_temporal_params(tp)) { return fail(RT3_ERR_INVALID, "rt3_denoise_temporal: %s", why); }
+    RT3_CUDA(cudaSetDevice(ctx->device));
+    const rt3_kparams& kp = ctx->accum_kp;
+    const uint32_t w = kp.width, h = kp.height;
+    const size_t n = (size_t) w * h;
+    const bool have_prev = !tp->reset && ctx->dn_hist_valid && ctx->dn_hist_width == w && ctx->dn_hist_height == h && ctx->dn_hist_scene_id == ctx->scene_id;
+    ctx->dn_hist_valid = false;
+    const uint32_t cur = ctx->dn_hist_cur, next = cur ^ 1u;
+    if ((rc = reserve_denoise(ctx, n, true, host_rgb != nullptr)) != RT3_OK) { return rc; }
+    for (uint32_t i = 0; i < 2; i++) {
+        if ((rc = ctx->dn_hist_col[i].reserve(n)) != RT3_OK || (rc = ctx->dn_hist_mom[i].reserve(n)) != RT3_OK || (rc = ctx->dn_hist_guide[i].reserve(n)) != RT3_OK) {
+            return rc;
+        }
+    }
+    if (host_length && (rc = ctx->dn_hist_length.reserve(n)) != RT3_OK) { return rc; }
+    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
+    if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
+    const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid = denoise_grid(w, h);
+    denoise_temporal_kernel<<<grid, block, 0, stream>>>(kp, ctx->path_aovs_kp, ctx->path_aovs_cam, ctx->dn_hist_cam, *tp, have_prev, ctx->accum.ptr,
+                                                        ctx->aov_albedo.ptr, ctx->aov_normal.ptr, ctx->aov_t.ptr, ctx->dn_hist_col[cur].ptr,
+                                                        ctx->dn_hist_mom[cur].ptr, ctx->dn_hist_guide[cur].ptr, ctx->dn_hist_col[next].ptr,
+                                                        ctx->dn_hist_mom[next].ptr, ctx->dn_hist_guide[next].ptr, ctx->dn_col[1].ptr, ctx->dn_guide.ptr,
+                                                        host_length ? ctx->dn_hist_length.ptr : nullptr);
+    RT3_CUDA(cudaGetLastError());
+    const rt3_denoise_params& fp = tp->filter;
+    denoise_temporal_variance_kernel<<<grid, block, 0, stream>>>(w, h, fp.sigma_depth, (uint32_t) fp.sigma_normal, ctx->dn_col[1].ptr, ctx->dn_guide.ptr,
+                                                                 ctx->dn_hist_col[next].ptr, ctx->dn_hist_mom[next].ptr, ctx->dn_col[0].ptr);
+    RT3_CUDA(cudaGetLastError());
+    if ((rc = enqueue_atrous(ctx, &fp, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, 2u, host_rgb != nullptr, stream)) != RT3_OK) { return rc; }
+    if (host_length) { RT3_CUDA(cudaMemcpyAsync(host_length, ctx->dn_hist_length.ptr, n * sizeof(float), cudaMemcpyDeviceToHost, stream)); }
+    if ((rc = read_back_denoised(ctx, n, host_frame, host_rgb, stream)) != RT3_OK) { return rc; }
+    ctx->dn_hist_cur = next;
+    ctx->dn_hist_valid = true;
+    ctx->dn_hist_cam = ctx->path_aovs_cam;
+    ctx->dn_hist_width = w; ctx->dn_hist_height = h;
+    ctx->dn_hist_scene_id = ctx->scene_id;
+    return RT3_OK;
 }
 
 /* Where the planes of a stage of rt3_denoise_stage_words(w, h) words start (include/rt3cuda.h). */
@@ -1120,6 +1199,10 @@ int rt3_render_path_aovs(rt3_ctx* ctx, const rt3_camera* camera, const rt3_param
 
 int rt3_denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame, float* host_rgb) {
     return denoise(ctx, params, host_frame, host_rgb);
+}
+
+int rt3_denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* params, uint32_t* host_frame, float* host_rgb, float* host_history_length) {
+    return denoise_temporal(ctx, params, host_frame, host_rgb, host_history_length);
 }
 
 uint64_t rt3_denoise_stage_words(uint32_t width, uint32_t height) {

@@ -230,6 +230,23 @@ int rt3host_denoise(void* s, uint32_t width, uint32_t height, float focal, float
         if (rgb_out) { std::memcpy(rgb_out, rgb.data(), rgb.size() * sizeof(float)); }
     });
 }
+/* CudaRenderer::denoise_temporal with the reference camera (outputs as rt3host_denoise's). */
+int rt3host_denoise_temporal(void* s, uint32_t width, uint32_t height, float focal, float vw, float vh, const rt3_denoise_temporal_params* p, uint32_t* frame_out,
+                             float* rgb_out) {
+    HostScene* hs = (HostScene*) s;
+    if (!hs->renderer) { g_error = "create the renderer first"; return -1; }
+    return guarded([&] {
+        hs->camera.update(width, height, focal, vw, vh);
+        CudaDenoiseTemporalSettings st;
+        st.filter.iterations = p->filter.iterations; st.filter.sigma_luminance = p->filter.sigma_luminance;
+        st.filter.sigma_normal = p->filter.sigma_normal; st.filter.sigma_depth = p->filter.sigma_depth;
+        st.alpha_color = p->alpha_color; st.alpha_moments = p->alpha_moments; st.depth_tolerance = p->depth_tolerance; st.normal_cos = p->normal_cos;
+        std::vector<float> rgb;
+        hs->renderer->denoise_temporal(hs->camera, st, p->reset != 0, rgb_out ? &rgb : nullptr);
+        if (frame_out) { std::memcpy(frame_out, hs->camera.get_frame().d(), (size_t) width * height * sizeof(uint32_t)); }
+        if (rgb_out) { std::memcpy(rgb_out, rgb.data(), rgb.size() * sizeof(float)); }
+    });
+}
 int rt3host_camera_vectors(uint32_t width, uint32_t height, const float* look, float* out19) {
     return guarded([&] {
         Camera cam;

@@ -450,6 +450,25 @@ void CudaRenderer::denoise(Camera& camera, const CudaDenoiseSettings& settings, 
     check(rt3_get_stats(this->ctx, &this->last_stats), "Could not read the statistics");
 }
 
+void CudaRenderer::denoise_temporal(Camera& camera, const CudaDenoiseTemporalSettings& settings, bool reset, std::vector<float>* rgb) const {
+    if (!this->helpers.empty()) {
+        DLOG(fatal, "Temporal denoising needs a renderer on one device: with " + std::to_string(this->n_devices()) +
+                    " each context holds only its own rows of the frame, and the filter reaches across them.");
+    }
+    rt3_denoise_temporal_params params;
+    std::memset(&params, 0, sizeof params);
+    params.filter.width = camera.w(); params.filter.height = camera.h();
+    params.filter.iterations = settings.filter.iterations;
+    params.filter.sigma_luminance = settings.filter.sigma_luminance; params.filter.sigma_normal = settings.filter.sigma_normal;
+    params.filter.sigma_depth = settings.filter.sigma_depth;
+    params.alpha_color = settings.alpha_color; params.alpha_moments = settings.alpha_moments;
+    params.depth_tolerance = settings.depth_tolerance; params.normal_cos = settings.normal_cos;
+    params.reset = reset ? 1u : 0u;
+    if (rgb) { rgb->assign((size_t) params.filter.width * params.filter.height * 3, 0.0f); }
+    check(rt3_denoise_temporal(this->ctx, &params, camera.get_frame().d(), rgb ? rgb->data() : nullptr, nullptr), "Temporal denoising failed");
+    check(rt3_get_stats(this->ctx, &this->last_stats), "Could not read the statistics");
+}
+
 void CudaRenderer::write_path_aovs_pfm(const CudaPathAovs& aovs, const std::string& dir) const {
     const std::string base = dir.empty() ? std::string(".") : dir;
     write_pfm(base + "/albedo.pfm", aovs.width, aovs.height, 3, aovs.albedo.data());

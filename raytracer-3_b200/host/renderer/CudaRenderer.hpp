@@ -69,6 +69,12 @@ namespace RayTracer {
         float sigma_luminance = 4.0f, sigma_normal = 128.0f, sigma_depth = 1.0f;
     };
 
+    /* Parameters of CudaRenderer::denoise_temporal (rt3_denoise_temporal_params; SVGF's defaults). */
+    struct CudaDenoiseTemporalSettings {
+        CudaDenoiseSettings filter;
+        float alpha_color = 0.2f, alpha_moments = 0.2f, depth_tolerance = 0.05f, normal_cos = 0.9f;
+    };
+
     class CudaRenderer : public Renderer {
         rt3_ctx* ctx;                 /* first device: owns the frame when there are several */
         std::vector<rt3_ctx*> helpers; /* further devices (SURVEY 8e): each renders its row tiles straight into ctx's frame */
@@ -123,6 +129,9 @@ namespace RayTracer {
          * the linear float image (3 per pixel). One device only: each context of a renderer with several holds only its own
          * rows, and the filter reaches across them. */
         void denoise(Camera& camera, const CudaDenoiseSettings& settings = {}, std::vector<float>* rgb = nullptr) const;
+        /* denoise() with the history of the earlier calls reprojected through the camera's motion and accumulated
+         * (rt3_denoise_temporal; `reset` drops the history first). Render each frame with its own seed. One device only. */
+        void denoise_temporal(Camera& camera, const CudaDenoiseTemporalSettings& settings = {}, bool reset = false, std::vector<float>* rgb = nullptr) const;
         /* albedo.pfm and normal.pfm ("PF", 3 channels) and depth.pfm ("Pf", hit_t; +inf where the primary ray missed) in `dir`. */
         void write_path_aovs_pfm(const CudaPathAovs& aovs, const std::string& dir) const;
 
