@@ -442,18 +442,19 @@ class Context:
         self._check(self.lib.rt3_read_radiance(self.handle, _ptr(out), width, height))
         return out
 
-    def denoise(self, width, height, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
+    def denoise(self, width, height, **filter):
         """rt3_denoise: the last path-traced render of this (width x height) frame, filtered under the guidance of the last
-        render_path_aovs. Returns (frame [H, W] uint32 packed like render's, rgb [H, W, 3] float32 linear)."""
+        render_path_aovs; ``filter`` takes denoise_params' keywords. Returns (frame [H, W] uint32 packed like render's, rgb
+        [H, W, 3] float32 linear)."""
         frame = np.zeros((height, width), np.uint32)
         rgb = np.zeros((height, width, 3), np.float32)
-        p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
+        p = denoise_params(width, height, **filter)
         self._check(self.lib.rt3_denoise(self.handle, C.byref(p), _ptr(frame), _ptr(rgb)))
         return frame, rgb
 
     def denoise_temporal(self, width, height, reset=False, alpha_color=0.2, alpha_moments=0.2, depth_tolerance=0.05, normal_cos=0.9, **filter):
         """rt3_denoise_temporal: ``denoise`` with the context's history of earlier frames reprojected through the camera's motion
-        and accumulated (``reset`` drops it first); ``filter`` takes ``denoise``'s keywords. Render each frame with its own seed.
+        and accumulated (``reset`` drops it first); ``filter`` takes denoise_params' keywords. Render each frame with its own seed.
         Returns (frame [H, W] uint32, rgb [H, W, 3] float32, history_length [H, W] float32)."""
         frame = np.zeros((height, width), np.uint32)
         rgb = np.zeros((height, width, 3), np.float32)
@@ -462,19 +463,19 @@ class Context:
         self._check(self.lib.rt3_denoise_temporal(self.handle, C.byref(p), _ptr(frame), _ptr(rgb), _ptr(length)))
         return frame, rgb, length
 
-    def denoise_stage(self, width, height, stage_ptr, tag, stream_ptr=None, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
+    def denoise_stage(self, width, height, stage_ptr, tag, stream_ptr=None, **filter):
         """rt3_denoise_stage: this context's rows of a frame rendered in parts, prepared into the stage at ``stage_ptr`` (a device
-        pointer of denoise_stage_words(width, height) words, possibly mapped from another process) for frame ``tag``.
-        Asynchronous: ``stats()`` waits for it."""
-        p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
+        pointer of denoise_stage_words(width, height) words, possibly mapped from another process) for frame ``tag``;
+        ``filter`` takes denoise_params' keywords. Asynchronous: ``stats()`` waits for it."""
+        p = denoise_params(width, height, **filter)
         self._check(self.lib.rt3_denoise_stage(self.handle, C.byref(p), int(tag), C.c_void_p(stage_ptr), C.c_void_p(stream_ptr or 0)))
 
-    def denoise_staged(self, width, height, stage_ptr, tag, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0):
-        """rt3_denoise_staged: on the stage's owner, after every part staged frame ``tag``: the whole frame filtered from the stage.
-        Returns (frame [H, W] uint32, rgb [H, W, 3] float32) like ``denoise``."""
+    def denoise_staged(self, width, height, stage_ptr, tag, **filter):
+        """rt3_denoise_staged: on the stage's owner, after every part staged frame ``tag``: the whole frame filtered from the stage
+        (``filter``: denoise_params' keywords). Returns (frame [H, W] uint32, rgb [H, W, 3] float32) like ``denoise``."""
         frame = np.zeros((height, width), np.uint32)
         rgb = np.zeros((height, width, 3), np.float32)
-        p = denoise_params(width, height, iterations, sigma_luminance, sigma_normal, sigma_depth)
+        p = denoise_params(width, height, **filter)
         self._check(self.lib.rt3_denoise_staged(self.handle, C.byref(p), int(tag), C.c_void_p(stage_ptr), _ptr(frame), _ptr(rgb)))
         return frame, rgb
 

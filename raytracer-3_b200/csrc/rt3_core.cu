@@ -667,12 +667,17 @@ int check_denoise_inputs(rt3_ctx* ctx, const rt3_denoise_params* params, const c
 
 dim3 denoise_grid(uint32_t w, uint32_t h) { return dim3((w + RT3_DN_BLOCK_X - 1) / RT3_DN_BLOCK_X, (h + RT3_DN_BLOCK_Y - 1) / RT3_DN_BLOCK_Y); }
 
-/* The `iterations` à-trous passes over dn_col[0] (colour and variance) and guides `guide`, ping-ponging through dn_col, the
- * last pass remodulating by `albedo` into dn_frame and dn_rgb; ends the timed kernels. `launches` is the number of
- * kernels the caller enqueued before. */
-int enqueue_atrous(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_guide* guide, const float* albedo, uint32_t launches, bool want_rgb,
-                   cudaStream_t stream) {
+/* The stream rt3_read_radiance and the denoise calls enqueue on: the one of the render that filled the accumulators. */
+cudaStream_t accum_stream(const rt3_ctx* ctx) { return ctx->last_stream ? ctx->last_stream : ctx->stream; }
+
+/* The end of every filtering call, after the caller enqueued its preparation and variance kernels into dn_col[0] (colour
+ * and variance) and counted them: the `iterations` à-trous passes guided by `guide`, ping-ponging through dn_col, the last
+ * remodulating by `albedo` into dn_frame and dn_rgb; then the copies of the history length (when `host_length` is not
+ * NULL), the frame and rgb to the host. Ends the pass begun by the caller, blocking, and reads its statistics. */
+int atrous_to_host(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_guide* guide, const float* albedo, uint32_t* host_frame, float* host_rgb,
+                   float* host_length, cudaStream_t stream) {
     const uint32_t w = params->width, h = params->height, n_pow = (uint32_t) params->sigma_normal;
+    const size_t n = (size_t) w * h;
     const float sigma_l = params->sigma_luminance, sigma_z = params->sigma_depth;
     const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid = denoise_grid(w, h);
     const bool gamma = !(ctx->accum_kp.flags & RT3_FLAG_NO_GAMMA);
@@ -683,38 +688,19 @@ int enqueue_atrous(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_
             denoise_atrous_kernel<false><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, guide, out, nullptr, gamma, nullptr, nullptr);
         } else {
             denoise_atrous_kernel<true><<<grid, block, 0, stream>>>(w, h, 1u << i, sigma_l, sigma_z, n_pow, in, guide, nullptr, albedo, gamma,
-                                                                    ctx->dn_frame.ptr, want_rgb ? ctx->dn_rgb.ptr : nullptr);
+                                                                    ctx->dn_frame.ptr, host_rgb ? ctx->dn_rgb.ptr : nullptr);
         }
         RT3_CUDA(cudaGetLastError());
     }
     RT3_CUDA(cudaEventRecord(ctx->ev_k1, stream));
     RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
-    ctx->stats.kernel_launches = launches + params->iterations;
-    return RT3_OK;
-}
-
-/* Copies the filtered frame and rgb to the host (after any copies the caller enqueued), ends the pass, blocking, and
- * reads its statistics. */
-int read_back_denoised(rt3_ctx* ctx, size_t n, uint32_t* host_frame, float* host_rgb, cudaStream_t stream) {
+    ctx->stats.kernel_launches += params->iterations;
+    if (host_length) { RT3_CUDA(cudaMemcpyAsync(host_length, ctx->dn_hist_length.ptr, n * sizeof(float), cudaMemcpyDeviceToHost, stream)); }
     if (host_frame) { RT3_CUDA(cudaMemcpyAsync(host_frame, ctx->dn_frame.ptr, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, stream)); }
     if (host_rgb) { RT3_CUDA(cudaMemcpyAsync(host_rgb, ctx->dn_rgb.ptr, 3 * n * sizeof(float), cudaMemcpyDeviceToHost, stream)); }
     int rc = end_pass(ctx, stream);
     if (rc != RT3_OK) { return rc; }
     return collect_stats(ctx);
-}
-
-/* The variance and `iterations` à-trous passes over prepared colour `col` and guides `guide`, ping-ponging through dn_col
- * (col itself is only read), the last pass remodulating by `albedo`; then the copies to the host. Ends the pass begun by
- * the caller, blocking; `launches` is the number of kernels the caller enqueued before. */
-int filter_to_host(rt3_ctx* ctx, const rt3_denoise_params* params, const rt3_dn_px* col, const rt3_dn_guide* guide, const float* albedo, uint32_t launches,
-                   uint32_t* host_frame, float* host_rgb, cudaStream_t stream) {
-    const uint32_t w = params->width, h = params->height;
-    denoise_variance_kernel<<<denoise_grid(w, h), dim3(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), 0, stream>>>(w, h, params->sigma_depth, (uint32_t) params->sigma_normal,
-                                                                                                   col, guide, ctx->dn_col[0].ptr);
-    RT3_CUDA(cudaGetLastError());
-    int rc = enqueue_atrous(ctx, params, guide, albedo, launches + 1, host_rgb != nullptr, stream);
-    if (rc != RT3_OK) { return rc; }
-    return read_back_denoised(ctx, (size_t) w * h, host_frame, host_rgb, stream);
 }
 
 /* The filter's ping-pong buffers and outputs (plus the guides when `guide`), sized on first use. */
@@ -737,13 +723,17 @@ int denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame
     const rt3_kparams& kp = ctx->accum_kp;
     const size_t n = (size_t) kp.width * kp.height;
     if ((rc = reserve_denoise(ctx, n, true, host_rgb != nullptr)) != RT3_OK) { return rc; }
-    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
+    cudaStream_t stream = accum_stream(ctx);
     if ((rc = begin_pass(ctx, false, kp.height, stream, nullptr)) != RT3_OK) { return rc; }
     RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
     denoise_prepare_kernel<<<(unsigned) ((n + 255) / 256), 256, 0, stream>>>(kp, ctx->accum.ptr, ctx->aov_albedo.ptr, ctx->aov_normal.ptr, ctx->aov_t.ptr,
                                                                            ctx->dn_col[1].ptr, ctx->dn_guide.ptr);
     RT3_CUDA(cudaGetLastError());
-    return filter_to_host(ctx, params, ctx->dn_col[1].ptr, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, 1u, host_frame, host_rgb, stream);
+    denoise_variance_kernel<<<denoise_grid(kp.width, kp.height), dim3(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), 0, stream>>>(
+        kp.width, kp.height, params->sigma_depth, (uint32_t) params->sigma_normal, ctx->dn_col[1].ptr, ctx->dn_guide.ptr, ctx->dn_col[0].ptr);
+    RT3_CUDA(cudaGetLastError());
+    ctx->stats.kernel_launches += 2;
+    return atrous_to_host(ctx, params, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, host_frame, host_rgb, nullptr, stream);
 }
 
 /* rt3_denoise_temporal: rt3_denoise's checks and the temporal parameters', then the accumulation into the history not in
@@ -769,7 +759,7 @@ int denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* tp, uint32
         }
     }
     if (host_length && (rc = ctx->dn_hist_length.reserve(n)) != RT3_OK) { return rc; }
-    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
+    cudaStream_t stream = accum_stream(ctx);
     if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
     RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
     const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid = denoise_grid(w, h);
@@ -783,9 +773,8 @@ int denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* tp, uint32
     denoise_temporal_variance_kernel<<<grid, block, 0, stream>>>(w, h, fp.sigma_depth, (uint32_t) fp.sigma_normal, ctx->dn_col[1].ptr, ctx->dn_guide.ptr,
                                                                  ctx->dn_hist_col[next].ptr, ctx->dn_hist_mom[next].ptr, ctx->dn_col[0].ptr);
     RT3_CUDA(cudaGetLastError());
-    if ((rc = enqueue_atrous(ctx, &fp, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, 2u, host_rgb != nullptr, stream)) != RT3_OK) { return rc; }
-    if (host_length) { RT3_CUDA(cudaMemcpyAsync(host_length, ctx->dn_hist_length.ptr, n * sizeof(float), cudaMemcpyDeviceToHost, stream)); }
-    if ((rc = read_back_denoised(ctx, n, host_frame, host_rgb, stream)) != RT3_OK) { return rc; }
+    ctx->stats.kernel_launches += 2;
+    if ((rc = atrous_to_host(ctx, &fp, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, host_frame, host_rgb, host_length, stream)) != RT3_OK) { return rc; }
     ctx->dn_hist_cur = next;
     ctx->dn_hist_valid = true;
     ctx->dn_hist_cam = ctx->path_aovs_cam;
@@ -838,7 +827,7 @@ int denoise_stage(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame
     const rt3_kparams& kp = ctx->accum_kp;
     if (rt3_denoise_stage_words(kp.width, kp.height) == 0) { return fail(RT3_ERR_INVALID, "rt3_denoise_stage: a %ux%u frame does not fit in a stage", kp.width, kp.height); }
     RT3_CUDA(cudaSetDevice(ctx->device));
-    cudaStream_t stream = user_stream ? user_stream : ctx->last_stream ? ctx->last_stream : ctx->stream;
+    cudaStream_t stream = user_stream ? user_stream : accum_stream(ctx);
     const stage_view s = stage_planes(device_stage, kp.width, kp.height);
     if ((rc = begin_pass(ctx, false, kp.owned_rows, stream, nullptr)) != RT3_OK) { return rc; }
     RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
@@ -863,7 +852,7 @@ int denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t fram
     const uint32_t w = kp.width, h = kp.height;
     if (rt3_denoise_stage_words(w, h) == 0) { return fail(RT3_ERR_INVALID, "rt3_denoise_staged: a %ux%u frame does not fit in a stage", w, h); }
     RT3_CUDA(cudaSetDevice(ctx->device));
-    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream;
+    cudaStream_t stream = accum_stream(ctx);
     const stage_view s = stage_planes(const_cast<uint32_t*>(device_stage), w, h);
     std::vector<unsigned long long> rows(h);
     RT3_CUDA(cudaMemcpyAsync(rows.data(), s.fingerprint, h * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
@@ -880,7 +869,11 @@ int denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t fram
     if ((rc = reserve_denoise(ctx, (size_t) w * h, false, host_rgb != nullptr)) != RT3_OK) { return rc; }
     if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
     RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
-    return filter_to_host(ctx, params, s.col, s.guide, s.albedo, 0u, host_frame, host_rgb, stream);
+    denoise_variance_kernel<<<denoise_grid(w, h), dim3(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), 0, stream>>>(w, h, params->sigma_depth, (uint32_t) params->sigma_normal,
+                                                                                                   s.col, s.guide, ctx->dn_col[0].ptr);
+    RT3_CUDA(cudaGetLastError());
+    ctx->stats.kernel_launches += 1;
+    return atrous_to_host(ctx, params, s.guide, s.albedo, host_frame, host_rgb, nullptr, stream);
 }
 
 /* Reads back the timings and counters of the most recent render (synchronises its stream). */
@@ -1440,7 +1433,7 @@ int rt3_read_radiance(rt3_ctx* ctx, float* host_rgb, uint32_t width, uint32_t he
     DeviceBuffer<float> rgb;
     int rc = rgb.reserve(n);
     if (rc != RT3_OK) { return rc; }
-    cudaStream_t stream = ctx->last_stream ? ctx->last_stream : ctx->stream; /* behind the render that filled the accumulators */
+    cudaStream_t stream = accum_stream(ctx);
     RT3_CUDA(cudaMemsetAsync(rgb.ptr, 0, n * sizeof(float), stream));
     if (kp.n_pixels) {
         radiance_kernel<<<(unsigned) ((kp.n_pixels + 255ull) / 256ull), 256, 0, stream>>>(kp, ctx->accum.ptr, rgb.ptr);

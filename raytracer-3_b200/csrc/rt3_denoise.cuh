@@ -3,7 +3,7 @@
  * load, call it and store. Every kernel but the stage covers the whole frame (rt3_denoise needs part_count <= 1), one
  * thread per pixel.
  *
- *   denoise_prepare_kernel   : radiance (radiance_kernel's expression) / albedo -> colour + luminance, normal + depth -> guide.
+ *   denoise_prepare_kernel   : radiance (mean_radiance) / albedo -> colour + luminance, normal + depth -> guide.
  *   denoise_stage_kernel     : the same for a partition's owned rows, into a stage buffer (rt3_denoise_stage), + row fingerprints.
  *   denoise_variance_kernel  : 7x7 luminance variance.
  *   denoise_atrous_kernel<F> : one 5x5 pass at step 2^i; F = the last pass, which remodulates and resolves like resolve_kernel.
@@ -16,26 +16,37 @@
 
 #include "rt3_denoise.h"
 #include "rt3_device.cuh"
-#include "rt3_kernels.cuh" /* owned_row_to_global */
+#include "rt3_kernels.cuh" /* owned_row_to_global, mean_radiance */
 
 #define RT3_DN_BLOCK_X 32
 #define RT3_DN_BLOCK_Y 8
+
+/* Loads pixel idx of the render (its mean radiance) and of its albedo, normal and depth AOVs and prepares it
+ * (rt3_dn_prepare_px). Returns the depth; the albedo is returned in a[], for the stage kernel to store. */
+__device__ __forceinline__ float dn_load_prepare(const rt3_kparams& P, const unsigned long long* __restrict__ accum, const float* __restrict__ albedo,
+                                                 const float* __restrict__ normal, const float* __restrict__ depth, size_t idx, float a[3], rt3_dn_px* px,
+                                                 rt3_dn_guide* g) {
+    float c[3], n[3];
+#pragma unroll
+    for (int k = 0; k < 3; k++) {
+        c[k] = mean_radiance(P, accum, idx, k);
+        a[k] = albedo[3 * idx + k];
+        n[k] = normal[3 * idx + k];
+    }
+    const float z = depth[idx];
+    rt3_dn_prepare_px(c, a, n, z, px, g);
+    return z;
+}
 
 __global__ void __launch_bounds__(256) denoise_prepare_kernel(rt3_kparams P, const unsigned long long* __restrict__ accum, const float* __restrict__ albedo,
                                                              const float* __restrict__ normal, const float* __restrict__ depth, rt3_dn_px* __restrict__ col,
                                                              rt3_dn_guide* __restrict__ guide) {
     const unsigned long long idx = (unsigned long long) blockIdx.x * blockDim.x + threadIdx.x;
     if (idx >= P.n_pixels) { return; }
-    float c[3], a[3], n[3];
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        c[k] = (float) ((double) accum[3 * idx + k] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE));
-        a[k] = albedo[3 * idx + k];
-        n[k] = normal[3 * idx + k];
-    }
+    float a[3];
     rt3_dn_px px;
     rt3_dn_guide g;
-    rt3_dn_prepare_px(c, a, n, depth[idx], &px, &g);
+    dn_load_prepare(P, accum, albedo, normal, depth, idx, a, &px, &g);
     col[idx] = px;
     guide[idx] = g;
 }
@@ -52,16 +63,10 @@ __global__ void __launch_bounds__(256) denoise_stage_kernel(rt3_kparams P, const
     const uint32_t local_row = (uint32_t) (p / P.width), x = (uint32_t) (p - (unsigned long long) local_row * P.width);
     const uint32_t y = owned_row_to_global(P, local_row);
     const size_t idx = (size_t) y * P.width + x;
-    float c[3], a[3], n[3];
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        c[k] = (float) ((double) accum[3 * idx + k] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE));
-        a[k] = albedo[3 * idx + k];
-        n[k] = normal[3 * idx + k];
-    }
+    float a[3];
     rt3_dn_px px;
     rt3_dn_guide g;
-    rt3_dn_prepare_px(c, a, n, depth[idx], &px, &g);
+    dn_load_prepare(P, accum, albedo, normal, depth, idx, a, &px, &g);
     col[idx] = px;
     guide[idx] = g;
 #pragma unroll
@@ -115,17 +120,10 @@ __global__ void __launch_bounds__(RT3_DN_BLOCK_X * RT3_DN_BLOCK_Y) denoise_tempo
     const uint32_t x = blockIdx.x * RT3_DN_BLOCK_X + threadIdx.x, y = blockIdx.y * RT3_DN_BLOCK_Y + threadIdx.y;
     if (x >= w || y >= h) { return; }
     const size_t idx = (size_t) y * w + x;
-    float c[3], a[3], n[3];
-#pragma unroll
-    for (int k = 0; k < 3; k++) {
-        c[k] = (float) ((double) accum[3 * idx + k] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE));
-        a[k] = albedo[3 * idx + k];
-        n[k] = normal[3 * idx + k];
-    }
+    float a[3];
     rt3_dn_px e;
     rt3_dn_guide g;
-    const float z = depth[idx];
-    rt3_dn_prepare_px(c, a, n, z, &e, &g);
+    const float z = dn_load_prepare(P, accum, albedo, normal, depth, idx, a, &e, &g);
     int have = 0;
     float px = 0.0f, py = 0.0f, dist = 0.0f;
     if (have_prev) {

@@ -1543,6 +1543,12 @@ __global__ void path_aov_resolve_kernel(rt3_kparams P, const unsigned long long*
     }
 }
 
+/* Mean radiance of channel k of pixel idx over the resolve_spp samples in the accumulators: the one expression that
+ * resolve_kernel, radiance_kernel and the denoiser's input kernels share. */
+__device__ __forceinline__ float mean_radiance(const rt3_kparams& P, const unsigned long long* __restrict__ accum, size_t idx, int k) {
+    return (float) ((double) accum[3 * idx + k] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE));
+}
+
 /* Mean over samples, gamma 2, reference packing (SequentialRenderer.cpp:297). */
 __global__ void resolve_kernel(rt3_kparams P, const unsigned long long* __restrict__ accum, uint32_t* __restrict__ frame) {
     unsigned long long p = (unsigned long long) blockIdx.x * blockDim.x + threadIdx.x;
@@ -1553,7 +1559,7 @@ __global__ void resolve_kernel(rt3_kparams P, const unsigned long long* __restri
     uint32_t ch[3];
 #pragma unroll
     for (int c = 0; c < 3; c++) {
-        float m = (float) ((double) accum[3 * idx + c] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE));
+        float m = mean_radiance(P, accum, idx, c);
         if (gamma) { m = sqrtf(m); }
         ch[c] = unorm8(m);
     }
@@ -1567,7 +1573,7 @@ __global__ void radiance_kernel(rt3_kparams P, const unsigned long long* __restr
     uint32_t local_row = (uint32_t) (p / P.width), x = (uint32_t) (p - (unsigned long long) local_row * P.width);
     size_t idx = (size_t) owned_row_to_global(P, local_row) * P.width + x;
 #pragma unroll
-    for (int c = 0; c < 3; c++) { rgb[3 * idx + c] = (float) ((double) accum[3 * idx + c] / ((double) P.resolve_spp * (double) RT3_ACC_SCALE)); }
+    for (int c = 0; c < 3; c++) { rgb[3 * idx + c] = mean_radiance(P, accum, idx, c); }
 }
 
 /* Clears the accumulators of the owned rows. */

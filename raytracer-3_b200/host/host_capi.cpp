@@ -40,6 +40,12 @@ namespace {
         catch (std::exception& e) { g_error = e.what(); return -1; }
     }
     glm::vec3 v3(const float* p) { return glm::vec3(p[0], p[1], p[2]); }
+    /* The settings CudaRenderer::denoise turns back into `p` (its width and height come from the camera). */
+    CudaDenoiseSettings denoise_settings_of(const rt3_denoise_params& p) {
+        CudaDenoiseSettings st;
+        st.iterations = p.iterations; st.sigma_luminance = p.sigma_luminance; st.sigma_normal = p.sigma_normal; st.sigma_depth = p.sigma_depth;
+        return st;
+    }
 }
 
 extern "C" {
@@ -222,10 +228,8 @@ int rt3host_denoise(void* s, uint32_t width, uint32_t height, float focal, float
     if (!hs->renderer) { g_error = "create the renderer first"; return -1; }
     return guarded([&] {
         hs->camera.update(width, height, focal, vw, vh);
-        CudaDenoiseSettings st;
-        st.iterations = p->iterations; st.sigma_luminance = p->sigma_luminance; st.sigma_normal = p->sigma_normal; st.sigma_depth = p->sigma_depth;
         std::vector<float> rgb;
-        hs->renderer->denoise(hs->camera, st, rgb_out ? &rgb : nullptr);
+        hs->renderer->denoise(hs->camera, denoise_settings_of(*p), rgb_out ? &rgb : nullptr);
         if (frame_out) { std::memcpy(frame_out, hs->camera.get_frame().d(), (size_t) width * height * sizeof(uint32_t)); }
         if (rgb_out) { std::memcpy(rgb_out, rgb.data(), rgb.size() * sizeof(float)); }
     });
@@ -238,8 +242,7 @@ int rt3host_denoise_temporal(void* s, uint32_t width, uint32_t height, float foc
     return guarded([&] {
         hs->camera.update(width, height, focal, vw, vh);
         CudaDenoiseTemporalSettings st;
-        st.filter.iterations = p->filter.iterations; st.filter.sigma_luminance = p->filter.sigma_luminance;
-        st.filter.sigma_normal = p->filter.sigma_normal; st.filter.sigma_depth = p->filter.sigma_depth;
+        st.filter = denoise_settings_of(p->filter);
         st.alpha_color = p->alpha_color; st.alpha_moments = p->alpha_moments; st.depth_tolerance = p->depth_tolerance; st.normal_cos = p->normal_cos;
         std::vector<float> rgb;
         hs->renderer->denoise_temporal(hs->camera, st, p->reset != 0, rgb_out ? &rgb : nullptr);

@@ -435,32 +435,34 @@ void CudaRenderer::render_path_aovs(const Camera& camera, CudaPathAovs& out) con
     this->last_stats = total;
 }
 
-void CudaRenderer::denoise(Camera& camera, const CudaDenoiseSettings& settings, std::vector<float>* rgb) const {
-    if (!this->helpers.empty()) {
-        DLOG(fatal, "Denoising needs a renderer on one device: with " + std::to_string(this->n_devices()) +
-                    " each context holds only its own rows of the frame, and the filter reaches across them.");
+namespace {
+    /* The filter's parameters for `camera`'s frame. Denoising needs a renderer on one device: with several, each context
+     * holds only its own rows of the frame, and the filter reaches across them. `what` names the call in the refusal. */
+    rt3_denoise_params denoise_params_of(const CudaDenoiseSettings& settings, const Camera& camera, size_t n_devices, const char* what) {
+        if (n_devices > 1) {
+            DLOG(fatal, std::string(what) + " needs a renderer on one device: with " + std::to_string(n_devices) +
+                        " each context holds only its own rows of the frame, and the filter reaches across them.");
+        }
+        rt3_denoise_params params;
+        std::memset(&params, 0, sizeof params);
+        params.width = camera.w(); params.height = camera.h();
+        params.iterations = settings.iterations;
+        params.sigma_luminance = settings.sigma_luminance; params.sigma_normal = settings.sigma_normal; params.sigma_depth = settings.sigma_depth;
+        return params;
     }
-    rt3_denoise_params params;
-    std::memset(&params, 0, sizeof params);
-    params.width = camera.w(); params.height = camera.h();
-    params.iterations = settings.iterations;
-    params.sigma_luminance = settings.sigma_luminance; params.sigma_normal = settings.sigma_normal; params.sigma_depth = settings.sigma_depth;
+}
+
+void CudaRenderer::denoise(Camera& camera, const CudaDenoiseSettings& settings, std::vector<float>* rgb) const {
+    const rt3_denoise_params params = denoise_params_of(settings, camera, this->n_devices(), "Denoising");
     if (rgb) { rgb->assign((size_t) params.width * params.height * 3, 0.0f); }
     check(rt3_denoise(this->ctx, &params, camera.get_frame().d(), rgb ? rgb->data() : nullptr), "Denoising failed");
     check(rt3_get_stats(this->ctx, &this->last_stats), "Could not read the statistics");
 }
 
 void CudaRenderer::denoise_temporal(Camera& camera, const CudaDenoiseTemporalSettings& settings, bool reset, std::vector<float>* rgb) const {
-    if (!this->helpers.empty()) {
-        DLOG(fatal, "Temporal denoising needs a renderer on one device: with " + std::to_string(this->n_devices()) +
-                    " each context holds only its own rows of the frame, and the filter reaches across them.");
-    }
     rt3_denoise_temporal_params params;
     std::memset(&params, 0, sizeof params);
-    params.filter.width = camera.w(); params.filter.height = camera.h();
-    params.filter.iterations = settings.filter.iterations;
-    params.filter.sigma_luminance = settings.filter.sigma_luminance; params.filter.sigma_normal = settings.filter.sigma_normal;
-    params.filter.sigma_depth = settings.filter.sigma_depth;
+    params.filter = denoise_params_of(settings.filter, camera, this->n_devices(), "Temporal denoising");
     params.alpha_color = settings.alpha_color; params.alpha_moments = settings.alpha_moments;
     params.depth_tolerance = settings.depth_tolerance; params.normal_cos = settings.normal_cos;
     params.reset = reset ? 1u : 0u;

@@ -1,8 +1,8 @@
 """Loaders for the path-traced AOVs (TEST INFRASTRUCTURE): the CPU restatement ``tests/path_aov_oracle.c`` (the oracle's
 closest-hit code compiled together with the AOV pass) and the host backend's ``render_path_aovs`` / ``write_path_aovs_pfm``.
 
-The restatement is compiled on first use into a temporary directory, keyed by the hash of its sources, so that the
-repository tree is never written to."""
+The restatements under tests/ are compiled on first use into a temporary directory, keyed by the hash of their sources,
+so that the repository tree is never written to (``load_restatement``, which tests/denoise_lib.py uses too)."""
 import ctypes as C
 import hashlib
 import os
@@ -22,17 +22,24 @@ AOV_KEYS = ("hit_prim", "hit_entity", "hit_t", "albedo", "normal")
 _oracle = None
 
 
+def load_restatement(name, sources):
+    """The restatement sources[0] (which includes the rest of `sources`) compiled with the oracle's flags, loaded. The
+    library is named after `name` and the hash of all the sources; a concurrent first use by another process is harmless
+    (each compiles to its own file, then renames it into place)."""
+    digest = hashlib.sha256(b"".join(open(p, "rb").read() for p in sources)).hexdigest()[:16]
+    path = os.path.join(tempfile.gettempdir(), f"rt3_{name}_oracle_{os.getuid()}_{digest}.so")
+    if not os.path.exists(path):
+        tmp = f"{path}.{os.getpid()}"
+        subprocess.run([os.environ.get("CC", "gcc"), "-std=c11", "-O2", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-shared", "-pthread",
+                        "-Wall", "-Wextra", "-I", os.path.join(ROOT, "include"), "-o", tmp, sources[0], "-lm"], check=True)
+        os.replace(tmp, path)
+    return C.CDLL(path)
+
+
 def oracle_lib():
     global _oracle
     if _oracle is None:
-        digest = hashlib.sha256(b"".join(open(p, "rb").read() for p in SOURCES)).hexdigest()[:16]
-        path = os.path.join(tempfile.gettempdir(), f"rt3_path_aov_oracle_{os.getuid()}_{digest}.so")
-        if not os.path.exists(path):
-            tmp = f"{path}.{os.getpid()}"
-            subprocess.run([os.environ.get("CC", "gcc"), "-std=c11", "-O2", "-ffp-contract=off", "-fno-fast-math", "-fPIC", "-shared", "-pthread",
-                            "-Wall", "-Wextra", "-I", os.path.join(ROOT, "include"), "-o", tmp, SOURCES[0], "-lm"], check=True)
-            os.replace(tmp, path)
-        lib = C.CDLL(path)
+        lib = load_restatement("path_aov", SOURCES)
         lib.orc_render_path_aovs.argtypes = [C.POINTER(abi.Scene), C.POINTER(abi.Camera), C.POINTER(abi.Params), C.POINTER(abi.PathAovs), C.c_int]
         _oracle = lib
     return _oracle

@@ -1,16 +1,13 @@
 """rt3_denoise_temporal without a GPU: the header's reprojection and accumulation (include/rt3_denoise.h) through the CPU
-restatement (tests/denoise_temporal_oracle.c) on hand-checkable cases, against the float64 reference (tests/denoise_temporal_ref.py), and
-with single-rule mutations of that reference; the parameter checks; the ABI; the new kernels' resources."""
+restatement (tests/denoise_oracle.c) on hand-checkable cases, against the float64 reference (tests/denoise_temporal_ref.py), and
+with single-rule mutations of that reference; the parameter checks; the ABI. The kernels' resources are checked in
+tests/test_sass_denoise.py."""
 import ctypes as C
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 
 import denoise_lib as dl
-import denoise_temporal_lib as dtl
 import denoise_temporal_ref as tref
 from rt3_b200 import abi
 
@@ -80,7 +77,7 @@ def test_unchanged_camera_maps_every_pixel_to_itself(lens):
     rays[:, :3] += rng.normal(0, 0.05, (len(rays), 3)).astype(f32)            # lens offsets
     depth = rng.uniform(0.5, 50, len(rays)).astype(f32)
     depth[::7] = np.inf
-    pos = dtl.reproject(cam, cam, w, h, xy, rays, depth)
+    pos = dl.reproject(cam, cam, w, h, xy, rays, depth)
     assert np.all(pos[:, 3] == 1)
     assert np.array_equal(pos[:, :2], xy)
 
@@ -94,7 +91,7 @@ def test_image_plane_pan_moves_by_k(k):
     rays, xy = rays_of(cur, w, h)
     depth = np.random.default_rng(2).uniform(1, 20, len(rays)).astype(f32)
     depth[::5] = np.inf
-    pos = dtl.reproject(cur, prev, w, h, xy, rays, depth)
+    pos = dl.reproject(cur, prev, w, h, xy, rays, depth)
     assert np.all(pos[:, 3] == 1)
     assert np.max(np.abs(pos[:, 0] - (xy[:, 0] + k))) < 1e-3
     assert np.max(np.abs(pos[:, 1] - xy[:, 1])) < 1e-3
@@ -105,7 +102,7 @@ def test_point_behind_the_previous_camera_has_no_history():
     cur = abi.reference_camera(w, h)
     prev = shifted(cur, origin=(0, 0, -10), llc=(0, 0, -10))                  # 10 units further along -z, looking the same way
     rays, xy = rays_of(cur, w, h)
-    pos = dtl.reproject(cur, prev, w, h, xy, rays, np.full(len(rays), 1.0, f32))  # points near z = -1: behind the previous camera
+    pos = dl.reproject(cur, prev, w, h, xy, rays, np.full(len(rays), 1.0, f32))  # points near z = -1: behind the previous camera
     assert np.all(pos[:, 3] == 0)
 
 
@@ -113,7 +110,7 @@ def run(frames, w, h, **kw):
     """Runs the restatement over [(camera, inputs, reset)], returns the (frame, rgb, length, history) of every call."""
     hist, out = None, []
     for cam, ins, reset in frames:
-        res = dtl.oracle_denoise_temporal(*ins, cam, params(w, h), hist, reset=reset, **kw)
+        res = dl.oracle_denoise_temporal(*ins, cam, params(w, h), hist, reset=reset, **kw)
         hist = res[3]
         out.append(res)
     return out
@@ -203,7 +200,7 @@ def test_reset_and_size_change_drop_the_history():
     res = run([(cam, ins, False), (cam, ins, False), (cam, ins, True), (cam, ins, False)], w, h)
     assert [float(r[2].max()) for r in res] == [1, 2, 1, 2]
     cam2 = abi.reference_camera(w + 1, h)
-    big = dtl.oracle_denoise_temporal(*plane_scene(cam2, w + 1, h), cam2, params(w + 1, h), res[-1][3])
+    big = dl.oracle_denoise_temporal(*plane_scene(cam2, w + 1, h), cam2, params(w + 1, h), res[-1][3])
     assert np.all(big[2] == 1)
 
 
@@ -213,13 +210,13 @@ def test_reset_and_size_change_drop_the_history():
     (dict(normal_cos=-1.5), "normal_cos"), (dict(normal_cos=float("nan")), "normal_cos"), (dict(iterations=0), "iterations"),
     (dict(sigma_normal=0.5), "sigma_normal")])
 def test_invalid_parameters_are_refused_with_a_message(bad, msg):
-    got = dtl.check_temporal_params(width=8, height=8, **bad)
+    got = dl.check_temporal_params(width=8, height=8, **bad)
     assert got is not None and got.startswith(msg), got
 
 
 def test_valid_parameter_edges_are_accepted():
     for ok in (dict(), dict(alpha_color=1.0, alpha_moments=1.0), dict(normal_cos=-1.0), dict(normal_cos=1.0), dict(depth_tolerance=1e30)):
-        assert dtl.check_temporal_params(width=8, height=8, **ok) is None, ok
+        assert dl.check_temporal_params(width=8, height=8, **ok) is None, ok
 
 
 # ---- the float64 reference ---------------------------------------------------------------------------------------------
@@ -240,8 +237,8 @@ def sequence_case(kind, lens, frames, w=27, h=19):
         ins = plane_scene(cam, w, h, sky_rows=4 + i % 2, seed=i)
         ins = (ins[0], ins[1], ins[2], (ins[3] * f32(1 + 0.02 * np.sin(np.arange(w) / 3.0))).astype(f32))
         p = params(w, h, seed=7 + i, flags=0)
-        _, _, _, hist = dtl.oracle_denoise_temporal(*ins, cam, p, hist)
-        r = yield hist, ins, dtl.primary_rays(cam, p), cam, ref_hist
+        _, _, _, hist = dl.oracle_denoise_temporal(*ins, cam, p, hist)
+        r = yield hist, ins, dl.primary_rays(cam, p), cam, ref_hist
         ref_hist = r["history"]
 
 
@@ -292,7 +289,7 @@ def test_mutations_are_far_from_the_restatement(mutation):
     assert worst > 10 * TAU, f"{mutation}: at most {worst} from the restatement"
 
 
-# ---- ABI and resources ------------------------------------------------------------------------------------------------
+# ---- ABI ------------------------------------------------------------------------------------------------------------
 
 def test_abi_symbol_and_layout(built):
     assert "rt3_denoise_temporal" in abi.EXPORTED_SYMBOLS
@@ -304,14 +301,3 @@ def test_abi_symbol_and_layout(built):
     assert (p.alpha_color, p.alpha_moments, p.depth_tolerance, p.normal_cos, p.reset) == (f32(0.2), f32(0.2), f32(0.05), f32(0.9), 0)
     assert (p.filter.iterations, p.filter.sigma_luminance, p.filter.sigma_normal, p.filter.sigma_depth) == (5, 4.0, 128.0, 1.0)
 
-
-@pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump not on PATH")
-@pytest.mark.parametrize("needle", ["denoise_temporal_kernel", "denoise_temporal_variance_kernel"])
-def test_new_kernels_keep_to_registers(built, needle):
-    text = subprocess.run(["cuobjdump", "-res-usage", abi.CORE_LIB_PATH], check=True, capture_output=True, text=True).stdout
-    found = [(m.group(1), int(m.group(2)), int(m.group(3)), int(m.group(4))) for m in
-             re.finditer(r"Function (\S+):\s*\n\s*REG:(\d+) STACK:(\d+) SHARED:\d+ LOCAL:(\d+)", text) if re.search(rf"\d{needle}", m.group(1))]
-    assert len(found) == 1, found
-    name, reg, stack, local = found[0]
-    assert local == 0 and stack == 0, f"{name}: {local} bytes of local memory, {stack} bytes of stack"
-    assert reg <= 64, f"{name}: {reg} registers"

@@ -1,5 +1,5 @@
 """rt3_denoise_temporal on the GPU: every frame of camera sequences bit for bit against the CPU restatement
-(tests/denoise_temporal_oracle.c) fed the same read_radiance / render_path_aovs arrays and carrying its own history; the contracts
+(tests/denoise_oracle.c) fed the same read_radiance / render_path_aovs arrays and carrying its own history; the contracts
 (no history: rt3_denoise; an unchanged camera: n = the call count; a pan: the entering columns start again; a new scene
 upload or size: n = 1); every refusal without a change; the other calls' state left alone; quality against rt3_denoise;
 the host backend."""
@@ -7,7 +7,6 @@ import numpy as np
 import pytest
 
 import denoise_lib as dl
-import denoise_temporal_lib as dtl
 import fullsize as fs
 import oraclelib as ol
 from rt3_b200 import abi, scenes
@@ -73,7 +72,7 @@ class Sequence:
 
     def denoise(self, reset=False):
         gpu = self.ctx.denoise_temporal(self.w, self.h, reset=reset, **self.dn)
-        *cpu, self.history = dtl.oracle_denoise_temporal(self.rgb, self.aov["albedo"], self.aov["normal"], self.aov["hit_t"], self.cam, self.aov_params,
+        *cpu, self.history = dl.oracle_denoise_temporal(self.rgb, self.aov["albedo"], self.aov["normal"], self.aov["hit_t"], self.cam, self.aov_params,
                                                         self.history, scene=self.scene, flags=self.flags, reset=reset, **self.dn)
         return gpu, tuple(cpu)
 
@@ -313,11 +312,11 @@ def test_host_backend(built):
     pal.host_path_aovs(hs, w, h, 5, focal=1.0)
     plain = dl.host_denoise(hs, w, h, focal=1.0)
     for i in range(4):
-        got = dtl.host_denoise_temporal(hs, w, h, focal=1.0, reset=i == 0)
+        got = dl.host_denoise_temporal(hs, w, h, focal=1.0, reset=i == 0)
         same = np.array_equal(got[0], plain[0]) and np.array_equal(got[1].view(np.uint32), plain[1].view(np.uint32))
         assert same == (i < 3), i
     multi = host_rtiow(w, h, True)
     multi.render(w, h, focal=1.0)
     pal.host_path_aovs(multi, w, h, 5, focal=1.0)
     with pytest.raises(hostlib.HostError, match="one device"):
-        dtl.host_denoise_temporal(multi, w, h, focal=1.0)
+        dl.host_denoise_temporal(multi, w, h, focal=1.0)

@@ -1,5 +1,6 @@
-"""The denoiser's kernels (rt3_denoise) keep to registers (no GPU needed: cuobjdump on librt3cuda.so): no local memory in any
-of them, no stack but the division slow path's, and the register counts ptxas reports leave every 256-thread CTA room for full occupancy (at most 64 per thread,
+"""The denoiser's kernels (rt3_denoise, the stage of a frame denoised in parts, rt3_denoise_temporal) keep to registers (no
+GPU needed: cuobjdump on librt3cuda.so): no local memory in any of them, no stack but the division slow path's, and the
+register counts ptxas reports leave every 256-thread CTA room for full occupancy (at most 64 per thread,
 65 536 / (256 * 4)). The existing kernels were left unchanged by them; DESIGN.md 3.8 says how that was checked."""
 import re
 import shutil
@@ -11,7 +12,9 @@ from rt3_b200 import abi
 
 pytestmark = pytest.mark.skipif(shutil.which("cuobjdump") is None, reason="cuobjdump not on PATH")
 
-KERNELS = ["denoise_prepare_kernel", "denoise_variance_kernel", "denoise_atrous_kernelILb0E", "denoise_atrous_kernelILb1E"]
+# the kernel's name and template arguments as mangled, without the length of the name that precedes them
+KERNELS = ["denoise_prepare_kernel", "denoise_variance_kernel", "denoise_atrous_kernelILb0E", "denoise_atrous_kernelILb1E", "denoise_stage_kernel",
+           "denoise_temporal_kernel", "denoise_temporal_variance_kernel"]
 
 
 @pytest.fixture(scope="module")
@@ -23,7 +26,8 @@ def resources(built):
 
 @pytest.mark.parametrize("needle", KERNELS)
 def test_no_local_memory_and_few_registers(resources, needle):
-    found = [r for r in resources if needle in r[0]]
+    kernel = needle.split("ILb")[0]
+    found = [r for r in resources if r[0].startswith(f"_Z{len(kernel)}{needle}")]
     assert len(found) == 1, found
     name, reg, stack, local = found[0]
     assert local == 0, f"{name}: {local} bytes of local memory"
