@@ -314,7 +314,8 @@ typedef struct rt3_denoise_temporal_params {
  * Writes host_frame and host_rgb as rt3_denoise does, and each pixel's new history length to host_history_length; any
  * may be NULL. Blocking. A refused call (RT3_ERR_INVALID) changes nothing; a call that fails with a CUDA error drops the
  * history. The accumulators, the AOV buffers and the RT3_FLAG_ACCUMULATE state are not touched, and rt3_denoise is not
- * affected by it. rt3_get_stats then describes this call (device_ms, kernel_launches, rays = 0). */
+ * affected by it. rt3_get_stats then describes this call (device_ms, kernel_launches, rays = 0). The history is the one
+ * rt3_denoise_staged_temporal uses on this context. */
 int rt3_denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* params, uint32_t* host_frame, float* host_rgb,
                          float* host_history_length);
 
@@ -359,6 +360,25 @@ int rt3_denoise_stage(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t f
  * RT3_FLAG_ACCUMULATE state are not touched; rt3_get_stats then describes this call (device_ms of the filter). */
 int rt3_denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, const uint32_t* device_stage,
                        uint32_t* host_frame, float* host_rgb);
+
+/* rt3_denoise_staged with temporal accumulation: the counterpart of rt3_denoise_temporal for a frame rendered in parts.
+ * On the stage's owner, after every part's rt3_denoise_stage for frame_tag has completed (the parts stage exactly as for
+ * rt3_denoise_staged and hold no history). Checks and refuses what rt3_denoise_staged does (NULL device_stage, a frame
+ * too large for a stage, every row whose fingerprint differs from the owner's, naming the first and the count), plus
+ * NULL params and the temporal parameters as rt3_denoise_temporal checks them; messages name
+ * rt3_denoise_staged_temporal. Each pixel's primary ray is regenerated on the owner from the global pixel index, the
+ * camera, the AOV call's seed, first_sample and RT3_FLAG_NO_JITTER, which the fingerprints prove every part shared, so
+ * the owner reprojects rows it did not render. The history is the owner's rt3_denoise_temporal history, with the same
+ * rules: dropped on reset, when there is none, or when the size or the owner's scene upload differ, and kept only when
+ * a call succeeds. Every part must therefore upload a new scene when the owner does. For each frame of a sequence the
+ * result (host_frame, host_rgb, host_history_length; any may be NULL) is bit-equal to rt3_denoise_temporal over
+ * one-context renders of the same frames, so a sequence may mix both calls on the owner's context and still gives the
+ * bits of an all-one-context sequence; a call with no usable history is bit-equal to rt3_denoise_staged. Blocking. A
+ * refused call (RT3_ERR_INVALID) changes nothing, the stage and the history included; a CUDA error drops the history.
+ * The accumulators, the AOV buffers and the RT3_FLAG_ACCUMULATE state are only read; rt3_get_stats then describes this
+ * call (device_ms, kernel_launches = 2 + iterations, rays = 0). */
+int rt3_denoise_staged_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* params, uint64_t frame_tag, const uint32_t* device_stage,
+                                uint32_t* host_frame, float* host_rgb, float* host_history_length);
 
 /* Device-resident variant for multi-GPU plumbing: renders this partition's
  * rows into `device_frame` (a device pointer to width*height uint32, full-frame

@@ -250,6 +250,7 @@ def load_core():
     lib.rt3_denoise_stage_words.restype = C.c_uint64
     lib.rt3_denoise_stage.argtypes = [vp, C.POINTER(DenoiseParams), C.c_uint64, vp, vp]
     lib.rt3_denoise_staged.argtypes = [vp, C.POINTER(DenoiseParams), C.c_uint64, vp, vp, vp]
+    lib.rt3_denoise_staged_temporal.argtypes = [vp, C.POINTER(DenoiseTemporalParams), C.c_uint64, vp, vp, vp, vp]
     lib.rt3_get_stats.argtypes = [vp, C.POINTER(Stats)]
     lib.rt3_measure_fma_peak.argtypes = [vp, C.POINTER(C.c_double)]
     _core = lib
@@ -263,7 +264,8 @@ EXPORTED_SYMBOLS = [
     "rt3_frame_alloc", "rt3_frame_free", "rt3_frame_export", "rt3_frame_import", "rt3_frame_release",
     "rt3_frame_attach", "rt3_frame_read",
     "rt3_uv_sphere_faces", "rt3_uv_sphere_vertices", "rt3_tessellate_spheres",
-    "rt3_read_radiance", "rt3_denoise", "rt3_denoise_temporal", "rt3_denoise_stage_words", "rt3_denoise_stage", "rt3_denoise_staged", "rt3_get_stats", "rt3_measure_fma_peak",
+    "rt3_read_radiance", "rt3_denoise", "rt3_denoise_temporal", "rt3_denoise_stage_words", "rt3_denoise_stage", "rt3_denoise_staged",
+    "rt3_denoise_staged_temporal", "rt3_get_stats", "rt3_measure_fma_peak",
 ]
 
 
@@ -478,6 +480,18 @@ class Context:
         p = denoise_params(width, height, **filter)
         self._check(self.lib.rt3_denoise_staged(self.handle, C.byref(p), int(tag), C.c_void_p(stage_ptr), _ptr(frame), _ptr(rgb)))
         return frame, rgb
+
+    def denoise_staged_temporal(self, width, height, stage_ptr, tag, reset=False, alpha_color=0.2, alpha_moments=0.2, depth_tolerance=0.05, normal_cos=0.9,
+                                **filter):
+        """rt3_denoise_staged_temporal: ``denoise_staged`` with this context's ``denoise_temporal`` history (the two calls share
+        it: ``reset`` drops it first); on the stage's owner, after every part staged frame ``tag``. ``filter`` takes
+        denoise_params' keywords. Returns (frame [H, W] uint32, rgb [H, W, 3] float32, history_length [H, W] float32)."""
+        frame = np.zeros((height, width), np.uint32)
+        rgb = np.zeros((height, width, 3), np.float32)
+        length = np.zeros((height, width), np.float32)
+        p = denoise_temporal_params(width, height, reset, alpha_color, alpha_moments, depth_tolerance, normal_cos, **filter)
+        self._check(self.lib.rt3_denoise_staged_temporal(self.handle, C.byref(p), int(tag), C.c_void_p(stage_ptr), _ptr(frame), _ptr(rgb), _ptr(length)))
+        return frame, rgb, length
 
     def stats(self):
         st = Stats()

@@ -736,6 +736,34 @@ int denoise(rt3_ctx* ctx, const rt3_denoise_params* params, uint32_t* host_frame
     return atrous_to_host(ctx, params, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, host_frame, host_rgb, nullptr, stream);
 }
 
+/* The start of a temporal call (rt3_denoise_temporal, rt3_denoise_staged_temporal), after every check: whether the
+ * history may be read (*have_prev: not reset, and one of this size and scene upload), then drops it until keep_history
+ * and sizes both histories (and the length for the host when `length`) and the filter's buffers (reserve_denoise). */
+int begin_history(rt3_ctx* ctx, const rt3_denoise_temporal_params* tp, uint32_t w, uint32_t h, bool guide, bool rgb, bool length, bool* have_prev) {
+    const size_t n = (size_t) w * h;
+    *have_prev = !tp->reset && ctx->dn_hist_valid && ctx->dn_hist_width == w && ctx->dn_hist_height == h && ctx->dn_hist_scene_id == ctx->scene_id;
+    ctx->dn_hist_valid = false;
+    int rc;
+    if ((rc = reserve_denoise(ctx, n, guide, rgb)) != RT3_OK) { return rc; }
+    for (uint32_t i = 0; i < 2; i++) {
+        if ((rc = ctx->dn_hist_col[i].reserve(n)) != RT3_OK || (rc = ctx->dn_hist_mom[i].reserve(n)) != RT3_OK || (rc = ctx->dn_hist_guide[i].reserve(n)) != RT3_OK) {
+            return rc;
+        }
+    }
+    if (length && (rc = ctx->dn_hist_length.reserve(n)) != RT3_OK) { return rc; }
+    return RT3_OK;
+}
+
+/* The end of a temporal call that succeeded: the history it wrote becomes the one the next call reads, with the AOVs'
+ * camera, the frame's size and the scene upload. */
+void keep_history(rt3_ctx* ctx, uint32_t w, uint32_t h) {
+    ctx->dn_hist_cur ^= 1u;
+    ctx->dn_hist_valid = true;
+    ctx->dn_hist_cam = ctx->path_aovs_cam;
+    ctx->dn_hist_width = w; ctx->dn_hist_height = h;
+    ctx->dn_hist_scene_id = ctx->scene_id;
+}
+
 /* rt3_denoise_temporal: rt3_denoise's checks and the temporal parameters', then the accumulation into the history not in
  * use, its variance, the à-trous passes and the read-back, blocking. The history is dropped when the call proceeds and
  * kept (swapped in) only when everything succeeded; a refusal changes nothing. */
@@ -748,17 +776,9 @@ int denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* tp, uint32
     RT3_CUDA(cudaSetDevice(ctx->device));
     const rt3_kparams& kp = ctx->accum_kp;
     const uint32_t w = kp.width, h = kp.height;
-    const size_t n = (size_t) w * h;
-    const bool have_prev = !tp->reset && ctx->dn_hist_valid && ctx->dn_hist_width == w && ctx->dn_hist_height == h && ctx->dn_hist_scene_id == ctx->scene_id;
-    ctx->dn_hist_valid = false;
+    bool have_prev;
+    if ((rc = begin_history(ctx, tp, w, h, true, host_rgb != nullptr, host_length != nullptr, &have_prev)) != RT3_OK) { return rc; }
     const uint32_t cur = ctx->dn_hist_cur, next = cur ^ 1u;
-    if ((rc = reserve_denoise(ctx, n, true, host_rgb != nullptr)) != RT3_OK) { return rc; }
-    for (uint32_t i = 0; i < 2; i++) {
-        if ((rc = ctx->dn_hist_col[i].reserve(n)) != RT3_OK || (rc = ctx->dn_hist_mom[i].reserve(n)) != RT3_OK || (rc = ctx->dn_hist_guide[i].reserve(n)) != RT3_OK) {
-            return rc;
-        }
-    }
-    if (host_length && (rc = ctx->dn_hist_length.reserve(n)) != RT3_OK) { return rc; }
     cudaStream_t stream = accum_stream(ctx);
     if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
     RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
@@ -775,11 +795,7 @@ int denoise_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* tp, uint32
     RT3_CUDA(cudaGetLastError());
     ctx->stats.kernel_launches += 2;
     if ((rc = atrous_to_host(ctx, &fp, ctx->dn_guide.ptr, ctx->aov_albedo.ptr, host_frame, host_rgb, host_length, stream)) != RT3_OK) { return rc; }
-    ctx->dn_hist_cur = next;
-    ctx->dn_hist_valid = true;
-    ctx->dn_hist_cam = ctx->path_aovs_cam;
-    ctx->dn_hist_width = w; ctx->dn_hist_height = h;
-    ctx->dn_hist_scene_id = ctx->scene_id;
+    keep_history(ctx, w, h);
     return RT3_OK;
 }
 
@@ -843,19 +859,17 @@ int denoise_stage(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame
     return RT3_OK;
 }
 
-/* rt3_denoise_staged: checks every row's fingerprint on the host, then the filter over the stage's planes, blocking. */
-int denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, const uint32_t* device_stage, uint32_t* host_frame, float* host_rgb) {
-    int rc = check_denoise_inputs(ctx, params, "rt3_denoise_staged", true);
-    if (rc != RT3_OK) { return rc; }
-    if (!device_stage) { return fail(RT3_ERR_INVALID, "rt3_denoise_staged: device_stage is NULL"); }
-    const rt3_kparams& kp = ctx->accum_kp;
-    const uint32_t w = kp.width, h = kp.height;
-    if (rt3_denoise_stage_words(w, h) == 0) { return fail(RT3_ERR_INVALID, "rt3_denoise_staged: a %ux%u frame does not fit in a stage", w, h); }
+/* The checks of the owner's calls on a stage (rt3_denoise_staged, rt3_denoise_staged_temporal, named by `fn`), after
+ * check_denoise_inputs: a stage, a frame that fits one, and every row's fingerprint equal to this context's for frame_tag,
+ * read back on `stream` (blocking). Sets the device and *s, the stage's planes. */
+int check_stage_rows(rt3_ctx* ctx, const char* fn, uint64_t frame_tag, const uint32_t* device_stage, cudaStream_t stream, stage_view* s) {
+    if (!device_stage) { return fail(RT3_ERR_INVALID, "%s: device_stage is NULL", fn); }
+    const uint32_t w = ctx->accum_kp.width, h = ctx->accum_kp.height;
+    if (rt3_denoise_stage_words(w, h) == 0) { return fail(RT3_ERR_INVALID, "%s: a %ux%u frame does not fit in a stage", fn, w, h); }
     RT3_CUDA(cudaSetDevice(ctx->device));
-    cudaStream_t stream = accum_stream(ctx);
-    const stage_view s = stage_planes(const_cast<uint32_t*>(device_stage), w, h);
+    *s = stage_planes(const_cast<uint32_t*>(device_stage), w, h);
     std::vector<unsigned long long> rows(h);
-    RT3_CUDA(cudaMemcpyAsync(rows.data(), s.fingerprint, h * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
+    RT3_CUDA(cudaMemcpyAsync(rows.data(), s->fingerprint, h * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream));
     RT3_CUDA(cudaStreamSynchronize(stream));
     const unsigned long long expect = stage_fingerprint(ctx, frame_tag);
     uint32_t bad = 0, first_bad = 0;
@@ -863,9 +877,21 @@ int denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t fram
         if (rows[y] != expect && bad++ == 0) { first_bad = y; }
     }
     if (bad) {
-        return fail(RT3_ERR_INVALID, "rt3_denoise_staged: row %u (and %u rows in all, of %u) was not staged for this frame: a part that did not run, a stale row of "
-                    "another frame_tag, or a part rendered with other parameters", first_bad, bad, h);
+        return fail(RT3_ERR_INVALID, "%s: row %u (and %u rows in all, of %u) was not staged for this frame: a part that did not run, a stale row of "
+                    "another frame_tag, or a part rendered with other parameters", fn, first_bad, bad, h);
     }
+    return RT3_OK;
+}
+
+/* rt3_denoise_staged: checks every row's fingerprint on the host, then the filter over the stage's planes, blocking. */
+int denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, const uint32_t* device_stage, uint32_t* host_frame, float* host_rgb) {
+    int rc = check_denoise_inputs(ctx, params, "rt3_denoise_staged", true);
+    if (rc != RT3_OK) { return rc; }
+    const rt3_kparams& kp = ctx->accum_kp;
+    const uint32_t w = kp.width, h = kp.height;
+    cudaStream_t stream = accum_stream(ctx);
+    stage_view s;
+    if ((rc = check_stage_rows(ctx, "rt3_denoise_staged", frame_tag, device_stage, stream, &s)) != RT3_OK) { return rc; }
     if ((rc = reserve_denoise(ctx, (size_t) w * h, false, host_rgb != nullptr)) != RT3_OK) { return rc; }
     if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
     RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
@@ -874,6 +900,46 @@ int denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t fram
     RT3_CUDA(cudaGetLastError());
     ctx->stats.kernel_launches += 1;
     return atrous_to_host(ctx, params, s.guide, s.albedo, host_frame, host_rgb, nullptr, stream);
+}
+
+/* rt3_denoise_staged_temporal: rt3_denoise_staged's checks and the temporal parameters', then rt3_denoise_temporal's
+ * steps on the owner's history with the pixels read from the stage, blocking. The rays are regenerated from the owner's
+ * AOV kparams with the partition removed: every part traced its rows with the same seed, sample range, flags and camera
+ * (the fingerprints), and start_path then takes the pixel index. */
+int denoise_staged_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* tp, uint64_t frame_tag, const uint32_t* device_stage, uint32_t* host_frame,
+                            float* host_rgb, float* host_length) {
+    if (!ctx) { return fail(RT3_ERR_INVALID, "ctx is NULL"); }
+    if (!tp) { return fail(RT3_ERR_INVALID, "rt3_denoise_staged_temporal: params is NULL"); }
+    int rc = check_denoise_inputs(ctx, &tp->filter, "rt3_denoise_staged_temporal", true);
+    if (rc != RT3_OK) { return rc; }
+    if (const char* why = rt3_dn_check_temporal_params(tp)) { return fail(RT3_ERR_INVALID, "rt3_denoise_staged_temporal: %s", why); }
+    const uint32_t w = ctx->accum_kp.width, h = ctx->accum_kp.height;
+    cudaStream_t stream = accum_stream(ctx);
+    stage_view s;
+    if ((rc = check_stage_rows(ctx, "rt3_denoise_staged_temporal", frame_tag, device_stage, stream, &s)) != RT3_OK) { return rc; }
+    bool have_prev;
+    if ((rc = begin_history(ctx, tp, w, h, false, host_rgb != nullptr, host_length != nullptr, &have_prev)) != RT3_OK) { return rc; }
+    const uint32_t cur = ctx->dn_hist_cur, next = cur ^ 1u;
+    rt3_kparams whole = ctx->path_aovs_kp;
+    whole.part_index = 0; whole.part_count = 1; whole.owned_rows = h;
+    whole.n_pixels = (unsigned long long) w * h;
+    whole.n_items = whole.n_pixels * whole.spp;
+    if ((rc = begin_pass(ctx, false, h, stream, nullptr)) != RT3_OK) { return rc; }
+    RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
+    const dim3 block(RT3_DN_BLOCK_X, RT3_DN_BLOCK_Y), grid = denoise_grid(w, h);
+    denoise_staged_temporal_kernel<<<grid, block, 0, stream>>>(whole, ctx->path_aovs_cam, ctx->dn_hist_cam, *tp, have_prev, s.col, s.guide,
+                                                               ctx->dn_hist_col[cur].ptr, ctx->dn_hist_mom[cur].ptr, ctx->dn_hist_guide[cur].ptr,
+                                                               ctx->dn_hist_col[next].ptr, ctx->dn_hist_mom[next].ptr, ctx->dn_hist_guide[next].ptr,
+                                                               ctx->dn_col[1].ptr, host_length ? ctx->dn_hist_length.ptr : nullptr);
+    RT3_CUDA(cudaGetLastError());
+    const rt3_denoise_params& fp = tp->filter;
+    denoise_temporal_variance_kernel<<<grid, block, 0, stream>>>(w, h, fp.sigma_depth, (uint32_t) fp.sigma_normal, ctx->dn_col[1].ptr, s.guide,
+                                                                 ctx->dn_hist_col[next].ptr, ctx->dn_hist_mom[next].ptr, ctx->dn_col[0].ptr);
+    RT3_CUDA(cudaGetLastError());
+    ctx->stats.kernel_launches += 2;
+    if ((rc = atrous_to_host(ctx, &fp, s.guide, s.albedo, host_frame, host_rgb, host_length, stream)) != RT3_OK) { return rc; }
+    keep_history(ctx, w, h);
+    return RT3_OK;
 }
 
 /* Reads back the timings and counters of the most recent render (synchronises its stream). */
@@ -1212,6 +1278,11 @@ int rt3_denoise_stage(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t f
 int rt3_denoise_staged(rt3_ctx* ctx, const rt3_denoise_params* params, uint64_t frame_tag, const uint32_t* device_stage, uint32_t* host_frame,
                        float* host_rgb) {
     return denoise_staged(ctx, params, frame_tag, device_stage, host_frame, host_rgb);
+}
+
+int rt3_denoise_staged_temporal(rt3_ctx* ctx, const rt3_denoise_temporal_params* params, uint64_t frame_tag, const uint32_t* device_stage,
+                                uint32_t* host_frame, float* host_rgb, float* host_history_length) {
+    return denoise_staged_temporal(ctx, params, frame_tag, device_stage, host_frame, host_rgb, host_history_length);
 }
 
 int rt3_render_device(rt3_ctx* ctx, const rt3_camera* camera, const rt3_params* params, uint32_t* device_frame, void* cuda_stream) {

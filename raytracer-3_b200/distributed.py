@@ -73,7 +73,9 @@ class SharedFrame:
     ``SharedFrame(ctx, dist, abi.denoise_stage_words(w, h), rank, world, device)``. Each rank then calls
     ``ctx.denoise_stage(w, h, shared.ptr, tag)`` and ``ctx.stats()`` (which waits for its stores), all ranks meet in a
     barrier that holds the host (``dist.barrier()``; ``finish()`` only orders torch's stream, not the library's), and the
-    owner calls ``ctx.denoise_staged(w, h, shared.ptr, tag)``.
+    owner calls ``ctx.denoise_staged(w, h, shared.ptr, tag)``, or ``ctx.denoise_staged_temporal(w, h, shared.ptr, tag)`` to
+    accumulate the frames of a sequence in the owner's history (the other ranks stage exactly as before and keep none; every
+    rank uploads a new scene when the owner does).
     """
 
     def __init__(self, ctx, dist, n_pixels, rank, world, device, owner=0):
