@@ -263,7 +263,8 @@ static inline const char* rt3_dn_check_params(const rt3_denoise_params* p) {
  * For pixel p = (x, y): e, L and the guide from rt3_dn_prepare_px; the surface point X = o + z d^ of the primary ray (o, d^)
  * of the AOV call's sample first_sample (a miss: the direction d^, a point at infinity); its continuous position in the
  * previous frame pos = (x, y) + (proj(prev, X) - proj(cur, X)); the 2x2 bilinear taps of the history around pos that
- * agree in geometry, weight-normalised, give c_h, m1_h, m2_h, n_h (none when their weights sum to <= 0.01); then
+ * agree in geometry, weight-normalised, give c_h, m1_h, m2_h and n_h = n_0 + sum w (n_q - n_0) / sum w, n_0 the first used
+ * tap's length (none when their weights sum to <= 0.01); then
  * n = n_h + 1, c = c_h + max(alpha_color, 1/n) (e - c_h), m1, m2 likewise towards L and L L with alpha_moments; without
  * history c = e, m1 = L, m2 = L L, n = 1. The variance is max(0, m2 - m1 m1) from n >= 4, else the 7x7 estimate over the
  * accumulated colour. */
@@ -337,7 +338,9 @@ RT3_HD int rt3_dn_history_tap_ok(rt3_dn_guide p, rt3_dn_guide q, float dist, flo
 RT3_HD void rt3_dn_accumulate_px(const rt3_dn_hist* RT3_DN_RESTRICT prev_col, const rt3_dn_moments* RT3_DN_RESTRICT prev_mom,
                                  const rt3_dn_guide* RT3_DN_RESTRICT prev_guide, uint32_t w, uint32_t h, int have, float px, float py, float dist,
                                  rt3_dn_px e, rt3_dn_guide gp, const rt3_denoise_temporal_params* tp, rt3_dn_hist* col, rt3_dn_moments* mom) {
-    float sw = 0.0f, sr = 0.0f, sg = 0.0f, sb = 0.0f, sn = 0.0f, s1 = 0.0f, s2 = 0.0f;
+    /* The length is summed relative to the first used tap's, n0: taps that all carry one length give exactly that length
+     * (sum w n / sum w rounds 3 to 2.9999998 for some weights), so a whole number of frames stays whole (step 7's n >= 4). */
+    float sw = 0.0f, sr = 0.0f, sg = 0.0f, sb = 0.0f, sn = 0.0f, s1 = 0.0f, s2 = 0.0f, n0 = 0.0f;
     if (have && px > -1.0f && px < (float) w && py > -1.0f && py < (float) h) {
         const float fx0 = floorf(px), fy0 = floorf(py);
         const float fx = px - fx0, fy = py - fy0;
@@ -355,9 +358,10 @@ RT3_HD void rt3_dn_accumulate_px(const rt3_dn_hist* RT3_DN_RESTRICT prev_col, co
                 if (!rt3_dn_history_tap_ok(gp, prev_guide[q], dist, tp->depth_tolerance, tp->normal_cos)) { continue; }
                 const rt3_dn_hist hq = prev_col[q];
                 const rt3_dn_moments mq = prev_mom[q];
+                if (sw == 0.0f) { n0 = hq.n; }
                 sw = sw + wt;
                 sr = sr + wt * hq.r; sg = sg + wt * hq.g; sb = sb + wt * hq.b;
-                sn = sn + wt * hq.n;
+                sn = sn + wt * (hq.n - n0);
                 s1 = s1 + wt * mq.m1; s2 = s2 + wt * mq.m2;
             }
         }
@@ -369,7 +373,7 @@ RT3_HD void rt3_dn_accumulate_px(const rt3_dn_hist* RT3_DN_RESTRICT prev_col, co
         return;
     }
     const float hr = sr / sw, hg = sg / sw, hb = sb / sw, h1 = s1 / sw, h2 = s2 / sw;
-    const float n = sn / sw + 1.0f;
+    const float n = (n0 + sn / sw) + 1.0f;
     const float inv = 1.0f / n;
     const float ac = tp->alpha_color > inv ? tp->alpha_color : inv, am = tp->alpha_moments > inv ? tp->alpha_moments : inv;
     col->r = hr + ac * (e.r - hr); col->g = hg + ac * (e.g - hg); col->b = hb + ac * (e.b - hb); col->n = n;

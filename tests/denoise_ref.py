@@ -183,6 +183,15 @@ def denoise(rgb, albedo, normal, depth, iterations=5, sigma_luminance=4.0, sigma
     g = guide(normal, depth, mutation)
     var, cancellation = variance(Taps(h, w, 3, clamp=mutation == "clamp_border"), g, luminance(e0), sigma_z=sigma_depth, sigma_n=sigma_normal,
                                  mutation=mutation)
+    passes = atrous_passes(e0, var, g, iterations, sigma_luminance, sigma_normal, sigma_depth, mutation)
+    out = passes[-1] * d
+    level, frame = resolve(out, gamma)
+    return {"input": e0, "passes": passes, "rgb": out, "level": level, "frame": frame, "cancellation": cancellation}
+
+
+def atrous_passes(e0, var, g, iterations=5, sigma_luminance=4.0, sigma_normal=128.0, sigma_depth=1.0, mutation=None):
+    """The ``iterations`` passes over demodulated colour e0 [H, W, 3] with its luminance variance var [H, W] and guide g:
+    the demodulated output of every pass."""
     e = e0
     passes = []
     for i in range(iterations):
@@ -190,6 +199,4 @@ def denoise(rgb, albedo, normal, depth, iterations=5, sigma_luminance=4.0, sigma
         lum_stop = luminance(e0 if mutation == "luminance_of_input" else e)
         e, var = atrous_pass(e, var, lum_stop, g, step, sigma_luminance, sigma_depth, sigma_normal, mutation)
         passes.append(e)
-    out = e * d
-    level, frame = resolve(out, gamma)
-    return {"input": e0, "passes": passes, "rgb": out, "level": level, "frame": frame, "cancellation": cancellation}
+    return passes

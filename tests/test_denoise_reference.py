@@ -266,17 +266,19 @@ def ill_conditioned(res, iterations):
     return out
 
 
-def compare(inp, passes, frame, what, flags=0, skip_ill=False, **dn):
+def compare(inp, passes, frame, what, flags=0, skip_ill=False, res=None, hull_input=None, **dn):
     """Every pass of a filter's output (demodulated, from its float32 rgb) and its frame against the reference on the same
     inputs: the error per pass at most tau, every pass inside its taps' hull, the frame by the rounding-boundary rule. With
     ``skip_ill``, the pixels that depend on an ill-conditioned luminance stop (ill_conditioned()) are held to the hull only.
-    Returns the worst error."""
-    res = ref.denoise(*inp, gamma=not flags & abi.FLAG_NO_GAMMA, **dn)
+    ``res`` is the reference's result when it is not ``ref.denoise`` of ``inp`` (the temporal call's), ``hull_input`` the
+    colour the first pass filtered when it is not the reference's input (the float32 accumulated colour). Returns the
+    worst error."""
+    res = ref.denoise(*inp, gamma=not flags & abi.FLAG_NO_GAMMA, **dn) if res is None else res
     ill = ill_conditioned(res, len(passes)) if skip_ill else [np.zeros(inp[3].shape, bool)] * len(passes)
     errs = [rel_error(np.where(m[..., None], b, a), b) for a, b, m in zip(passes, res["passes"], ill)]
     t = tau(dn.get("sigma_normal", 128.0))
     assert max(errs) <= t, f"{what}: error per pass {['%.3g' % e for e in errs]} (tau {t:.3g})"
-    assert_in_hull(res["input"], passes, what)
+    assert_in_hull(res["input"] if hull_input is None else hull_input, passes, what)
     near, bad = frame_check(frame, res, inp[1], t, ill[-1], gamma=not flags & abi.FLAG_NO_GAMMA)
     assert bad == 0, f"{what}: {bad} channels of the 8-bit frame differ from the reference's"
     print(f"{what}: worst error {max(errs):.3g} (tau {t:.3g}), {near} pixels off by one at an 8-bit rounding boundary"

@@ -221,22 +221,27 @@ def test_valid_parameter_edges_are_accepted():
 
 # ---- the float64 reference ---------------------------------------------------------------------------------------------
 
-def sequence_case(kind, lens, frames, w=27, h=19):
-    """Yields (restatement history, reference step) of a sequence on a wavy plane under a sky whose lower edge moves by a
-    row every other frame, jittered rays, and the camera `still`, panned by 0.995 px per frame (the last column's only
-    tap then weighs 0.005, under the 0.01 floor), translated sideways and up, or dollied forward."""
+def case_frame(kind, lens, i, w=27, h=19):
+    """Frame i of sequence_case: (camera, (rgb, albedo, normal, depth), AOV params)."""
     base = abi.reference_camera(w, h)
     if lens:
         thin_lens(base)
     _, hor, _, _ = cam_arrays(base)
+    cam = {"still": base, "pan": shifted(base, llc=0.995 * i * hor / (w - 1)),
+           "translate": shifted(base, origin=(0.04 * i, 0.01 * i, 0), llc=(0.04 * i, 0.01 * i, 0)),
+           "dolly": shifted(base, origin=(0, 0, -0.25 * i), llc=(0, 0, -0.25 * i))}[kind]
+    ins = plane_scene(cam, w, h, sky_rows=4 + i % 2, seed=i)
+    ins = (ins[0], ins[1], ins[2], (ins[3] * f32(1 + 0.02 * np.sin(np.arange(w) / 3.0))).astype(f32))
+    return cam, ins, params(w, h, seed=7 + i, flags=0)
+
+
+def sequence_case(kind, lens, frames, w=27, h=19):
+    """Yields (restatement history, reference step) of a sequence on a wavy plane under a sky whose lower edge moves by a
+    row every other frame, jittered rays, and the camera `still`, panned by 0.995 px per frame (the last column's only
+    tap then weighs 0.005, under the 0.01 floor), translated sideways and up, or dollied forward."""
     hist = ref_hist = None
     for i in range(frames):
-        cam = {"still": base, "pan": shifted(base, llc=0.995 * i * hor / (w - 1)),
-               "translate": shifted(base, origin=(0.04 * i, 0.01 * i, 0), llc=(0.04 * i, 0.01 * i, 0)),
-               "dolly": shifted(base, origin=(0, 0, -0.25 * i), llc=(0, 0, -0.25 * i))}[kind]
-        ins = plane_scene(cam, w, h, sky_rows=4 + i % 2, seed=i)
-        ins = (ins[0], ins[1], ins[2], (ins[3] * f32(1 + 0.02 * np.sin(np.arange(w) / 3.0))).astype(f32))
-        p = params(w, h, seed=7 + i, flags=0)
+        cam, ins, p = case_frame(kind, lens, i, w, h)
         _, _, _, hist = dl.oracle_denoise_temporal(*ins, cam, p, hist)
         r = yield hist, ins, dl.primary_rays(cam, p), cam, ref_hist
         ref_hist = r["history"]
