@@ -410,6 +410,15 @@ int end_pass(rt3_ctx* ctx, cudaStream_t stream) {
     return RT3_OK;
 }
 
+/* Records the path-traced render just enqueued as the one the accumulators hold: its rows (none, for a partition that owns
+ * no rows), sample range and camera, which rt3_read_radiance, RT3_FLAG_ACCUMULATE and the denoise calls check against. */
+void record_accum(rt3_ctx* ctx, const rt3_camera* cam, const rt3_kparams& kp, bool accumulate) {
+    ctx->accum_kp = kp;
+    ctx->accum_valid = true;
+    if (!accumulate) { ctx->accum_cam = *cam; ctx->accum_cam_mixed = false; ctx->accum_first = kp.first_sample; }
+    else if (memcmp(&ctx->accum_cam, cam, sizeof *cam) != 0) { ctx->accum_cam_mixed = true; }
+}
+
 /* Enqueues one render of this partition into device_frame (full-frame indexing). */
 int enqueue_render(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params, const rt3_kparams& kp_in, uint32_t* device_frame,
                    uint32_t* prim, uint32_t* ent, float* t, cudaStream_t stream) {
@@ -437,10 +446,15 @@ int enqueue_render(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params
     kp.resident = plan.resident ? 1u : 0u;
     std::unique_lock<std::mutex> bank_lock; /* released when this function returns, i.e. after the launch below */
     if ((rc = begin_pass(ctx, plan.accel, kp.owned_rows, stream, plan.resident && kp.n_pixels != 0 ? &bank_lock : nullptr)) != RT3_OK) { return rc; }
+    const bool path = params->mode == RT3_MODE_PATHTRACE;
+    const bool accumulate = path && (params->flags & RT3_FLAG_ACCUMULATE) != 0;
+    if (path && !accumulate) { ctx->accum_valid = false; } /* the accumulators no longer hold the previous render */
     if (kp.n_pixels == 0) {
+        /* a partition that owns no rows: nothing to trace, but it is this render the accumulators now stand for */
         RT3_CUDA(cudaEventRecord(ctx->ev_k0, stream));
         RT3_CUDA(cudaEventRecord(ctx->ev_k1, stream));
         RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
+        if (path) { record_accum(ctx, cam, kp, accumulate); }
         return RT3_OK;
     }
     if (params->mode == RT3_MODE_REFERENCE) {
@@ -455,9 +469,7 @@ int enqueue_render(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params
         return rc;
     }
     size_t n_acc = (size_t) kp.width * kp.height * 3;
-    const bool accumulate = (params->flags & RT3_FLAG_ACCUMULATE) != 0;
     if (!accumulate) {
-        ctx->accum_valid = false;
         rc = ctx->accum.reserve(n_acc);
         if (rc != RT3_OK) { return rc; }
         unsigned clear_grid = (unsigned) ((kp.n_pixels * 3ull + 255ull) / 256ull);
@@ -505,10 +517,7 @@ int enqueue_render(rt3_ctx* ctx, const rt3_camera* cam, const rt3_params* params
     RT3_CUDA(cudaGetLastError());
     RT3_CUDA(cudaEventRecord(ctx->ev_end, stream));
     ctx->stats.kernel_launches = accumulate ? 2 : 3;
-    ctx->accum_kp = kp;
-    ctx->accum_valid = true;
-    if (!accumulate) { ctx->accum_cam = *cam; ctx->accum_cam_mixed = false; ctx->accum_first = kp.first_sample; }
-    else if (memcmp(&ctx->accum_cam, cam, sizeof *cam) != 0) { ctx->accum_cam_mixed = true; }
+    record_accum(ctx, cam, kp, accumulate);
     return RT3_OK;
 }
 
